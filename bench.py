@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- BACS loss step throughput (pixels/s, forward + backward) on B200.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--config NAME]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--config NAME] [--dump-outputs DIR]
 
 One "step" = one pass of the whole BACS loss path (SURVEY 8a rows 3-12) over one batch of
 synthetic network outputs: prototype update, seen-head logits, fused weighted-CE + focal +
@@ -41,7 +41,9 @@ UNIT = "pixels/s"
 def parse():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=200)
+    ap.add_argument("--steps", type=int, default=None,
+                    help="timed steps of every timed window (default: 200; 2 with --impl reference, whose step takes "
+                         "seconds on the host; 20 with --config cityscapes_eval)")
     ap.add_argument("--warmup", type=int, default=10)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--config", default="voc15-1_b24")
@@ -55,7 +57,34 @@ def parse():
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-fused-lowres", action="store_true",
                     help="skip the extra timing of BACSLoss(fused_logit_upsample=True) (low-res logits in, N=1 only)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last timed step returned (loss, arg-max, gradients, "
+                         "updated prototypes and counts) as DIR/<name>.npy, to compare two builds output for output")
+    args = ap.parse_args()
+    if args.steps is None:
+        args.steps = 2 if args.impl == "reference" else 20 if args.config == "cityscapes_eval" else 200
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl == "reference" or args.config == "cityscapes_eval"):
+        ap.error("--dump-outputs writes what the BACS loss step on the GPU returns; --impl reference and "
+                 "--config cityscapes_eval do not run that step")
+    return args
+
+
+DUMP_SAMPLE = 1 << 20
+
+
+def host_sample(t):
+    """-> a host numpy copy of ``t``: float64 stays float64, everything else becomes float32.  A tensor of more than
+    DUMP_SAMPLE elements is replaced by its elements at DUMP_SAMPLE flat positions drawn from a generator with a fixed
+    seed, so every run of every build keeps the same positions (at most 8 MB per array)."""
+    import numpy as np
+    import torch
+    t = t.detach()
+    if t.numel() > DUMP_SAMPLE:
+        idx = np.sort(np.random.default_rng(0).integers(0, t.numel(), DUMP_SAMPLE))
+        t = t.reshape(-1)[torch.from_numpy(idx).to(t.device)]
+    return t.to(torch.float64 if t.dtype == torch.float64 else torch.float32).cpu().numpy()
 
 
 def peaks():
@@ -162,7 +191,7 @@ def run_reference(args):
         ncores = os.cpu_count() or 1
     torch.set_num_threads(max(1, ncores))
     cfg = synth.CONFIGS[args.config]
-    steps, warmup = max(1, min(args.steps, 2)), 0
+    steps, warmup = args.steps, 0
     batch = max(1, min(args.ref_sample_batch, cfg.B))
     value, dt, sample, kind = cpu_step_time(cfg, batch, steps, warmup)
     cores = torch.get_num_threads()
@@ -182,7 +211,7 @@ def workload_name(cfg):
             (cfg.name, cfg.B, cfg.K, cfg.old_cl, cfg.T, cfg.H, cfg.W, cfg.h, cfg.w, cfg.D, cfg.A))
 
 
-def integer_rows(timed_fn, dev, peak, shape=(4, 1024, 2048), K=20):
+def integer_rows(timed_fn, dev, peak, shape=(4, 1024, 2048), K=20, steps=20):
     """The integer rows of the path, each timed alone on inputs larger than L2 (SURVEY 8a rows 14, 0, 3):
     * confusion-matrix histogram at the Cityscapes evaluation shape (training/metrics.py:38-50): 16 B of int64
       predictions + targets per pixel; on uniformly random classes (every lane a different bin: the worst case for
@@ -221,7 +250,7 @@ def integer_rows(timed_fn, dev, peak, shape=(4, 1024, 2048), K=20):
             ("label_downsample_task [%d,%d,%d] -> /16" % (B, H, W),
              lambda: ops.label_downsample_task(target, H // 16, W // 16, task_lut, 4), (32 + 13) * (px // 256),
              "latency: one 32-byte sector per low-res pixel + block scan; 1/256 of the labels are read")):
-        ms = timed_fn(fn, 20, 3)
+        ms = timed_fn(fn, steps, 3)
         gbs = nbytes / (ms * 1e-3) / 1e9
         rows.append({"name": name, "us": ms * 1e3, "algorithmic_bytes": nbytes, "GB/s": gbs,
                      "frac_of_hbm_peak": gbs / peak, "limiter": limiter})
@@ -230,12 +259,12 @@ def integer_rows(timed_fn, dev, peak, shape=(4, 1024, 2048), K=20):
     f = torch.randn(Bc, Dc, hc, wc, device=dev, generator=g).to(torch.bfloat16)
     c = torch.randn(Kc, Dc, device=dev, generator=g).to(torch.bfloat16)
     lab = torch.randint(0, Kc + 1, (Bc, hc, wc), device=dev, generator=g, dtype=torch.int64)
-    ms = timed_fn(lambda: ops.class_distance(f, c), 20, 3)
+    ms = timed_fn(lambda: ops.class_distance(f, c), steps, 3)
     flop = 2.0 * Bc * hc * wc * 160 * Dc
     rows.append({"name": "class_distance [%d,%d,%d,%d] x %d classes (tcgen05, bf16)" % (Bc, Dc, hc, wc, Kc), "us": ms * 1e3,
                  "algorithmic_bytes": int(f.numel() * 2 + Bc * Kc * hc * wc * 4), "TFLOP/s": flop / (ms * 1e-3) / 1e12,
                  "limiter": "prototype fill from L2 + 192 tiles on 148 SMs (a 4 GFLOP product)"})
-    ms = timed_fn(lambda: ops.class_sums(f, lab, Kc + 1), 20, 3)
+    ms = timed_fn(lambda: ops.class_sums(f, lab, Kc + 1), steps, 3)
     rows.append({"name": "class_sums [%d,%d,%d,%d] into %d classes" % (Bc, Dc, hc, wc, Kc + 1), "us": ms * 1e3,
                  "algorithmic_bytes": int(f.numel() * 2), "GB/s": f.numel() * 2 / (ms * 1e-3) / 1e9,
                  "limiter": "shared-memory table update per pixel + per-class warp sums"})
@@ -248,7 +277,7 @@ def integer_rows(timed_fn, dev, peak, shape=(4, 1024, 2048), K=20):
     z = torch.randn(cfg.B, cfg.T, cfg.h, cfg.w, device=dev, generator=g)
     kw = dict(want_grad=True, z=z, want_distill_mask=True, old_cl=cfg.old_cl, focal_head=cfg.T - 1)
     variant = ops.pixel_loss(logits, mask, _cabi.PIX_WEIGHTED_CE, **kw)["variant"]
-    ms = timed_fn(lambda: ops.pixel_loss(logits, mask, _cabi.PIX_WEIGHTED_CE, **kw), 10, 3)
+    ms = timed_fn(lambda: ops.pixel_loss(logits, mask, _cabi.PIX_WEIGHTED_CE, **kw), steps, 3)
     nbytes = cfg.B * cfg.H * cfg.W * (2 * cfg.K * 2 + 17)
     gbs = nbytes / (ms * 1e-3) / 1e9
     rows.append({"name": "pixel_loss ade100-50 [%d,%d,%d,%d] bf16 (variant %d: one pass, channel column in registers)"
@@ -276,19 +305,19 @@ def run_integer_rows(args, dev, world, rank):
         torch.cuda.synchronize()
         return e0.elapsed_time(e1) / steps
     peak, peak_src = peaks()
-    rows = integer_rows(timed, dev, peak, shape=(8, 1024, 2048), K=20)
+    rows = integer_rows(timed, dev, peak, shape=(8, 1024, 2048), K=20, steps=args.steps)
     cm = rows[1]                      # the evaluation-like input
     px = 8 * 1024 * 2048
     if rank == 0:
         print(json.dumps({"metric": "confusion-matrix pixels/sec (Cityscapes 1024x2048 evaluation)", "value": px / (cm["us"] * 1e-6),
-                          "unit": UNIT, "n_gpus": 1, "steps": 20, "warmup": 3, "ms_per_step": cm["us"] * 1e-3,
+                          "unit": UNIT, "n_gpus": 1, "steps": args.steps, "warmup": 3, "ms_per_step": cm["us"] * 1e-3,
                           "higher_is_better": True, "scaling": "weak", "vs_baseline": None, "dtype": "int64",
                           "data": "synthetic", "config": {"workload": "cityscapes_eval: " + cm["name"],
                                                           "l2_policy": "inputs larger than L2 (268 MB per launch)"},
                           "roofline": {"bound": "hbm", "kernel": "confmat_kernel", "achieved": cm["GB/s"], "peak": peak,
                                        "unit": "GB/s", "frac": cm["frac_of_hbm_peak"], "traffic": None,
                                        "peak_source": peak_src},
-                          "other_kernels": rows, "gpu_launches": 23 * len(rows)}), flush=True)
+                          "other_kernels": rows, "gpu_launches": (args.steps + 3) * len(rows)}), flush=True)
 
 
 def verify_ranks(loss_fn, leaves, batch, cfg, dev, world, rank):
@@ -342,6 +371,7 @@ def main():
     if args.impl == "reference":
         return run_reference(args)
 
+    import numpy as np
     import torch
     import torch.distributed as dist
     from bacs_b200 import _cabi, ops, synth
@@ -366,13 +396,23 @@ def main():
     protos0 = loss_fn._prototypes._prototypes_tensors.clone()
     counts0 = loss_fn._prototypes._count_features.clone()
     pixels = cfg.B * cfg.H * cfg.W
+    last = {}                         # the outputs of the latest step (the graph's own buffers once it is captured)
 
     def step():
         for v in leaves.values():
             v.grad = None
         loss, preds = loss_fn.compute_loss(batch, net, train=True)
         loss.backward()
+        last["loss"], last["preds"] = loss.detach(), preds     # detached: the autograd graph must not outlive the step
         return loss, preds
+
+    def snapshot():
+        """host copies of what the latest step returned to its caller"""
+        torch.cuda.synchronize()
+        out = {"loss": last["loss"], "preds": last["preds"], "prototypes": loss_fn.prototypes,
+               "prototype_counts": loss_fn._prototypes._count_features}
+        out.update(("grad_" + k, v.grad) for k, v in leaves.items() if v.grad is not None)
+        return {k: host_sample(v) for k, v in out.items()}
 
     def barrier():
         if world > 1:
@@ -413,6 +453,8 @@ def main():
     step()
     launches_per_step = int(lib.bacs_launch_count() - n0)
     ms_eager = timed(step, args.steps, max(args.warmup, 3))
+    # taken after each timed window, before anything below runs the loss again and moves the prototypes on
+    dumped = snapshot() if args.dump_outputs and rank == 0 else None
 
     # ---- the same step captured once in a CUDA graph (the step never synchronises with the host)
     ms_graph = None
@@ -428,11 +470,17 @@ def main():
             with torch.cuda.graph(graph):
                 step()
             ms_graph = timed(graph.replay, args.steps, max(args.warmup, 3))
+            if dumped is not None:
+                dumped = snapshot()
         except Exception as exc:                                  # noqa: BLE001
             sys.stderr.write("bench.py: CUDA-graph replay unavailable: %r\n" % (exc,))
             ms_graph = None
     ms_step = ms_eager if ms_graph is None else min(ms_eager, ms_graph)
     value = world * pixels / (ms_step * 1e-3)
+    if dumped is not None:
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for name, arr in dumped.items():
+            np.save(os.path.join(args.dump_outputs, name + ".npy"), arr)
 
     # ---- dominant kernel (fused pixel kernel) timed alone, back to back, on its launch stream
     es = torch.finfo(dtype).bits // 8

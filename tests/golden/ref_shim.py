@@ -1,18 +1,19 @@
 """Import shim for the upstream reference (test infrastructure only).
 
-Loads the reference's hot-path modules from /root/reference WITHOUT running its
-package __init__ files (they pull in pytorch_lightning / hydra / wandb, which are
-not installed), by registering empty namespace packages and stubbing the three
-third-party imports the hot path touches.  Nothing is copied from the reference;
-this only makes `import loss.bacs_loss` etc. work in this container so golden
-vectors can be generated and the oracle can be pinned.  The GPU box has no
-/root/reference, so nothing in the gpu tests / bench / smoke imports this file.
+Loads the reference's hot-path modules from its source tree (BACS_REFERENCE_ROOT, else the
+copy oracle/make_ref.py stages under oracle/_ref/) WITHOUT running its package __init__
+files (they pull in pytorch_lightning / hydra / wandb, which are not installed), by
+registering empty namespace packages and stubbing the three third-party imports the hot
+path touches.  Nothing is copied from the reference; this only makes `import
+loss.bacs_loss` etc. work so golden vectors can be generated and the oracle can be pinned.
+Nothing in the product package, the GPU tests, bench.py's GPU path or smoke() imports it.
 """
 import os
 import sys
 import types
 
-REFERENCE_ROOT = os.environ.get("BACS_REFERENCE_ROOT", "/root/reference")
+REFERENCE_ROOT = os.environ.get("BACS_REFERENCE_ROOT") or os.path.join(
+    os.path.dirname(os.path.dirname(os.path.dirname(os.path.abspath(__file__)))), "oracle", "_ref")
 
 
 def reference_available() -> bool:

@@ -45,7 +45,8 @@ def test_buffer_invariants(tmp_path, monkeypatch):
 
 
 @pytest.mark.reference
-@pytest.mark.skipif(not ref_shim.reference_available(), reason="no /root/reference")
+@pytest.mark.skipif(not ref_shim.reference_available(),
+                    reason="upstream BACS source tree not found (set BACS_REFERENCE_ROOT)")
 def test_buffer_matches_reference(tmp_path, monkeypatch):
     if not hasattr(np, "Inf"):
         monkeypatch.setattr(np, "Inf", np.inf, raising=False)     # the reference predates numpy 2

@@ -1,7 +1,10 @@
 """Pins oracle/bacs_oracle.py against the *imported* reference code (CPU, fp32).
 
-Runs only where /root/reference exists (this container); the committed fixtures in
-tests/golden/ carry the same checks to boxes without the reference tree."""
+The tests marked ``reference`` import the upstream BACS code and run only where its source tree
+is found (tests/golden/ref_shim.py).  Of what they check, only the reference's outputs for the
+full step at the ``tiny`` shape, the label remap, the class -> task map of five class splits and
+the IoU vector are stored (tests/golden/*.npz, checked by test_golden.py); the rest is checked
+nowhere else.  The other tests compare with PyTorch's own ops and run everywhere."""
 import math
 import warnings
 
@@ -14,12 +17,11 @@ from fake_net import FakeNet
 from oracle import bacs_oracle as O
 from bacs_b200 import synth
 
-pytestmark = [pytest.mark.reference,
-              pytest.mark.skipif(not ref_shim.reference_available(), reason="no /root/reference")]
-
 
 @pytest.fixture(scope="module")
 def ref():
+    if not ref_shim.reference_available():
+        pytest.skip("upstream BACS source tree not found (set BACS_REFERENCE_ROOT)")
     warnings.filterwarnings("ignore")
     return ref_shim.install()
 
@@ -55,13 +57,14 @@ def _ref_seen_net(ref, inp):
     return bg
 
 
-def test_label_downsample_matches_interpolate(ref):
+def test_label_downsample_matches_interpolate():
     for (H, W, h, w) in [(512, 512, 32, 32), (528, 528, 33, 33), (513, 513, 33, 33), (64, 96, 4, 6), (100, 75, 7, 5)]:
         t = torch.randint(0, 256, (2, H, W))
         want = torch.nn.functional.interpolate(t.unsqueeze(1).double(), size=(h, w), mode="nearest").long()[:, 0]
         assert torch.equal(O.downsample_labels(t, h, w), want)
 
 
+@pytest.mark.reference
 def test_class_to_task_matches(ref):
     for init, inc in [(16, 1), (16, 5), (11, 1), (101, 50), (15, 2), (20, 0)]:
         L = ref["loss.base_loss"].BaseLoss("x")
@@ -72,6 +75,7 @@ def test_class_to_task_matches(ref):
         assert np.array_equal(np.broadcast_to(np.asarray(want).astype(np.int64), got.shape), got), (init, inc)
 
 
+@pytest.mark.reference
 @pytest.mark.parametrize("name,B", [("tiny", 1), ("tiny", 2), ("small", 3)])
 def test_prototype_update_matches(ref, name, B):
     cfg = synth.CONFIGS[name]
@@ -99,6 +103,7 @@ def test_prototype_update_matches(ref, name, B):
         _close(s2, sums)
 
 
+@pytest.mark.reference
 def test_seen_probs_match(ref):
     inp = synth.make_step_inputs(synth.CONFIGS["tiny"], seed=1)
     bg = _ref_seen_net(ref, inp)
@@ -110,7 +115,7 @@ def test_seen_probs_match(ref):
     _close(O.bilinear_upsample(z, want_t.shape[-2:], True), want_t)
 
 
-def test_bilinear_matches_interpolate(ref):
+def test_bilinear_matches_interpolate():
     x = torch.randn(2, 3, 5, 7)
     for ac in (True, False):
         want = torch.nn.functional.interpolate(x, size=(80, 112), mode="bilinear", align_corners=ac)
@@ -120,7 +125,7 @@ def test_bilinear_matches_interpolate(ref):
 
 
 @pytest.mark.parametrize("shape,stride", [((2, 7, 4, 6), 16), ((1, 21, 33, 33), 16), ((2, 5, 8, 10), 8)])
-def test_upsample_sem_logits_matches_network_op(ref, shape, stride):
+def test_upsample_sem_logits_matches_network_op(shape, stride):
     """networks/deeplab_v3.py:157-160: F.interpolate(sem_logits, size=input_shape, mode="bilinear",
     align_corners=False) -- values and the gradient autograd sends back to sem_logits (oracle of the fused low-res path)"""
     g = torch.Generator().manual_seed(shape[1])
@@ -137,6 +142,7 @@ def test_upsample_sem_logits_matches_network_op(ref, shape, stride):
     _close(b.grad, a.grad, atol=1e-5 * float(a.grad.abs().max()))
 
 
+@pytest.mark.reference
 @pytest.mark.parametrize("ukd", [True, False])
 @pytest.mark.parametrize("name", ["tiny", "small"])
 def test_weighted_ce_matches(ref, name, ukd):
@@ -156,11 +162,16 @@ def test_weighted_ce_matches(ref, name, ukd):
     _close(x2.grad, x1.grad, atol=1e-6 * float(x1.grad.abs().max()))
 
 
-def test_cross_entropy_variants_match(ref):
+def _cross_entropy_case():
     cfg = synth.CONFIGS["small"]
     inp = synth.make_step_inputs(cfg, seed=4)
     gen = torch.Generator().manual_seed(2)
     mask = synth.make_labels(cfg, gen, classes=list(range(1, cfg.K)))
+    return cfg, inp, gen, mask
+
+
+def test_cross_entropy_matches_torch():
+    cfg, inp, _, mask = _cross_entropy_case()
     F = torch.nn.functional
     w = torch.zeros(cfg.K)
     w[1:cfg.old_cl] = 1
@@ -170,6 +181,11 @@ def test_cross_entropy_variants_match(ref):
     w2[0] = 0
     want = -1 * F.cross_entropy(inp.logits, mask, ignore_index=255, weight=w2, reduction="none").view(cfg.B, -1).mean(1)
     _close(O.cross_entropy_per_image_score(inp.logits, mask, w2), want)
+
+
+@pytest.mark.reference
+def test_cross_entropy_variants_match(ref):
+    cfg, inp, gen, mask = _cross_entropy_case()
     U = ref["training.loss_utils"].UnbiasedCrossEntropy(old_cl=cfg.old_cl)
     _close(O.unbiased_ce(inp.logits, mask, cfg.old_cl), U(inp.logits, mask))
     KD = ref["training.loss_utils"].UnbiasedKnowledgeDistillationLoss(alpha=1.0)
@@ -179,6 +195,7 @@ def test_cross_entropy_variants_match(ref):
     _close(O.unbiased_kd(inp.logits, old, mask=pm), KD(inp.logits, old, mask=pm))
 
 
+@pytest.mark.reference
 @pytest.mark.parametrize("with_seen", [True, False])
 def test_teacher_distill_matches(ref, with_seen):
     cfg = synth.CONFIGS["tiny"]
@@ -196,6 +213,7 @@ def test_teacher_distill_matches(ref, with_seen):
     _close(n2.grad, n1.grad, atol=1e-6 * float(n1.grad.abs().max()))
 
 
+@pytest.mark.reference
 def test_der_mse_matches(ref):
     cfg = synth.CONFIGS["tiny"]
     for seed, ncls in [(0, [5, 6]), (1, [7, 7]), (2, [4, 7])]:
@@ -219,6 +237,7 @@ def test_der_mse_matches(ref):
         _close(s2.grad, s1.grad, atol=1e-7)
 
 
+@pytest.mark.reference
 def test_der_transplant_quirk_bigger_batch(ref):
     # Br=5 with repeated class counts: exercises the sample-index-vs-mask quirk (Q5)
     K, Br = 9, 5
@@ -238,6 +257,7 @@ def test_der_transplant_quirk_bigger_batch(ref):
         _close(got, want)
 
 
+@pytest.mark.reference
 def test_focal_seen_loss_matches(ref):
     cfg = synth.CONFIGS["tiny"]
     inp = synth.make_step_inputs(cfg, seed=8)
@@ -257,7 +277,7 @@ def test_focal_seen_loss_matches(ref):
     assert float(O.focal_seen_loss(zf, no_bg)) == 0.0
 
 
-def test_confmat_known_answer(ref):
+def test_confmat_known_answer():
     # the reference's only known-answer vector: training/metrics.py:159-183
     label = np.zeros((1, 4, 4), dtype=np.int64)
     pred = np.zeros((1, 4, 4), dtype=np.float32)
@@ -269,6 +289,7 @@ def test_confmat_known_answer(ref):
     assert np.allclose(m["iou_per_class"], [2.0 / 12, 4.0 / 14], atol=1e-6)
 
 
+@pytest.mark.reference
 def test_transform_label_sequential(ref):
     TL = __import__("training.utils", fromlist=["TransformLabel"]).TransformLabel
     rng = np.random.RandomState(0)
@@ -291,6 +312,7 @@ def test_transform_label_sequential(ref):
         assert np.array_equal(lut2[mid], want.numpy())
 
 
+@pytest.mark.reference
 @pytest.mark.parametrize("name,first_task", [("tiny", False), ("tiny", True), ("small", False)])
 def test_full_step_matches(ref, name, first_task):
     cfg = synth.CONFIGS[name]
