@@ -165,6 +165,16 @@ struct PixCoef {
   float cg0, cg1, cg2, d0, dy;
 };
 
+// Last lane of the run of consecutive lanes that holds this lane's `key`.  A segmented shfl_down tree reduction may
+// add lane + o's partial sum only when lane + o <= this lane: a key can come back after a different one (a warp's
+// pixels wrapping into the next image row meet the same low-res cell again), and that later run is flushed by its
+// own first lane.
+__device__ __forceinline__ int run_end_lane(int key, int lane) {
+  const int next = __shfl_down_sync(0xffffffffu, key, 1);
+  const unsigned ends = __ballot_sync(0xffffffffu, lane == 31 || next != key);
+  return __ffs(ends & (0xffffffffu << lane)) - 1;
+}
+
 // Binary focal loss of one seen-head logit Z with target t (smp FocalLoss(mode="binary"), base_loss.py:255-272):
 //   bce = softplus(Z) - t Z,  pt = exp(-bce) = sigmoid(+-Z),  term = (1-pt)^g * bce [* alpha weight]; dterm = d term / dZ
 __device__ __forceinline__ void focal_term(const bacs_pixel_args& a, float Z, float t, float& term, float& dterm) {

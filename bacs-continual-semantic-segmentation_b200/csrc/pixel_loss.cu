@@ -607,12 +607,12 @@ __global__ void __launch_bounds__(kConsumers + 32, ((KREG > 0 || PPT == 1) ? 2 :
           float c10 = gfoc[j] * wy1g[j] * (1.f - wx1[j]);
           float c11 = gfoc[j] * wy1g[j] * wx1[j];
           const int key = cell[j] * 4 + cdx[j] + 2 * (cell_dy[j] != 0);
+          const int run_end = run_end_lane(key, lane);
 #pragma unroll
           for (int o = 1; o < 32; o <<= 1) {
             const float n00 = __shfl_down_sync(full, c00, o), n01 = __shfl_down_sync(full, c01, o);
             const float n10 = __shfl_down_sync(full, c10, o), n11 = __shfl_down_sync(full, c11, o);
-            const int nk = __shfl_down_sync(full, key, o);
-            if (lane + o < 32 && nk == key) {
+            if (lane + o <= run_end) {
               c00 += n00; c01 += n01; c10 += n10; c11 += n11;
             }
           }

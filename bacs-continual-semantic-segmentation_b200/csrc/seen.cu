@@ -140,6 +140,9 @@ __global__ void __launch_bounds__(32 * kSeenWarps, (TMAX * PX <= 32 ? 3 : (TMAX 
       }
     }
   }
+  // this CTA is done with its channel table; the leader's xfer region below can overlap its table, so the pushes
+  // wait (barrier.cluster.wait before them) until every CTA of the cluster, the leader included, has arrived here
+  if (cs > 1) asm volatile("barrier.cluster.arrive.release.aligned;" ::: "memory");
   __syncthreads();
   // cross-warp reduction through shared memory: red[warp][t][pixel], then across the cluster
   float* red = smem;
@@ -157,6 +160,7 @@ __global__ void __launch_bounds__(32 * kSeenWarps, (TMAX * PX <= 32 ? 3 : (TMAX 
     uint32_t remote;
     const uint32_t local = (uint32_t)__cvta_generic_to_shared(xfer + (size_t)rank * n_out);
     asm volatile("mapa.shared::cluster.u32 %0, %1, %2;" : "=r"(remote) : "r"(local), "r"(0));
+    asm volatile("barrier.cluster.wait.acquire.aligned;" ::: "memory");
     if (rank != 0) {
       for (int e = tid; e < n_out; e += 32 * kSeenWarps) {
         float s = 0.f;
