@@ -934,29 +934,70 @@ static bool make_regs_plan(const bacs_pixel_args& a, StreamPlan* plan) {
 
 struct LowresPlan {
   int SX, R, groups, nsrc_max, grid;
+  bool exact;  // W == SX * lw: the instantiation with compile-time pixel offsets
   size_t smem, part_bytes, g32_bytes;
 };
 
-// host copy of lerp_half_pixel (fp32, op by op)
-static void host_half_pixel(int dst, int in_size, float scale, int* i0, int* i1) {
+// host copy of lerp_half_pixel's source coordinate (fp32, op by op)
+static float host_src(int dst, float scale) {
   volatile float t = (float)dst + 0.5f;
   volatile float m = scale * t;
   float src = m - 0.5f;
-  if (src < 0.f) src = 0.f;
-  *i0 = std::min((int)src, in_size - 1);
+  return src < 0.f ? 0.f : src;
+}
+
+// host copy of lerp_half_pixel
+static void host_half_pixel(int dst, int in_size, float scale, int* i0, int* i1) {
+  *i0 = std::min((int)host_src(dst, scale), in_size - 1);
   *i1 = *i0 + (*i0 < in_size - 1 ? 1 : 0);
 }
 
+// host copy of lowres_span_start (pixel_lowres.cuh)
+static int host_span_start(int j, int lw, int W, float scale) {
+  auto owner = [&](int x) {
+    volatile float h = host_src(x, scale) + 0.5f;
+    return (int)h;
+  };
+  if (j >= lw) return W;
+  int x = (int)((int64_t)j * W / lw);
+  while (x > 0 && owner(x - 1) >= j) --x;
+  while (x < W && owner(x) < j) ++x;
+  return x;
+}
+
+// Accepted geometry: W == SX * lw with SX 8 or 16 and H a multiple of lh, or the network's output stride s = 16 or 8
+// applied to any input, lh == ceil(H / s) and lw == ceil(W / s) (DeepLab's padded stride-2 convolutions; s = 16 where
+// both match).  The seen heads (a.z) need the first form.
 static bool make_lowres_plan(const bacs_pixel_args& a, int lh, int lw, LowresPlan* plan) {
-  if (lh <= 0 || lw <= 0 || lw > kLowresThreads || a.W % lw != 0 || a.H % lh != 0) return false;
-  const int SX = a.W / lw;
-  if (SX != 16 && SX != 8) return false;
-  if (a.K > 255) return false;
+  if (lh <= 0 || lw <= 0 || lw > kLowresThreads || a.K > 255) return false;
+  int SX = 0;
+  bool exact = false;
+  if (a.W % lw == 0 && a.H % lh == 0 && (a.W / lw == 16 || a.W / lw == 8)) {
+    SX = a.W / lw;
+    exact = true;
+  } else {
+    for (int s : {16, 8})
+      if (lh == (a.H + s - 1) / s && lw == (a.W + s - 1) / s) {
+        SX = s;
+        break;
+      }
+    if (SX == 0 || a.z) return false;
+    exact = a.W == SX * lw;  // whole spans in x; the kernel's rows take any H
+    if (!exact) {            // every column's span fits the kernel's SX-pixel arrays
+      const float hx = hp_scale(lw, a.W);
+      for (int j = 0, x0 = 0; j < lw; ++j) {
+        const int x1 = host_span_start(j + 1, lw, a.W, hx);
+        if (x1 - x0 > SX) return false;
+        x0 = x1;
+      }
+    }
+  }
   int R = 1;
   while (2 * R * lw <= kLowresThreads && 2 * R <= a.H) R *= 2;
   const float hy = hp_scale(lh, a.H);
   int groups, nsrc;
-  for (;; R /= 2) {  // a row group may touch at most kLowresMaxSrc source rows
+  size_t smem;
+  for (;; R /= 2) {  // a row group may touch at most kLowresMaxSrc source rows, and its staging must fit
     groups = (a.H + R - 1) / R;
     nsrc = 1;
     for (int g = 0; g < groups; ++g) {
@@ -965,18 +1006,20 @@ static bool make_lowres_plan(const bacs_pixel_args& a, int lh, int lw, LowresPla
       host_half_pixel(std::min(g * R + R, a.H) - 1, lh, hy, &l0, &l1);
       nsrc = std::max(nsrc, l1 - f0 + 1);
     }
-    if (nsrc <= kLowresMaxSrc || R == 1) break;
+    smem = ((size_t)nsrc * a.K * (lw + 2) + (size_t)3 * R * kLowresChunk * lw + (size_t)nsrc * R +
+            (a.z ? (size_t)R * a.T * a.w : 0) + (size_t)R * (a.w + 1)) * 4 + 16;
+    if ((nsrc <= kLowresMaxSrc && smem <= kLowresMaxSmem) || R == 1) break;
   }
   plan->SX = SX;
+  plan->exact = exact;
   plan->R = R;
   plan->groups = groups;
   plan->nsrc_max = nsrc;
   plan->grid = groups * a.B;
-  plan->smem = ((size_t)nsrc * a.K * (lw + 2) + (size_t)3 * R * kLowresChunk * lw + (size_t)nsrc * R +
-                (a.z ? (size_t)R * a.T * a.w : 0) + (size_t)R * (a.w + 1)) * 4 + 16;
+  plan->smem = smem;
   plan->part_bytes = align_up((size_t)plan->grid * BACS_NACC * sizeof(double), 256);
   plan->g32_bytes = (a.dlogits && a.dtype != BACS_F32) ? align_up((size_t)a.B * a.K * lh * lw * 4, 256) : 0;
-  return plan->smem <= (size_t)200 * 1024;
+  return plan->smem <= kLowresMaxSmem;
 }
 
 }  // namespace bacs
@@ -1013,8 +1056,10 @@ int bacs_pixel_loss_lowres(const bacs_pixel_args* a, int32_t lh, int32_t lw, voi
     BACS_REQUIRE(a->score && !a->dlogits, "bacs_pixel_loss_lowres: SCORE mode needs score and no gradient");
   LowresPlan plan;
   if (!make_lowres_plan(*a, lh, lw, &plan)) {
-    set_error("bacs_pixel_loss_lowres: unsupported geometry (H=%d W=%d lh=%d lw=%d K=%d): W/lw must be 8 or 16, "
-              "lw <= 256, K <= 255", a->H, a->W, lh, lw, a->K);
+    set_error("bacs_pixel_loss_lowres: unsupported geometry (H=%d W=%d lh=%d lw=%d K=%d%s): needs W == s*lw with "
+              "s = 8 or 16 and H a multiple of lh, or lh == ceil(H/s) and lw == ceil(W/s) for s = 8 or 16 (not with "
+              "the seen logits z); lw <= 256, K <= 255, staging within %zu bytes of shared memory",
+              a->H, a->W, lh, lw, a->K, a->z ? ", seen logits z given" : "", kLowresMaxSmem);
     return BACS_ERR_UNSUPPORTED;
   }
   if (!workspace || workspace_bytes < plan.part_bytes + plan.g32_bytes) {
@@ -1044,9 +1089,10 @@ int bacs_pixel_loss_lowres(const bacs_pixel_args* a, int32_t lh, int32_t lw, voi
   p.sy = a->z ? ac_scale(a->h, a->H) : 0.f;
   p.sx = a->z ? ac_scale(a->w, a->W) : 0.f;
   p.partials = reinterpret_cast<double*>(workspace);
-#define LAUNCH_LR(SXV)                                                                                          \
+  p.hx = hp_scale(lw, a->W);
+#define LAUNCH_LR(SXV, EXACT)                                                                                   \
   do {                                                                                                          \
-    auto kern = pixel_lowres_kernel<SXV>;                                                                       \
+    auto kern = pixel_lowres_kernel<SXV, EXACT>;                                                                \
     if (plan.smem > 48 * 1024 &&                                                                                \
         cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)plan.smem) != cudaSuccess) { \
       set_error("bacs_pixel_loss_lowres: cannot opt in to %zu bytes of shared memory", plan.smem);              \
@@ -1054,8 +1100,13 @@ int bacs_pixel_loss_lowres(const bacs_pixel_args* a, int32_t lh, int32_t lw, voi
     }                                                                                                           \
     kern<<<plan.grid, kLowresThreads, plan.smem, s>>>(p);                                                       \
   } while (0)
-  if (plan.SX == 16) LAUNCH_LR(16);
-  else LAUNCH_LR(8);
+  if (plan.exact) {
+    if (plan.SX == 16) LAUNCH_LR(16, true);
+    else LAUNCH_LR(8, true);
+  } else {
+    if (plan.SX == 16) LAUNCH_LR(16, false);
+    else LAUNCH_LR(8, false);
+  }
 #undef LAUNCH_LR
   BACS_CHECK_LAUNCH("bacs_pixel_loss_lowres");
   if (a->dlogits && a->dtype != BACS_F32) {

@@ -12,8 +12,11 @@
 // Work split: a thread owns the SX = W/lw consecutive pixels [SX*j, SX*j+SX) of one image row.  Inside that span the
 // up-sampled logit of channel c is  v_j + s_i * D  with s_i = (i+0.5)/SX - 0.5 and D = v_j - v_{j-1} (left half,
 // s_i < 0) or v_{j+1} - v_j (right half) -- v_* are the low-res columns interpolated in y for this row, columns
-// clamped at the image border exactly like ATen's half-pixel rule.  The channel loop is the OUTER loop (any K, no
-// shared-memory logit tile): pass 1a max / arg-max, pass 1b exponent sums, per-pixel terms, pass 2 gradients, which
+// clamped at the image border exactly like ATen's half-pixel rule.  Any other width (EXACT = false: lw = ceil(W / SX),
+// what a backbone with padded stride-2 convolutions returns for an input that is not a multiple of its output
+// stride): thread j owns the pixels whose half-pixel source column rounds to j, at most SX of them; s_i = src_x - j
+// is a runtime per-pixel value and pixels past the span are predicated off.  The channel loop is the OUTER loop (any
+// K, no shared-memory logit tile): pass 1a max / arg-max, pass 1b exponent sums, per-pixel terms, pass 2 gradients, which
 // are reduced over the SX pixels in registers (sum g, sum s_i g per half) before they touch memory: three plain
 // shared-memory stores per (thread, channel); after every chunk of 8 channels the CTA sums its rows with their
 // y-weights and sends one global fp32 RED per low-res cell (shared-memory fp32 atomics are CAS loops on sm_100).
@@ -27,7 +30,7 @@ namespace bacs {
 struct alignas(16) LowresParams {
   bacs_pixel_args a;     // logits = sem_logits [B,K,lh,lw]; dlogits unused by the kernel (see g32)
   float* g32;            // [B,K,lh,lw] fp32 gradient accumulator (zeroed by the caller) or nullptr
-  int lh, lw;            // low-res logit size; W == lw * SX, H == lh * (H / lh)
+  int lh, lw;            // low-res logit size; W == lw * SX (EXACT) or lw == ceil(W / SX)
   int R;                 // image rows per CTA (R * lw <= 256 threads)
   int groups_per_image;  // ceil(H / R)
   int nsrc_max;          // source rows staged per CTA (shared-memory sizing)
@@ -35,13 +38,31 @@ struct alignas(16) LowresParams {
   float inv_n;           // 1 / (B*H*W)
   float sy, sx;          // align_corners=True scales of the seen heads
   double* partials;      // [grid, BACS_NACC]
+  float hx;              // half-pixel scale lw / W (EXACT = false)
 };
 
 constexpr int kLowresThreads = 256;
 constexpr int kLowresChunk = 8;   // channels per gradient-reduction round
 constexpr int kLowresMaxSrc = 8;  // source rows a row group may touch (the host halves R until it holds)
+constexpr size_t kLowresMaxSmem = (size_t)200 * 1024;  // dynamic shared memory of one CTA (two CTAs per SM)
 
-template <int SX>
+// half-pixel source column of output pixel x (lerp_half_pixel's src, op by op) and the column it rounds to
+__device__ __forceinline__ float lowres_src(int x, float scale) {
+  const float s = __fsub_rn(__fmul_rn(scale, __fadd_rn((float)x, 0.5f)), 0.5f);
+  return s < 0.f ? 0.f : s;
+}
+__device__ __forceinline__ int lowres_owner(int x, float scale) { return (int)__fadd_rn(lowres_src(x, scale), 0.5f); }
+// first pixel of column j's span (W for j == lw).  The owner is monotone in x, so the spans [start(j), start(j+1))
+// cover the row once; host_span_start (pixel_loss.cu) is the host copy the plan checks the span lengths with.
+__device__ __forceinline__ int lowres_span_start(int j, int lw, int W, float scale) {
+  if (j >= lw) return W;
+  int x = (int)((int64_t)j * W / lw);
+  while (x > 0 && lowres_owner(x - 1, scale) >= j) --x;
+  while (x < W && lowres_owner(x, scale) < j) ++x;
+  return x;
+}
+
+template <int SX, bool EXACT>
 __global__ void __launch_bounds__(kLowresThreads, 2) pixel_lowres_kernel(const __grid_constant__ LowresParams p) {
   extern __shared__ __align__(16) unsigned char lr_smem[];
   __shared__ float red_scratch[kLowresThreads / 32][BACS_NACC];
@@ -130,7 +151,17 @@ __global__ void __launch_bounds__(kLowresThreads, 2) pixel_lowres_kernel(const _
   const int r = tid / lw, j = tid - r * lw;
   const bool active = r < rows;
   constexpr float kInvSX = 1.f / (float)SX;
-#define BACS_LR_S(i) (((float)(i) + 0.5f) * kInvSX - 0.5f)
+  // the thread's pixels of its image row: [xs, xs + npx); sxr[i] = src_x - j of pixel i (0 past the span)
+  int xs = SX * j, npx = SX;
+  float sxr[SX];
+  if constexpr (!EXACT) {
+    xs = lowres_span_start(j, lw, a.W, p.hx);
+    npx = lowres_span_start(j + 1, lw, a.W, p.hx) - xs;
+#pragma unroll
+    for (int i = 0; i < SX; ++i) sxr[i] = i < npx ? lowres_src(xs + i, p.hx) - (float)j : 0.f;
+  }
+#define BACS_LR_S(i) (EXACT ? (((float)(i) + 0.5f) * kInvSX - 0.5f) : sxr[i])
+#define BACS_LR_LEFT(i) (EXACT ? (i) < SX / 2 : sxr[i] < 0.f)
 
   // per-thread state that lives from the forward passes to the gradient pass
   F2 nm2[SX / 2], cg1p[SX / 2], cg2p[SX / 2];  // pixel pairs (2i, 2i+1) as packed fp32 (FFMA2 / FMUL2 / FADD2)
@@ -158,10 +189,30 @@ __global__ void __launch_bounds__(kLowresThreads, 2) pixel_lowres_kernel(const _
     wy0 = 1.f - ly.w1;
     s0 = src + (size_t)(ly.i0 - base) * K * LWP + j;  // columns j-1, j, j+1 at [0], [1], [2]
     s1 = src + (size_t)(ly.i1 - base) * K * LWP + j;
-    const int64_t pix0 = (int64_t)b * HW + (int64_t)Y * a.W + (int64_t)SX * j;
+    const int64_t pix0 = (int64_t)b * HW + (int64_t)Y * a.W + (EXACT ? (int64_t)SX * j : (int64_t)xs);
 
     // ---- labels: SX int64 -> one byte each (255 = ignored / invalid) ----------------------------------------------
-    {
+    if constexpr (!EXACT) {  // scalar loads; pixels past the span read as ignored
+      const int64_t* lp = a.labels + pix0;
+#pragma unroll
+      for (int q = 0; q < SX / 4; ++q) ypk[q] = 0;
+#pragma unroll
+      for (int i = 0; i < SX; ++i) {
+        uint32_t y8 = 255u;
+        if (i < npx) {
+          const long long l = __ldg(lp + i);
+          if (l == a.ignore_index) {
+          } else if (l >= 0 && l < K) {
+            y8 = (uint32_t)l;
+            ymin = min(ymin, (int)l);
+            ymax = max(ymax, (int)l);
+          } else {
+            acc[BACS_ACC_INVALID] += 1.f;
+          }
+        }
+        ypk[i >> 2] |= y8 << (8 * (i & 3));
+      }
+    } else {
       const int64_t* lp = a.labels + pix0;
 #pragma unroll
       for (int q = 0; q < SX / 4; ++q) ypk[q] = 0;
@@ -198,8 +249,8 @@ __global__ void __launch_bounds__(kLowresThreads, 2) pixel_lowres_kernel(const _
     // (x16 align_corners=True: the thread's SX pixels touch the low-res columns cb, cb+1, cb+2 only)
     float Lseen[SX], Lzf[SX], Lwx1[SX];
     uint32_t fdm = 0;  // bit i: pixel i's left tap is column cb+1 (else cb); its right tap is the next column, clamped
-    const int cb = a.z ? lerp_align_corners(SX * j, a.w, p.sx).i0 : 0;
-    if (a.z) {
+    const int cb = (EXACT && a.z) ? lerp_align_corners(SX * j, a.w, p.sx).i0 : 0;
+    if (EXACT && a.z) {  // (the plan accepts the seen logits at the exact geometry only)
       float wx1[SX], zmx[SX], zf[SX];
 #pragma unroll
       for (int i = 0; i < SX; ++i) {
@@ -248,7 +299,7 @@ __global__ void __launch_bounds__(kLowresThreads, 2) pixel_lowres_kernel(const _
         trio(c, vj, dl, dr);
 #pragma unroll
         for (int i = 0; i < SX; ++i) {
-          const float x = fmaf(BACS_LR_S(i), i < SX / 2 ? dl : dr, vj);
+          const float x = fmaf(BACS_LR_S(i), BACS_LR_LEFT(i) ? dl : dr, vj);
           if (x > mx[i]) {
             mx[i] = x;
             am[i] = c;
@@ -257,13 +308,14 @@ __global__ void __launch_bounds__(kLowresThreads, 2) pixel_lowres_kernel(const _
       }
       if (a.preds) {
         int64_t* out = a.preds + pix0;
-        if ((reinterpret_cast<uintptr_t>(out) & 15) == 0) {
+        if (EXACT && (reinterpret_cast<uintptr_t>(out) & 15) == 0) {
 #pragma unroll
           for (int i = 0; i < SX; i += 2)
             *reinterpret_cast<longlong2*>(out + i) = make_longlong2((long long)am[i], (long long)am[i + 1]);
         } else {
 #pragma unroll
-          for (int i = 0; i < SX; ++i) out[i] = am[i];
+          for (int i = 0; i < SX; ++i)
+            if (EXACT || i < npx) out[i] = am[i];
         }
       }
     }
@@ -279,8 +331,8 @@ __global__ void __launch_bounds__(kLowresThreads, 2) pixel_lowres_kernel(const _
     // exp2((v_j + s_i D) log2e - max log2e) of one pixel pair
     // (the two up-sampled logits come from scalar FFMAs with immediate s_i -- a packed FFMA2 would need the constant
     // pair in registers, re-materialised per channel -- and are identical to the values of pass 1a)
-    auto exp_pair = [&](int ip, float s_lo, float s_hi, float side, float vj) {
-      const F2 arg = fma2(f2(fmaf(s_lo, side, vj), fmaf(s_hi, side, vj)), l2e2, nm2[ip]);
+    auto exp_pair = [&](int ip, float s_lo, float s_hi, float side_lo, float side_hi, float vj) {
+      const F2 arg = fma2(f2(fmaf(s_lo, side_lo, vj), fmaf(s_hi, side_hi, vj)), l2e2, nm2[ip]);
       return f2(ex2_fast(f2lo(arg)), ex2_fast(f2hi(arg)));
     };
 #pragma unroll 1
@@ -289,7 +341,8 @@ __global__ void __launch_bounds__(kLowresThreads, 2) pixel_lowres_kernel(const _
       trio(c, vj, dl, dr);
 #pragma unroll
       for (int ip = 0; ip < SX / 2; ++ip)
-        so2[ip] = add2(so2[ip], exp_pair(ip, BACS_LR_S(2 * ip), BACS_LR_S(2 * ip + 1), ip < SX / 4 ? dl : dr, vj));
+        so2[ip] = add2(so2[ip], exp_pair(ip, BACS_LR_S(2 * ip), BACS_LR_S(2 * ip + 1), BACS_LR_LEFT(2 * ip) ? dl : dr,
+                                       BACS_LR_LEFT(2 * ip + 1) ? dl : dr, vj));
     }
 #pragma unroll 1
     for (int c = max(old_cl, 1); c < K; ++c) {
@@ -297,17 +350,22 @@ __global__ void __launch_bounds__(kLowresThreads, 2) pixel_lowres_kernel(const _
       trio(c, vj, dl, dr);
 #pragma unroll
       for (int ip = 0; ip < SX / 2; ++ip)
-        sn2[ip] = add2(sn2[ip], exp_pair(ip, BACS_LR_S(2 * ip), BACS_LR_S(2 * ip + 1), ip < SX / 4 ? dl : dr, vj));
+        sn2[ip] = add2(sn2[ip], exp_pair(ip, BACS_LR_S(2 * ip), BACS_LR_S(2 * ip + 1), BACS_LR_LEFT(2 * ip) ? dl : dr,
+                                       BACS_LR_LEFT(2 * ip + 1) ? dl : dr, vj));
     }
 
     // ---- per-pixel terms: a rolled loop over dynamically indexed copies (local memory, L1) --------------------------
-    float Lmx[SX], Lso[SX], Lsn[SX], Lcg1[SX], Lcg2[SX];
+    float Lmx[SX], Lso[SX], Lsn[SX], Lcg1[SX], Lcg2[SX], Lsx[SX];
     uint32_t Ly[SX / 4];
 #pragma unroll
     for (int i = 0; i < SX; ++i) {
       Lmx[i] = mx[i];
       Lso[i] = (i & 1) ? f2hi(so2[i >> 1]) : f2lo(so2[i >> 1]);
       Lsn[i] = (i & 1) ? f2hi(sn2[i >> 1]) : f2lo(sn2[i >> 1]);
+      if constexpr (!EXACT) {
+        Lsx[i] = sxr[i];
+        Lcg1[i] = Lcg2[i] = 0.f;  // pixels past the span: no gradient in pass 2
+      }
     }
 #pragma unroll
     for (int q = 0; q < SX / 4; ++q) Ly[q] = ypk[q];
@@ -316,9 +374,9 @@ __global__ void __launch_bounds__(kLowresThreads, 2) pixel_lowres_kernel(const _
     float fa0 = 0.f, fa1 = 0.f, fa2 = 0.f;                              // focal gradient at columns cb, cb+1, cb+2
     uint32_t mbits = 0;
 #pragma unroll 1
-    for (int i = 0; i < SX; ++i) {
-      const bool left = i < SX / 2;
-      const float sI = ((float)i + 0.5f) * kInvSX - 0.5f;
+    for (int i = 0; i < (EXACT ? SX : npx); ++i) {
+      const float sI = EXACT ? ((float)i + 0.5f) * kInvSX - 0.5f : Lsx[i];
+      const bool left = EXACT ? i < SX / 2 : sI < 0.f;
       const uint32_t y8 = (Ly[i >> 2] >> (8 * (i & 3))) & 255u;
       const bool is_ign = y8 == 255u;
       const int y = is_ign ? -1 : (int)y8;
@@ -337,7 +395,7 @@ __global__ void __launch_bounds__(kLowresThreads, 2) pixel_lowres_kernel(const _
       }
       float seen = 0.f, zfoc = 0.f, wx1 = 0.f;
       int fd = 0, fhi = 0;
-      if (a.z) {
+      if (EXACT && a.z) {
         seen = Lseen[i];
         zfoc = Lzf[i];
         wx1 = Lwx1[i];
@@ -357,7 +415,7 @@ __global__ void __launch_bounds__(kLowresThreads, 2) pixel_lowres_kernel(const _
       G0 += g0;
       if (left) GL0 = fmaf(sI, g0, GL0);
       else GR0 = fmaf(sI, g0, GR0);
-      if (a.gz && gfoc != 0.f) {
+      if (EXACT && a.gz && gfoc != 0.f) {
         const float c_lo = gfoc * (1.f - wx1), c_hi = gfoc * wx1;
         fa0 += (fd == 0 ? c_lo : 0.f) + (fhi == 0 ? c_hi : 0.f);
         fa1 += (fd == 1 ? c_lo : 0.f) + (fhi == 1 ? c_hi : 0.f);
@@ -369,7 +427,7 @@ __global__ void __launch_bounds__(kLowresThreads, 2) pixel_lowres_kernel(const _
       cg1p[ip] = f2(Lcg1[2 * ip], Lcg1[2 * ip + 1]);
       cg2p[ip] = f2(Lcg2[2 * ip], Lcg2[2 * ip + 1]);
     }
-    if (a.gz) {
+    if (EXACT && a.gz) {
       float* grow = gacc + (size_t)r * (a.w + 1) + cb;
       if (fa0 != 0.f) atomicAdd(grow, fa0);
       if (fa1 != 0.f) atomicAdd(grow + 1, fa1);
@@ -383,12 +441,13 @@ __global__ void __launch_bounds__(kLowresThreads, 2) pixel_lowres_kernel(const _
         const uint32_t nib = (mbits >> (4 * q)) & 15u;
         mpk[q] = (nib & 1u) | ((nib & 2u) << 7) | ((nib & 4u) << 14) | ((nib & 8u) << 21);
       }
-      if ((reinterpret_cast<uintptr_t>(out) & (SX - 1)) == 0) {
+      if (EXACT && (reinterpret_cast<uintptr_t>(out) & (SX - 1)) == 0) {
         if (SX == 16) *reinterpret_cast<uint4*>(out) = make_uint4(mpk[0], mpk[1], mpk[2 % (SX / 4)], mpk[3 % (SX / 4)]);
         else *reinterpret_cast<uint2*>(out) = make_uint2(mpk[0], mpk[1]);
       } else {
 #pragma unroll
-        for (int i = 0; i < SX; ++i) out[i] = (uint8_t)((mbits >> i) & 1u);
+        for (int i = 0; i < SX; ++i)
+          if (EXACT || i < npx) out[i] = (uint8_t)((mbits >> i) & 1u);
       }
     }
   }
@@ -411,19 +470,16 @@ __global__ void __launch_bounds__(kLowresThreads, 2) pixel_lowres_kernel(const _
             float GLa = 0.f, GLb = 0.f, GRa = 0.f, GRb = 0.f;
 #pragma unroll
             for (int ip = 0; ip < SX / 2; ++ip) {
-              const float side = ip < SX / 4 ? dl : dr;
-              const F2 arg = fma2(f2(fmaf(BACS_LR_S(2 * ip), side, vj), fmaf(BACS_LR_S(2 * ip + 1), side, vj)), l2e2,
-                                  nm2[ip]);
+              const bool lo_left = BACS_LR_LEFT(2 * ip), hi_left = BACS_LR_LEFT(2 * ip + 1);
+              const F2 arg = fma2(f2(fmaf(BACS_LR_S(2 * ip), lo_left ? dl : dr, vj),
+                                     fmaf(BACS_LR_S(2 * ip + 1), hi_left ? dl : dr, vj)), l2e2, nm2[ip]);
               const F2 e2 = f2(ex2_fast(f2lo(arg)), ex2_fast(f2hi(arg)));
               const F2 g2 = mul2(e2, is_old ? cg1p[ip] : cg2p[ip]);
               G2 = add2(G2, g2);
-              if (ip < SX / 4) {
-                GLa = fmaf(BACS_LR_S(2 * ip), f2lo(g2), GLa);
-                GLb = fmaf(BACS_LR_S(2 * ip + 1), f2hi(g2), GLb);
-              } else {
-                GRa = fmaf(BACS_LR_S(2 * ip), f2lo(g2), GRa);
-                GRb = fmaf(BACS_LR_S(2 * ip + 1), f2hi(g2), GRb);
-              }
+              if (lo_left) GLa = fmaf(BACS_LR_S(2 * ip), f2lo(g2), GLa);
+              else GRa = fmaf(BACS_LR_S(2 * ip), f2lo(g2), GRa);
+              if (hi_left) GLb = fmaf(BACS_LR_S(2 * ip + 1), f2hi(g2), GLb);
+              else GRb = fmaf(BACS_LR_S(2 * ip + 1), f2hi(g2), GRb);
             }
             G = f2lo(G2) + f2hi(G2);
             GL = GLa + GLb;
@@ -437,7 +493,7 @@ __global__ void __launch_bounds__(kLowresThreads, 2) pixel_lowres_kernel(const _
               for (int i = 0; i < SX; ++i) {
                 if (((ypk[i >> 2] >> (8 * (i & 3))) & 255u) == (uint32_t)c) {
                   G -= dy;
-                  if (i < SX / 2) GL = fmaf(BACS_LR_S(i), -dy, GL);
+                  if (BACS_LR_LEFT(i)) GL = fmaf(BACS_LR_S(i), -dy, GL);
                   else GR = fmaf(BACS_LR_S(i), -dy, GR);
                 }
               }
@@ -500,6 +556,7 @@ __global__ void __launch_bounds__(kLowresThreads, 2) pixel_lowres_kernel(const _
     }
   }
 #undef BACS_LR_S
+#undef BACS_LR_LEFT
   __syncthreads();
 
   if (a.gz) {

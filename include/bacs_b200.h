@@ -257,7 +257,11 @@ int bacs_pixel_loss(const bacs_pixel_args* args_host, void* workspace, size_t wo
  * [B,K,H,W] logit or gradient tensor exists.  Arguments as bacs_pixel_loss except
  *   args->logits  = sem_logits [B,K,lh,lw]   (model(x, return_sem_logits=True), deeplab_v3.py:155-156)
  *   args->dlogits = d loss / d sem_logits [B,K,lh,lw], same dtype (or NULL)
- *   args->H, W    = label resolution; W / lw must be 8 or 16, H a multiple of lh, lw <= 256, K <= 255.
+ *   args->H, W    = label resolution: W == s * lw with s = 8 or 16 and H a multiple of lh, or, for an input of any
+ *                   size, lh == ceil(H / s) and lw == ceil(W / s) with s = 8 or 16 (the network's output stride);
+ *                   lw <= 256, K <= 255.  The seen logits args->z (focal term, WEIGHTED_CE's seen probabilities)
+ *                   need the first form, i.e. inputs that are multiples of 16 at seen_scale 16; args->seen_max
+ *                   works with both.  An unsupported geometry returns BACS_ERR_UNSUPPORTED (workspace size 0).
  * Workspace: bacs_pixel_lowres_workspace_bytes.  Asynchronous on `stream`; gradients are accumulated with fp32
  * atomics (summation order is not fixed: results agree to fp32 rounding, not bit for bit, between runs). */
 size_t bacs_pixel_lowres_workspace_bytes(const bacs_pixel_args* args_host, int32_t lh, int32_t lw);
