@@ -313,9 +313,26 @@ __device__ __forceinline__ float label_dy(const bacs_pixel_args& a, float inv_n,
 }
 
 struct PixelPlan {
-  int ppt, P, kreg, stages, grid, rowtile, fast, coop;
+  int ppt, P, kreg, stages, grid, rowtile, coop;
   size_t smem;
 };
+
+// Launches a pixel kernel with `smem` bytes of dynamic shared memory, opted in when above the 48 KB default; through
+// launch_pdl() when `pdl`.  `fn` (the entry point) starts the error message.
+template <typename... KArgs, typename... Args>
+static inline int launch_pixel_kernel(const char* fn, bool pdl, void (*kern)(KArgs...), dim3 grid, dim3 block,
+                                      size_t smem, cudaStream_t s, Args... args) {
+  if (smem > 48 * 1024) {
+    const cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    if (e != cudaSuccess) {
+      set_error("%s: cannot opt in to %zu bytes of shared memory: %s", fn, smem, cudaGetErrorString(e));
+      return BACS_ERR_CUDA;
+    }
+  }
+  if (pdl) launch_pdl(kern, grid, block, smem, s, args...);
+  else kern<<<grid, block, smem, s>>>(static_cast<KArgs>(args)...);
+  return BACS_OK;
+}
 
 // launchers of the register-resident fast path, one translation unit per storage type
 int launch_pixel_fast_f32(const PixelParams& p, const PixelPlan& plan, cudaStream_t s);

@@ -587,16 +587,8 @@ __global__ void __launch_bounds__(kFastThreads, 2) pixel_fast_kernel(const __gri
 
 template <typename T, int KREG, bool ROWTILE>
 static int launch_fast_one(const PixelParams& p, const PixelPlan& plan, cudaStream_t s) {
-  auto kern = pixel_fast_kernel<T, KREG, ROWTILE>;
-  if (plan.smem > 48 * 1024) {
-    cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)plan.smem);
-    if (e != cudaSuccess) {
-      set_error("bacs_pixel_loss: cannot opt in to %zu bytes of shared memory: %s", plan.smem, cudaGetErrorString(e));
-      return BACS_ERR_CUDA;
-    }
-  }
-  kern<<<plan.grid, kFastThreads, plan.smem, s>>>(p);
-  return BACS_OK;
+  return launch_pixel_kernel("bacs_pixel_loss", false, pixel_fast_kernel<T, KREG, ROWTILE>, dim3(plan.grid),
+                             dim3(kFastThreads), plan.smem, s, p);
 }
 
 template <typename T>

@@ -30,8 +30,8 @@ namespace bacs {
 // channel loops together on their two adjacent pixels as PACKED pairs, each taking every other channel, and
 // exchange max / arg-max / sums / coefficients by shuffle.  Rows are 64 bytes longer than P elements so that the
 // two halves of a warp (rows c and c+1) hit disjoint banks.
-template <typename T, int PPT, int KREG, bool ROWTILE, bool COOP = false>
-__global__ void __launch_bounds__(kConsumers + 32, ((KREG > 0 || PPT == 1) ? 2 : 1)) pixel_loss_kernel(const PixelParams p) {
+template <typename T, int PPT, bool ROWTILE, bool COOP = false>
+__global__ void __launch_bounds__(kConsumers + 32, PPT == 1 ? 2 : 1) pixel_loss_kernel(const PixelParams p) {
   extern __shared__ __align__(128) unsigned char smem_raw[];
   __shared__ uint64_t bar_full[kMaxStages];  // producer -> consumers: tile landed
   __shared__ uint64_t bar_done[kMaxStages];  // consumers -> producer: gradients written; store / refill the stage
@@ -48,6 +48,13 @@ __global__ void __launch_bounds__(kConsumers + 32, ((KREG > 0 || PPT == 1) ? 2 :
   float* zr = reinterpret_cast<float*>(smem_raw + ((S * tile_elems * sizeof(T) + 15) / 16) * 16);
   float* gacc = zr + (ROWTILE ? a.T * a.w : 0);
   const int my_tiles = (p.n_tiles - (int)blockIdx.x + (int)gridDim.x - 1) / (int)gridDim.x;
+  // k-th tile of this CTA: image b, first pixel p0, npx pixels
+  auto tile_geom = [&](int k, int& b, int64_t& p0, int& npx) {
+    const int tile = (int)blockIdx.x + k * (int)gridDim.x;
+    b = tile / p.tiles_per_image;
+    p0 = (int64_t)(tile - b * p.tiles_per_image) * P;
+    npx = (int)min((int64_t)P, HW - p0);
+  };
 
   if (tid == 0) {
     for (int s = 0; s < S; ++s) {
@@ -74,12 +81,6 @@ __global__ void __launch_bounds__(kConsumers + 32, ((KREG > 0 || PPT == 1) ? 2 :
   // =====================================================================================
   if (tid >= kConsumers) {
     const int lane = tid - kConsumers;
-    auto tile_geom = [&](int k, int& b, int64_t& p0, int& npx) {
-      const int tile = (int)blockIdx.x + k * (int)gridDim.x;
-      b = tile / p.tiles_per_image;
-      p0 = (int64_t)(tile - b * p.tiles_per_image) * P;
-      npx = (int)min((int64_t)P, HW - p0);
-    };
     auto load_tile = [&](int k) {
       int b, npx;
       int64_t p0;
@@ -141,12 +142,6 @@ __global__ void __launch_bounds__(kConsumers + 32, ((KREG > 0 || PPT == 1) ? 2 :
 #pragma unroll
   for (int i = 0; i < BACS_NACC; ++i) acc[i] = 0.f;
 
-  auto tile_geom = [&](int k, int& b, int64_t& p0, int& npx) {
-    const int tile = (int)blockIdx.x + k * (int)gridDim.x;
-    b = tile / p.tiles_per_image;
-    p0 = (int64_t)(tile - b * p.tiles_per_image) * P;
-    npx = (int)min((int64_t)P, HW - p0);
-  };
   auto load_labels = [&](int k, int64_t* lab) {
     int b, npx;
     int64_t p0;
@@ -289,67 +284,7 @@ __global__ void __launch_bounds__(kConsumers + 32, ((KREG > 0 || PPT == 1) ? 2 :
         xy[j] = (y[j] >= 0) ? DT<T>::to_f(col[(size_t)y[j] * PITCH + j]) : 0.f;
         x0[j] = DT<T>::to_f(col[j]);
       }
-      if (KREG > 0) {
-        // ---------------- register-resident path (K <= KREG) ----------------
-        constexpr int KR = KREG > 0 ? KREG : 1;
-        float e[KR][PPT];
-        float mx[PPT], nm[PPT], s_all[PPT], s_old[PPT], s_fg[PPT];
-#pragma unroll
-        for (int c = 0; c < KR; ++c)
-          if (c < K) Vec<T, PPT>::ld(col + (size_t)c * P, e[c]);
-#pragma unroll
-        for (int j = 0; j < PPT; ++j) mx[j] = e[0][j];
-#pragma unroll
-        for (int c = 1; c < KR; ++c)
-          if (c < K) {
-#pragma unroll
-            for (int j = 0; j < PPT; ++j)
-              if (e[c][j] > mx[j]) {
-                mx[j] = e[c][j];
-                amax[j] = c;
-              }
-          }
-#pragma unroll
-        for (int j = 0; j < PPT; ++j) {
-          nm[j] = -mx[j] * kLog2e;
-          s_fg[j] = s_old[j] = 0.f;
-        }
-        // the foreground sum is accumulated without channel 0 (S - e_0 would cancel when the background dominates)
-#pragma unroll
-        for (int c = 0; c < KR; ++c)
-          if (c < K) {
-#pragma unroll
-            for (int j = 0; j < PPT; ++j) {
-              e[c][j] = ex2_fast(fmaf(e[c][j], kLog2e, nm[j]));
-              if (c >= 1) {
-                s_fg[j] += e[c][j];
-                if (c < old_cl) s_old[j] += e[c][j];
-              }
-            }
-          }
-#pragma unroll
-        for (int j = 0; j < PPT; ++j) {
-          s_all[j] = s_fg[j] + e[0][j];
-          if (old_cl >= 1) s_old[j] += e[0][j];
-          pixel_terms(a, p.inv_n, s_norm, old_cl, y[j], is_ign[j], mx[j], s_all[j], s_old[j], s_fg[j], e[0][j], x0[j],
-                      xy[j], seen[j], have_seen, zfoc[j], acc, pc[j], gfoc[j], dmask[j]);
-        }
-        if (a.dlogits) {
-          float g[PPT];
-#pragma unroll
-          for (int c = 0; c < KR; ++c)
-            if (c < K) {
-#pragma unroll
-              for (int j = 0; j < PPT; ++j) {
-                const float cg = c == 0 ? pc[j].cg0 : (c < old_cl ? pc[j].cg1 : pc[j].cg2);
-                g[j] = e[c][j] * cg;
-                if (c == 0) g[j] -= pc[j].d0;
-                if (c == y[j]) g[j] -= pc[j].dy;
-              }
-              Vec<T, PPT>::st(col + (size_t)c * PITCH, g);
-            }
-        }
-      } else if constexpr (COOP) {
+      if constexpr (COOP) {
         // ---------------- cooperative packed path (large K) ----------------
         static_assert(!COOP || PPT == 1, "one pixel per thread");
         const unsigned full = live_mask;
@@ -776,7 +711,9 @@ static bool make_z_map(CUtensorMap* map, const float* z, int B, int T, int h, in
             CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
 }
 
-static bool make_plan(const bacs_pixel_args& a, PixelPlan* plan) {
+// Plan of the shared-memory tile kernels.  Returns the variant: 2 the training-step kernel, 1 the K <= 24 register
+// kernel, 0 the generic tile kernel, -1 when K fits no shared-memory tile.
+static int make_plan(const bacs_pixel_args& a, PixelPlan* plan) {
   const size_t es = dtype_size(a.dtype);
   const int64_t HW = (int64_t)a.H * a.W;
   const int sms = sm_count();
@@ -805,7 +742,8 @@ static bool make_plan(const bacs_pixel_args& a, PixelPlan* plan) {
                          (reinterpret_cast<uintptr_t>(a.z) & 15) == 0;
     // 228 KB of shared memory per SM, 1 KB reserved per resident CTA, < 0.5 KB static
     auto two_fit = [](size_t smem) { return 2 * (smem + 1024 + 512) <= (size_t)228 * 1024; };
-    // the training-step kernel also runs with a 3-stage ring when that is what lets two CTAs share an SM
+    // the training-step kernel (needs the tensor maps); it also runs with a 3-stage ring when that is what lets two
+    // CTAs share an SM
     const bool wce = rowtile && a.mode == BACS_PIX_WEIGHTED_CE && !a.seen_max && encode_tiled_fn() != nullptr &&
                      a.w <= 256 && a.T <= 256 && a.K <= 256;
     int stages = 4;
@@ -814,7 +752,6 @@ static bool make_plan(const bacs_pixel_args& a, PixelPlan* plan) {
     if (smem + 1024 <= cap) {
       const int per_sm = two_fit(smem) ? 2 : 1;
       const int64_t tiles = HW / 512 * a.B;
-      plan->fast = 1;
       plan->coop = 0;
       plan->ppt = 2;
       plan->P = 512;
@@ -823,12 +760,11 @@ static bool make_plan(const bacs_pixel_args& a, PixelPlan* plan) {
       plan->smem = smem;
       plan->grid = (int)std::min<int64_t>(tiles, (int64_t)sms * per_sm);
       plan->rowtile = rowtile ? 1 : 0;
-      return true;
+      return wce ? 2 : 1;
     }
   }
 
   // ---- generic path: any K that fits a shared-memory tile, ragged / unaligned shapes ----
-  plan->fast = 0;
   plan->kreg = 0;
   for (int min_stages = 2; min_stages >= 1; --min_stages)
     for (int ppt = 2; ppt >= 1; --ppt) {
@@ -866,9 +802,9 @@ static bool make_plan(const bacs_pixel_args& a, PixelPlan* plan) {
       plan->smem = smem;
       plan->grid = (int)std::min<int64_t>(tiles, (int64_t)sms * per_sm);
       plan->rowtile = (a.z != nullptr && P <= a.W && a.W % P == 0) ? 1 : 0;
-      return true;
+      return 0;
     }
-  return false;
+  return -1;
 }
 
 }  // namespace bacs
@@ -886,7 +822,6 @@ struct StreamPlan {
 
 // K >= 64 on 16-byte aligned, vector-divisible images (everything else stays on the tile kernel)
 static bool make_stream_plan(const bacs_pixel_args& a, StreamPlan* plan) {
-  if (getenv("BACS_NO_STREAM")) return false;
   const int64_t HW = (int64_t)a.H * a.W;
   const int n = a.dtype == BACS_F32 ? 4 : 8;
   auto al = [](const void* p, uintptr_t m) { return (reinterpret_cast<uintptr_t>(p) & (m - 1)) == 0; };
@@ -904,29 +839,19 @@ static bool make_stream_plan(const bacs_pixel_args& a, StreamPlan* plan) {
   return true;
 }
 
-// tile shape of the register-column kernel: 256 threads x 2 CTAs per SM, or (BACS_REGS_CFG=128) 128 threads x 3
-static int regs_threads() {
-  const char* e = getenv("BACS_REGS_CFG");
-  return (e && atoi(e) == 256) ? 256 : 128;
-}
-static int regs_ctas(int nt) {
-  const char* e = getenv("BACS_REGS_CTAS");
-  return nt == 256 ? 2 : ((e && atoi(e) == 3) ? 3 : 4);
-}
-
-// 16-bit logits with 64 <= K <= kRegsKMax on whole 256-pixel tiles: one pass with the channel column of a pixel pair in
-// the registers of two lanes (pixel_regs.cuh)
+// 16-bit logits with 64 <= K <= kRegsKMax on images of a multiple of 256 pixels: one pass with the channel column of a
+// pixel pair in the registers of two lanes (pixel_regs.cuh).  BACS_NO_REGS=1 leaves these shapes to the streaming
+// passes (the reference the register-column kernel is tested against).
 static bool make_regs_plan(const bacs_pixel_args& a, StreamPlan* plan) {
   if (getenv("BACS_NO_REGS")) return false;
   const int64_t HW = (int64_t)a.H * a.W;
   auto al = [](const void* p, uintptr_t m) { return (reinterpret_cast<uintptr_t>(p) & (m - 1)) == 0; };
-  const int nt = regs_threads();
   if (a.dtype == BACS_F32 || a.K < 64 || a.K > kRegsKMax || HW % 256 != 0 || encode_tiled_fn() == nullptr) return false;
   if (a.mode == BACS_PIX_SCORE) return false;  // (per-image sums: streaming path)
   if (!al(a.logits, 16) || !al(a.labels, 8) || (a.dlogits && !al(a.dlogits, 4))) return false;
-  const int64_t tiles = HW / nt * a.B;
+  const int64_t tiles = HW / kRegsNT * a.B;
   if (tiles > 0x3fffffff) return false;
-  plan->blocks_x = (int)std::min<int64_t>(tiles, (int64_t)sm_count() * regs_ctas(nt));  // persistent: one wave
+  plan->blocks_x = (int)std::min<int64_t>(tiles, (int64_t)sm_count() * kRegsCTAs);  // persistent: one wave
   plan->part_bytes = align_up((size_t)plan->blocks_x * BACS_NACC * sizeof(double), 256);
   plan->coef_bytes = 0;
   return true;
@@ -1022,6 +947,79 @@ static bool make_lowres_plan(const bacs_pixel_args& a, int lh, int lw, LowresPla
   return plan->smem <= kLowresMaxSmem;
 }
 
+// What bacs_pixel_loss runs for `a`.  The kernel is chosen here alone, so that bacs_pixel_kernel_variant and
+// bacs_pixel_workspace_bytes report what runs.
+struct PixelRoute {
+  int variant;       // 0 generic tiles, 1 K <= 24 registers, 2 training step (plan); 4 streaming passes, 5 register
+                     // column (sp); -1 when K fits no shared-memory tile
+  PixelPlan plan;
+  StreamPlan sp;
+  int64_t n_part, part_per_image;  // partial rows of pixel_reduce_kernel; per image in SCORE mode
+  size_t workspace;  // bacs_pixel_workspace_bytes
+};
+
+static PixelRoute pixel_route(const bacs_pixel_args& a) {
+  PixelRoute r = {};
+  if (make_regs_plan(a, &r.sp)) {
+    r.variant = 5;
+    r.n_part = r.part_per_image = r.sp.blocks_x;
+  } else if (make_stream_plan(a, &r.sp)) {
+    r.variant = 4;
+    r.n_part = (int64_t)r.sp.blocks_x * a.B;
+    r.part_per_image = r.sp.blocks_x;
+  } else {
+    r.variant = make_plan(a, &r.plan);
+    if (r.variant < 0) return r;
+    r.part_per_image = ((int64_t)a.H * a.W + r.plan.P - 1) / r.plan.P;  // tiles per image
+    r.n_part = a.mode == BACS_PIX_SCORE ? r.part_per_image * a.B : r.plan.grid;
+    r.workspace = align_up((size_t)r.n_part * BACS_NACC * sizeof(double), 256);
+    return r;
+  }
+  r.workspace = r.sp.part_bytes + r.sp.coef_bytes;
+  return r;
+}
+
+// The argument checks of bacs_pixel_loss and bacs_pixel_loss_lowres; `fn` starts each message.
+static int check_pixel_args(const bacs_pixel_args* a, const char* fn) {
+  BACS_REQUIRE(a && a->logits && a->labels && a->acc, "%s: logits, labels and acc are required", fn);
+  BACS_REQUIRE(a->B > 0 && a->K > 0 && a->H > 0 && a->W > 0, "%s: bad shape", fn);
+  BACS_REQUIRE(a->ignore_index >= a->K || a->ignore_index < 0, "%s: ignore_index inside the class range", fn);
+  BACS_REQUIRE(a->mode >= 0 && a->mode <= BACS_PIX_SCORE, "%s: unknown mode %d", fn, a->mode);
+  BACS_REQUIRE(a->dtype >= 0 && a->dtype <= BACS_F16, "%s: unknown dtype %d", fn, a->dtype);
+  if (a->z) {
+    BACS_REQUIRE(a->T > 0 && a->h > 0 && a->w > 0, "%s: seen logits given without T/h/w", fn);
+    BACS_REQUIRE(a->seen_scale > 0 && a->H == a->h * a->seen_scale && a->W == a->w * a->seen_scale,
+                 "%s: H,W must equal h,w * seen_scale (the reference's nn.Upsample(scale_factor))", fn);
+  }
+  if (a->gz) BACS_REQUIRE(a->z && a->focal_head >= 0 && a->focal_head < a->T, "%s: focal head out of range", fn);
+  if (a->mode == BACS_PIX_WEIGHTED_CE)
+    BACS_REQUIRE(a->old_cl >= 1 && (a->z || a->seen_max),
+                 "%s: WEIGHTED_CE needs old_cl >= 1 and the seen logits / probabilities", fn);
+  if (a->mode != BACS_PIX_WEIGHTED_CE && a->dlogits)
+    BACS_REQUIRE(a->hist, "%s: CE-type gradients need the label histogram", fn);
+  if (a->mode == BACS_PIX_SCORE)
+    BACS_REQUIRE(a->score && !a->dlogits, "%s: SCORE mode needs score and no gradient", fn);
+  return BACS_OK;
+}
+
+// pixel_reduce_kernel over the n_part partial rows (per_image of them per image in SCORE mode), with the step's
+// scalar epilogue
+static void launch_pixel_reduce(const bacs_pixel_args& a, const double* partials, int n_part, int per_image,
+                                cudaStream_t s) {
+  const PixelEpilogue ep = {a.ready, a.focal_scale_out, a.loss_out, a.focal_weight, a.loss_coef, a.loss_over_wsum};
+  launch_pdl(pixel_reduce_kernel, dim3(1 + (a.mode == BACS_PIX_SCORE ? a.B : 0)), dim3(256), 0, s, partials, n_part,
+             per_image, a.acc, a.score, 1.0 / ((double)a.H * (double)a.W), ep);
+}
+
+template <typename T>
+static int launch_tile_kernel(const PixelParams& p, const PixelPlan& plan, cudaStream_t s) {
+  auto kern = plan.ppt == 2 ? (plan.rowtile ? pixel_loss_kernel<T, 2, true> : pixel_loss_kernel<T, 2, false>)
+              : plan.coop ? (plan.rowtile ? pixel_loss_kernel<T, 1, true, true> : pixel_loss_kernel<T, 1, false, true>)
+                          : (plan.rowtile ? pixel_loss_kernel<T, 1, true> : pixel_loss_kernel<T, 1, false>);
+  return launch_pixel_kernel("bacs_pixel_loss", false, kern, dim3(plan.grid), dim3(kConsumers + 32), plan.smem, s,
+                             p);
+}
+
 }  // namespace bacs
 
 using namespace bacs;
@@ -1037,23 +1035,8 @@ size_t bacs_pixel_lowres_workspace_bytes(const bacs_pixel_args* a, int32_t lh, i
 
 int bacs_pixel_loss_lowres(const bacs_pixel_args* a, int32_t lh, int32_t lw, void* workspace, size_t workspace_bytes,
                            void* stream) {
-  BACS_REQUIRE(a && a->logits && a->labels && a->acc, "bacs_pixel_loss_lowres: null argument");
-  BACS_REQUIRE(a->B > 0 && a->K > 0 && a->H > 0 && a->W > 0, "bacs_pixel_loss_lowres: empty shape");
-  BACS_REQUIRE(a->dtype == BACS_F32 || a->dtype == BACS_BF16 || a->dtype == BACS_F16, "bacs_pixel_loss_lowres: dtype");
-  if (a->z) {
-    BACS_REQUIRE(a->T > 0 && a->h > 0 && a->w > 0, "bacs_pixel_loss_lowres: seen logits given without T/h/w");
-    BACS_REQUIRE(a->seen_scale > 0 && a->H == a->h * a->seen_scale && a->W == a->w * a->seen_scale,
-                 "bacs_pixel_loss_lowres: H,W must equal h,w * seen_scale");
-  }
-  if (a->gz)
-    BACS_REQUIRE(a->z && a->focal_head >= 0 && a->focal_head < a->T, "bacs_pixel_loss_lowres: focal head out of range");
-  if (a->mode == BACS_PIX_WEIGHTED_CE)
-    BACS_REQUIRE(a->old_cl >= 1 && (a->z || a->seen_max),
-                 "bacs_pixel_loss_lowres: WEIGHTED_CE needs old_cl >= 1 and the seen logits / probabilities");
-  if (a->mode != BACS_PIX_WEIGHTED_CE && a->dlogits)
-    BACS_REQUIRE(a->hist, "bacs_pixel_loss_lowres: CE-type gradients need the label histogram");
-  if (a->mode == BACS_PIX_SCORE)
-    BACS_REQUIRE(a->score && !a->dlogits, "bacs_pixel_loss_lowres: SCORE mode needs score and no gradient");
+  int rc = check_pixel_args(a, "bacs_pixel_loss_lowres");
+  if (rc != BACS_OK) return rc;
   LowresPlan plan;
   if (!make_lowres_plan(*a, lh, lw, &plan)) {
     set_error("bacs_pixel_loss_lowres: unsupported geometry (H=%d W=%d lh=%d lw=%d K=%d%s): needs W == s*lw with "
@@ -1090,24 +1073,11 @@ int bacs_pixel_loss_lowres(const bacs_pixel_args* a, int32_t lh, int32_t lw, voi
   p.sx = a->z ? ac_scale(a->w, a->W) : 0.f;
   p.partials = reinterpret_cast<double*>(workspace);
   p.hx = hp_scale(lw, a->W);
-#define LAUNCH_LR(SXV, EXACT)                                                                                   \
-  do {                                                                                                          \
-    auto kern = pixel_lowres_kernel<SXV, EXACT>;                                                                \
-    if (plan.smem > 48 * 1024 &&                                                                                \
-        cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)plan.smem) != cudaSuccess) { \
-      set_error("bacs_pixel_loss_lowres: cannot opt in to %zu bytes of shared memory", plan.smem);              \
-      return BACS_ERR_CUDA;                                                                                     \
-    }                                                                                                           \
-    kern<<<plan.grid, kLowresThreads, plan.smem, s>>>(p);                                                       \
-  } while (0)
-  if (plan.exact) {
-    if (plan.SX == 16) LAUNCH_LR(16, true);
-    else LAUNCH_LR(8, true);
-  } else {
-    if (plan.SX == 16) LAUNCH_LR(16, false);
-    else LAUNCH_LR(8, false);
-  }
-#undef LAUNCH_LR
+  auto kern = plan.exact ? (plan.SX == 16 ? pixel_lowres_kernel<16, true> : pixel_lowres_kernel<8, true>)
+                         : (plan.SX == 16 ? pixel_lowres_kernel<16, false> : pixel_lowres_kernel<8, false>);
+  rc = launch_pixel_kernel("bacs_pixel_loss_lowres", false, kern, dim3(plan.grid), dim3(kLowresThreads), plan.smem, s,
+                           p);
+  if (rc != BACS_OK) return rc;
   BACS_CHECK_LAUNCH("bacs_pixel_loss_lowres");
   if (a->dlogits && a->dtype != BACS_F32) {
     const int nb = (int)((n_low + 255) / 256);
@@ -1117,259 +1087,128 @@ int bacs_pixel_loss_lowres(const bacs_pixel_args* a, int32_t lh, int32_t lw, voi
       lowres_cast_kernel<__half><<<nb, 256, 0, s>>>(p.g32, reinterpret_cast<__half*>(a->dlogits), n_low);
     BACS_CHECK_LAUNCH("bacs_pixel_loss_lowres(cast)");
   }
-  const int nblk = 1 + (a->mode == BACS_PIX_SCORE ? a->B : 0);
-  PixelEpilogue ep;
-  ep.ready = a->ready;
-  ep.focal_scale_out = a->focal_scale_out;
-  ep.loss_out = a->loss_out;
-  ep.focal_weight = a->focal_weight;
-  ep.loss_coef = a->loss_coef;
-  ep.loss_over_wsum = a->loss_over_wsum;
-  launch_pdl(pixel_reduce_kernel, dim3(nblk), dim3(256), 0, s, p.partials, plan.grid, plan.groups, a->acc, a->score,
-                                           1.0 / ((double)a->H * (double)a->W), ep);
+  launch_pixel_reduce(*a, p.partials, plan.grid, plan.groups, s);
   BACS_CHECK_LAUNCH("bacs_pixel_loss_lowres(reduce)");
   return BACS_OK;
 }
 
-size_t bacs_pixel_workspace_bytes(const bacs_pixel_args* a) {
-  if (!a) return 0;
-  StreamPlan sp;
-  if (make_regs_plan(*a, &sp)) return sp.part_bytes;
-  if (make_stream_plan(*a, &sp)) return sp.part_bytes + sp.coef_bytes;
-  PixelPlan plan;
-  if (!make_plan(*a, &plan)) return 0;
-  const int64_t HW = (int64_t)a->H * a->W;
-  const int64_t tiles = (HW + plan.P - 1) / plan.P * a->B;
-  const int64_t n_part = a->mode == BACS_PIX_SCORE ? tiles : plan.grid;
-  return align_up((size_t)n_part * BACS_NACC * sizeof(double), 256);
-}
+size_t bacs_pixel_workspace_bytes(const bacs_pixel_args* a) { return a ? pixel_route(*a).workspace : 0; }
 
-static bool wce_eligible(const bacs_pixel_args& a, const PixelPlan& plan) {
-  return plan.fast && plan.rowtile && a.mode == BACS_PIX_WEIGHTED_CE && !a.seen_max && a.z && encode_tiled_fn() != nullptr &&
-         a.w <= 256 && a.T <= 256 && a.K <= 256;
-}
-
-int bacs_pixel_kernel_variant(const bacs_pixel_args* a) {
-  PixelPlan plan;
-  StreamPlan sp;
-  if (a && make_regs_plan(*a, &sp)) return 5;
-  if (a && make_stream_plan(*a, &sp)) return 4;
-  if (!a || !make_plan(*a, &plan)) return -1;
-  return wce_eligible(*a, plan) ? 2 : (plan.fast ? 1 : 0);
-}
+int bacs_pixel_kernel_variant(const bacs_pixel_args* a) { return a ? pixel_route(*a).variant : -1; }
 
 int bacs_pixel_loss(const bacs_pixel_args* a, void* workspace, size_t workspace_bytes, bacs_stream_t stream) {
-  BACS_REQUIRE(a, "bacs_pixel_loss: null args");
-  BACS_REQUIRE(a->logits && a->labels && a->acc, "bacs_pixel_loss: logits, labels and acc are required");
-  BACS_REQUIRE(a->B > 0 && a->K > 0 && a->H > 0 && a->W > 0, "bacs_pixel_loss: bad shape");
-  BACS_REQUIRE(a->ignore_index >= a->K || a->ignore_index < 0, "bacs_pixel_loss: ignore_index inside the class range");
-  BACS_REQUIRE(a->mode >= 0 && a->mode <= BACS_PIX_SCORE, "bacs_pixel_loss: unknown mode %d", a->mode);
-  BACS_REQUIRE(a->dtype >= 0 && a->dtype <= BACS_F16, "bacs_pixel_loss: unknown dtype %d", a->dtype);
-  if (a->z) {
-    BACS_REQUIRE(a->T > 0 && a->h > 0 && a->w > 0, "bacs_pixel_loss: seen logits given without T/h/w");
-    BACS_REQUIRE(a->seen_scale > 0 && a->H == a->h * a->seen_scale && a->W == a->w * a->seen_scale,
-                 "bacs_pixel_loss: H,W must equal h,w * seen_scale (the reference's nn.Upsample(scale_factor))");
-  }
-  if (a->gz) BACS_REQUIRE(a->z && a->focal_head >= 0 && a->focal_head < a->T, "bacs_pixel_loss: focal head out of range");
-  if (a->mode == BACS_PIX_WEIGHTED_CE)
-    BACS_REQUIRE(a->old_cl >= 1 && (a->z || a->seen_max),
-                 "bacs_pixel_loss: WEIGHTED_CE needs old_cl >= 1 and the seen logits / probabilities");
-  if (a->mode != BACS_PIX_WEIGHTED_CE && a->dlogits)
-    BACS_REQUIRE(a->hist, "bacs_pixel_loss: CE-type gradients need the label histogram");
-  if (a->mode == BACS_PIX_SCORE)
-    BACS_REQUIRE(a->score && !a->dlogits, "bacs_pixel_loss: SCORE mode needs score and no gradient");
-  StreamPlan sp;
-  if (make_regs_plan(*a, &sp)) {  // large K, 16-bit logits: one pass, channel column in registers (pixel_regs.cuh)
-    if (!workspace || workspace_bytes < sp.part_bytes) {
-      set_error("bacs_pixel_loss: workspace too small (%zu bytes)", workspace_bytes);
-      return BACS_ERR_WORKSPACE;
-    }
-    RegsParams rq;
-    StreamParams& q = rq.s;
-    q.a = *a;
-    q.partials = reinterpret_cast<double*>(workspace);
-    q.coef = a->dlogits ? reinterpret_cast<float*>(workspace) : nullptr;  // only "a gradient is wanted" (stream_norm)
-    q.blocks_x = sp.blocks_x;
-    q.b0 = 0;
-    q.inv_n = (float)(1.0 / ((double)a->B * (double)a->H * (double)a->W));
-    q.sy = a->z ? ac_scale(a->h, a->H) : 0.f;
-    q.sx = a->z ? ac_scale(a->w, a->W) : 0.f;
-    const int64_t HWr = (int64_t)a->H * a->W;
-    const int nt = regs_threads();
-    rq.tiles_per_image = (int)(HWr / nt);
-    rq.n_tiles = rq.tiles_per_image * a->B;
-    if (!make_tile_map(&rq.tmap_in, a->logits, a->dtype, a->B, a->K, HWr, (unsigned)nt)) {
-      set_error("bacs_pixel_loss: cuTensorMapEncodeTiled failed for the logits");
-      return BACS_ERR_CUDA;
-    }
-    cudaStream_t st = (cudaStream_t)stream;
-    dim3 grid((unsigned)sp.blocks_x);
-    const size_t smem = (size_t)a->K * nt * 2 + 128;
-#define LAUNCH_REGS(TT)                                                                                         \
-  do {                                                                                                          \
-    auto kern = nt == 256 ? pixel_regs_kernel<TT, kRegsKH, 256, 2>                                              \
-                          : (regs_ctas(nt) == 3 ? pixel_regs_kernel<TT, kRegsKH, 128, 3> : pixel_regs_kernel<TT, kRegsKH, 128, 4>); \
-    if (cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) != cudaSuccess) {    \
-      set_error("bacs_pixel_loss: cannot opt in to %zu bytes of shared memory", smem);                          \
-      return BACS_ERR_CUDA;                                                                                     \
-    }                                                                                                           \
-    kern<<<grid, nt, smem, st>>>(rq);                                                                 \
-  } while (0)
-    if (a->dtype == BACS_BF16) LAUNCH_REGS(__nv_bfloat16);
-    else LAUNCH_REGS(__half);
-#undef LAUNCH_REGS
-    BACS_CHECK_LAUNCH("bacs_pixel_loss(register column)");
-    const int nblk = 1 + (a->mode == BACS_PIX_SCORE ? a->B : 0);
-    PixelEpilogue ep;
-    ep.ready = a->ready;
-    ep.focal_scale_out = a->focal_scale_out;
-    ep.loss_out = a->loss_out;
-    ep.focal_weight = a->focal_weight;
-    ep.loss_coef = a->loss_coef;
-    ep.loss_over_wsum = a->loss_over_wsum;
-    launch_pdl(pixel_reduce_kernel, dim3(nblk), dim3(256), 0, st, q.partials, sp.blocks_x, sp.blocks_x, a->acc,
-               a->score, 1.0 / ((double)a->H * (double)a->W), ep);
-    BACS_CHECK_LAUNCH("bacs_pixel_loss(reduce)");
-    return BACS_OK;
-  }
-  if (make_stream_plan(*a, &sp)) {  // large K: two streaming passes (pixel_stream.cuh)
-    if (!workspace || workspace_bytes < sp.part_bytes + sp.coef_bytes) {
-      set_error("bacs_pixel_loss: workspace too small (%zu bytes)", workspace_bytes);
-      return BACS_ERR_WORKSPACE;
-    }
-    StreamParams q;
-    q.a = *a;
-    q.partials = reinterpret_cast<double*>(workspace);
-    q.coef = a->dlogits ? reinterpret_cast<float*>(reinterpret_cast<unsigned char*>(workspace) + sp.part_bytes) : nullptr;
-    q.blocks_x = sp.blocks_x;
-    q.inv_n = (float)(1.0 / ((double)a->B * (double)a->H * (double)a->W));
-    q.sy = a->z ? ac_scale(a->h, a->H) : 0.f;
-    q.sx = a->z ? ac_scale(a->w, a->W) : 0.f;
-    cudaStream_t st = (cudaStream_t)stream;
-    const int n_part = sp.blocks_x * a->B;
-    // (launching a few images at a time so that pass B re-reads them from the 126 MB L2 was measured: 1 / 2 / 4 / 8
-    //  images per launch pair 2.67 / 1.69 / 1.66 / 1.48 ms against 1.33 ms for all 24 at once -- under-filled launches
-    //  cost more than the second HBM read)
-    const int per = a->B;
-    for (int b0 = 0; b0 < a->B; b0 += per) {
-      q.b0 = b0;
-      dim3 grid((unsigned)sp.blocks_x, (unsigned)std::min(per, a->B - b0));
-      BACS_DISPATCH_DTYPE(a->dtype, TT, { pixel_stream_stats_kernel<TT><<<grid, kStreamThreads, 0, st>>>(q); });
-      BACS_CHECK_LAUNCH("bacs_pixel_loss(stream stats)");
-      if (a->dlogits) {
-        BACS_DISPATCH_DTYPE(a->dtype, TT, { pixel_stream_grad_kernel<TT><<<grid, kStreamThreads, 0, st>>>(q); });
-        BACS_CHECK_LAUNCH("bacs_pixel_loss(stream grad)");
-      }
-    }
-    const int nblk = 1 + (a->mode == BACS_PIX_SCORE ? a->B : 0);
-    PixelEpilogue ep;
-    ep.ready = a->ready;
-    ep.focal_scale_out = a->focal_scale_out;
-    ep.loss_out = a->loss_out;
-    ep.focal_weight = a->focal_weight;
-    ep.loss_coef = a->loss_coef;
-    ep.loss_over_wsum = a->loss_over_wsum;
-    launch_pdl(pixel_reduce_kernel, dim3(nblk), dim3(256), 0, st, q.partials, n_part, sp.blocks_x, a->acc, a->score,
-                                              1.0 / ((double)a->H * (double)a->W), ep);
-    BACS_CHECK_LAUNCH("bacs_pixel_loss(reduce)");
-    return BACS_OK;
-  }
-  PixelPlan plan;
-  if (!make_plan(*a, &plan)) {
+  int rc = check_pixel_args(a, "bacs_pixel_loss");
+  if (rc != BACS_OK) return rc;
+  const PixelRoute r = pixel_route(*a);
+  if (r.variant < 0) {
     set_error("bacs_pixel_loss: K=%d too large for a shared-memory tile", a->K);
     return BACS_ERR_UNSUPPORTED;
   }
-  const int64_t HW = (int64_t)a->H * a->W;
-  const int64_t tiles_per_image = (HW + plan.P - 1) / plan.P;
-  const int64_t n_tiles = tiles_per_image * a->B;
-  BACS_REQUIRE(n_tiles < 0x7fffffff, "bacs_pixel_loss: too many tiles");
-  const int64_t n_part = a->mode == BACS_PIX_SCORE ? n_tiles : plan.grid;
-  if (!workspace || workspace_bytes < (size_t)n_part * BACS_NACC * sizeof(double)) {
+  const bool tiles = r.variant <= 2;
+  BACS_REQUIRE(!tiles || r.part_per_image * a->B < 0x7fffffff, "bacs_pixel_loss: too many tiles");
+  // (the tile kernels write their partial rows alone; bacs_pixel_workspace_bytes rounds those up to 256 bytes)
+  const size_t need = tiles ? (size_t)r.n_part * BACS_NACC * sizeof(double) : r.workspace;
+  if (!workspace || workspace_bytes < need) {
     set_error("bacs_pixel_loss: workspace too small (%zu bytes)", workspace_bytes);
     return BACS_ERR_WORKSPACE;
   }
-  const size_t es = dtype_size(a->dtype);
-  PixelParams p;
-  p.a = *a;
-  p.P = plan.P;
-  p.tiles_per_image = (int)tiles_per_image;
-  p.n_tiles = (int)n_tiles;
-  p.stages = plan.stages;
-  p.inv_n = (float)(1.0 / ((double)a->B * (double)HW));
-  p.sy = a->z ? ac_scale(a->h, a->H) : 0.f;
-  p.sx = a->z ? ac_scale(a->w, a->W) : 0.f;
-  p.partials = reinterpret_cast<double*>(workspace);
-  p.use_tmap = 0;
-  if (plan.fast) {
-    const bool ok_in = make_tile_map(&p.tmap_in, a->logits, a->dtype, a->B, a->K, HW);
-    const bool ok_out = !a->dlogits || make_tile_map(&p.tmap_out, a->dlogits, a->dtype, a->B, a->K, HW);
-    const bool ok_z = !(plan.rowtile && a->z) || make_z_map(&p.tmap_z, a->z, a->B, a->T, a->h, a->w);
-    p.use_tmap = (ok_in && ok_out && ok_z) ? 1 : 0;
-  }
-  p.use_bulk = (((HW * es) % 16 == 0) && ((reinterpret_cast<uintptr_t>(a->logits) & 15) == 0) &&
-                (!a->dlogits || (reinterpret_cast<uintptr_t>(a->dlogits) & 15) == 0))
-                   ? 1
-                   : 0;
   cudaStream_t s = (cudaStream_t)stream;
-#define LAUNCH_PIX(TT, PPT, KREG, ROWT, COOPV)                                                                 \
-  do {                                                                                                         \
-    auto kern = pixel_loss_kernel<TT, PPT, KREG, ROWT, COOPV>;                                                        \
-    if (plan.smem > 48 * 1024) {                                                                               \
-      cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)plan.smem); \
-      if (e != cudaSuccess) {                                                                                  \
-        set_error("bacs_pixel_loss: cannot opt in to %zu bytes of shared memory: %s", plan.smem,              \
-                  cudaGetErrorString(e));                                                                      \
-        return BACS_ERR_CUDA;                                                                                  \
-      }                                                                                                        \
-    }                                                                                                          \
-    kern<<<plan.grid, kConsumers + 32, plan.smem, s>>>(p);                                                     \
-  } while (0)
-#define LAUNCH_PIX_K(TT, PPT, COOPV)                       \
-  do {                                                     \
-    if (plan.rowtile) LAUNCH_PIX(TT, PPT, 0, true, COOPV); \
-    else LAUNCH_PIX(TT, PPT, 0, false, COOPV);             \
-  } while (0)
-  const bool wce = p.use_tmap && wce_eligible(*a, plan);
-  if (plan.fast && plan.stages != 4 && !wce) {
-    set_error("bacs_pixel_loss: tensor-map creation failed for the 3-stage training kernel");
-    return BACS_ERR_CUDA;
-  }
-  if (wce) {  // the training step's kernel
-    int rc;
-    switch (a->dtype) {
-      case BACS_F32: rc = launch_pixel_wce_f32(p, plan, s); break;
-      case BACS_BF16: rc = launch_pixel_wce_bf16(p, plan, s); break;
-      default: rc = launch_pixel_wce_f16(p, plan, s); break;
+  unsigned char* ws = reinterpret_cast<unsigned char*>(workspace);
+  double* partials = reinterpret_cast<double*>(workspace);
+  const int64_t HW = (int64_t)a->H * a->W;
+  const float inv_n = (float)(1.0 / ((double)a->B * (double)HW));
+  const float sy = a->z ? ac_scale(a->h, a->H) : 0.f, sx = a->z ? ac_scale(a->w, a->W) : 0.f;
+  if (!tiles) {
+    StreamParams q;
+    q.a = *a;
+    q.partials = partials;
+    // the streaming passes' coefficient planes follow the partials; the register-column kernel only tests the pointer
+    // (a gradient is wanted)
+    q.coef = a->dlogits ? reinterpret_cast<float*>(ws + (r.variant == 4 ? r.sp.part_bytes : 0)) : nullptr;
+    q.blocks_x = r.sp.blocks_x;
+    q.b0 = 0;
+    q.inv_n = inv_n;
+    q.sy = sy;
+    q.sx = sx;
+    if (r.variant == 5) {  // large K, 16-bit logits: one pass, channel column in registers (pixel_regs.cuh)
+      RegsParams rq;
+      rq.s = q;
+      rq.tiles_per_image = (int)(HW / kRegsNT);
+      rq.n_tiles = rq.tiles_per_image * a->B;
+      if (!make_tile_map(&rq.tmap_in, a->logits, a->dtype, a->B, a->K, HW, (unsigned)kRegsNT)) {
+        set_error("bacs_pixel_loss: cuTensorMapEncodeTiled failed for the logits");
+        return BACS_ERR_CUDA;
+      }
+      auto kern = a->dtype == BACS_BF16 ? pixel_regs_kernel<__nv_bfloat16, kRegsKH, kRegsNT, kRegsCTAs>
+                                        : pixel_regs_kernel<__half, kRegsKH, kRegsNT, kRegsCTAs>;
+      rc = launch_pixel_kernel("bacs_pixel_loss", false, kern, dim3(r.sp.blocks_x), dim3(kRegsNT),
+                               (size_t)a->K * kRegsNT * 2 + 128, s, rq);
+      if (rc != BACS_OK) return rc;
+      BACS_CHECK_LAUNCH("bacs_pixel_loss(register column)");
+    } else {  // large K: two streaming passes (pixel_stream.cuh)
+      // (launching a few images at a time so that pass B re-reads them from the 126 MB L2 was measured: 1 / 2 / 4 / 8
+      //  images per launch pair 2.67 / 1.69 / 1.66 / 1.48 ms against 1.33 ms for all 24 at once -- under-filled
+      //  launches cost more than the second HBM read)
+      const dim3 grid((unsigned)r.sp.blocks_x, (unsigned)a->B);
+      BACS_DISPATCH_DTYPE(a->dtype, TT, { pixel_stream_stats_kernel<TT><<<grid, kStreamThreads, 0, s>>>(q); });
+      BACS_CHECK_LAUNCH("bacs_pixel_loss(stream stats)");
+      if (a->dlogits) {
+        BACS_DISPATCH_DTYPE(a->dtype, TT, { pixel_stream_grad_kernel<TT><<<grid, kStreamThreads, 0, s>>>(q); });
+        BACS_CHECK_LAUNCH("bacs_pixel_loss(stream grad)");
+      }
     }
-    if (rc != BACS_OK) return rc;
-  } else if (plan.fast) {
-    int rc;
-    switch (a->dtype) {
-      case BACS_F32: rc = launch_pixel_fast_f32(p, plan, s); break;
-      case BACS_BF16: rc = launch_pixel_fast_bf16(p, plan, s); break;
-      default: rc = launch_pixel_fast_f16(p, plan, s); break;
-    }
-    if (rc != BACS_OK) return rc;
   } else {
-    BACS_DISPATCH_DTYPE(a->dtype, TT, {
-      if (plan.ppt == 2) LAUNCH_PIX_K(TT, 2, false);
-      else if (plan.coop) LAUNCH_PIX_K(TT, 1, true);
-      else LAUNCH_PIX_K(TT, 1, false);
-    });
+    const size_t es = dtype_size(a->dtype);
+    PixelParams p;
+    p.a = *a;
+    p.P = r.plan.P;
+    p.tiles_per_image = (int)r.part_per_image;
+    p.n_tiles = (int)(r.part_per_image * a->B);
+    p.stages = r.plan.stages;
+    p.inv_n = inv_n;
+    p.sy = sy;
+    p.sx = sx;
+    p.partials = partials;
+    p.use_tmap = 0;
+    if (r.variant >= 1) {
+      const bool ok_in = make_tile_map(&p.tmap_in, a->logits, a->dtype, a->B, a->K, HW);
+      const bool ok_out = !a->dlogits || make_tile_map(&p.tmap_out, a->dlogits, a->dtype, a->B, a->K, HW);
+      const bool ok_z = !(r.plan.rowtile && a->z) || make_z_map(&p.tmap_z, a->z, a->B, a->T, a->h, a->w);
+      p.use_tmap = (ok_in && ok_out && ok_z) ? 1 : 0;
+    }
+    p.use_bulk = (((HW * es) % 16 == 0) && ((reinterpret_cast<uintptr_t>(a->logits) & 15) == 0) &&
+                  (!a->dlogits || (reinterpret_cast<uintptr_t>(a->dlogits) & 15) == 0))
+                     ? 1
+                     : 0;
+    // the training-step kernel needs the tensor maps: without them a 4-stage ring runs on pixel_fast_kernel, while a
+    // 3-stage ring (planned for the training-step kernel alone) has no kernel to run on
+    int variant = r.variant;
+    if (variant == 2 && !p.use_tmap) {
+      if (r.plan.stages != 4) {
+        set_error("bacs_pixel_loss: tensor-map creation failed for the 3-stage training kernel");
+        return BACS_ERR_CUDA;
+      }
+      variant = 1;
+    }
+    if (variant == 2) {
+      switch (a->dtype) {
+        case BACS_F32: rc = launch_pixel_wce_f32(p, r.plan, s); break;
+        case BACS_BF16: rc = launch_pixel_wce_bf16(p, r.plan, s); break;
+        default: rc = launch_pixel_wce_f16(p, r.plan, s); break;
+      }
+    } else if (variant == 1) {
+      switch (a->dtype) {
+        case BACS_F32: rc = launch_pixel_fast_f32(p, r.plan, s); break;
+        case BACS_BF16: rc = launch_pixel_fast_bf16(p, r.plan, s); break;
+        default: rc = launch_pixel_fast_f16(p, r.plan, s); break;
+      }
+    } else {
+      BACS_DISPATCH_DTYPE(a->dtype, TT, { rc = launch_tile_kernel<TT>(p, r.plan, s); });
+    }
+    if (rc != BACS_OK) return rc;
+    BACS_CHECK_LAUNCH("bacs_pixel_loss");
   }
-#undef LAUNCH_PIX_K
-#undef LAUNCH_PIX
-  BACS_CHECK_LAUNCH("bacs_pixel_loss");
-  const int nblk = 1 + (a->mode == BACS_PIX_SCORE ? a->B : 0);
-  PixelEpilogue ep;
-  ep.ready = a->ready;
-  ep.focal_scale_out = a->focal_scale_out;
-  ep.loss_out = a->loss_out;
-  ep.focal_weight = a->focal_weight;
-  ep.loss_coef = a->loss_coef;
-  ep.loss_over_wsum = a->loss_over_wsum;
-  launch_pdl(pixel_reduce_kernel, dim3(nblk), dim3(256), 0, s, p.partials, (int)n_part, p.tiles_per_image, a->acc, a->score,
-                                           1.0 / (double)HW, ep);
+  launch_pixel_reduce(*a, partials, (int)r.n_part, (int)r.part_per_image, s);
   BACS_CHECK_LAUNCH("bacs_pixel_loss(reduce)");
   return BACS_OK;
 }

@@ -2,13 +2,13 @@
 // over the logits, the [K] x 2-pixel column of a pixel pair held in the registers of TWO lanes.
 //
 // The two streaming passes of pixel_stream.cuh read every logit twice (3 K s bytes per pixel against the algorithmic
-// 2 K s).  Here a CTA of eight warps owns 256-pixel tiles.  Lanes l and l + 16 of a warp share one pair of adjacent
+// 2 K s).  Here a CTA of four warps owns 128-pixel tiles.  Lanes l and l + 16 of a warp share one pair of adjacent
 // pixels: lane l keeps channels 0 .. 75 of the pair, lane l + 16 channels 76 .. 151, one 32-bit register per channel
 // holding the packed pair exactly as it sits in memory (76 registers -> 128 registers per thread, 16 warps per SM; a
 // whole column per thread needs 255 registers, leaves two warps per scheduler and stalls on its own dependent
 // instructions: 1.18 ms).
-//   load      one 3-D tensor-map TMA box [K][256] (77 KB at K = 151) per tile into the CTA's single landing buffer; the
-//             threads copy their half column into registers (LDS.32 with immediate offsets), the CTA synchronises and
+//   load      one 3-D tensor-map TMA box [K][128] (38.6 KB at K = 151) per tile into the CTA's single landing buffer;
+//             the threads copy their half column into registers (LDS.32 with immediate offsets), the CTA synchronises and
 //             the box of the CTA's NEXT tile is requested at once -- it lands while this tile is computed from the
 //             registers, so the registers are the second pipeline stage and no warp waits on a cold load.  (First
 //             version: K independent 4-byte global loads per thread, 128 bytes per warp request: 957 us for the
@@ -33,6 +33,8 @@ namespace bacs {
 
 constexpr int kRegsKH = 76;      // channel registers of a thread; K <= 2 * kRegsKH
 constexpr int kRegsKMax = 2 * kRegsKH;
+constexpr int kRegsNT = 128;     // threads of a CTA = pixels of a tile
+constexpr int kRegsCTAs = 4;     // resident CTAs per SM (DESIGN 5.1a)
 
 struct alignas(64) RegsParams {
   CUtensorMap tmap_in;  // logits as (H*W, K, B), box (NT, K, 1)

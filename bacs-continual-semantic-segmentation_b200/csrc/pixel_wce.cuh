@@ -544,15 +544,7 @@ static int launch_wce_one(const PixelParams& p, const PixelPlan& plan, cudaStrea
   const bool std_hp = a.gamma == 2.f && a.ukd && (!a.gz || (a.focal_gamma == 2.f && a.focal_alpha < 0.f));
   auto kern = plan.stages == 3 ? (std_hp ? pixel_wce_kernel<T, KREG, true, 3> : pixel_wce_kernel<T, KREG, false, 3>)
                                : (std_hp ? pixel_wce_kernel<T, KREG, true, 4> : pixel_wce_kernel<T, KREG, false, 4>);
-  if (plan.smem > 48 * 1024) {
-    cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)plan.smem);
-    if (e != cudaSuccess) {
-      set_error("bacs_pixel_loss: cannot opt in to %zu bytes of shared memory: %s", plan.smem, cudaGetErrorString(e));
-      return BACS_ERR_CUDA;
-    }
-  }
-  launch_pdl(kern, dim3(plan.grid), dim3(kFastThreads), plan.smem, s, p);
-  return BACS_OK;
+  return launch_pixel_kernel("bacs_pixel_loss", true, kern, dim3(plan.grid), dim3(kFastThreads), plan.smem, s, p);
 }
 
 template <typename T>

@@ -1,5 +1,5 @@
 """Times the full-resolution pixel kernel (bacs_pixel_loss) at a named config and checks it against the device oracle.
-usage: pixel_time.py [config] [bf16|f16|f32] [B]      (BACS_NO_REGS=1 / BACS_NO_STREAM=1 select the older variants)"""
+usage: pixel_time.py [config] [bf16|f16|f32] [B]      (BACS_NO_REGS=1 selects the two streaming passes)"""
 import sys, torch
 sys.path.insert(0, '/root/repo')
 from bacs_b200 import synth, ops, _cabi
