@@ -58,6 +58,8 @@ _SIGNATURES = {
     "bacs_pixel_loss": (i32, [C.POINTER(PixelArgs), vp, sz, vp]),
     "bacs_pixel_lowres_workspace_bytes": (sz, [C.POINTER(PixelArgs), i32, i32]),
     "bacs_pixel_loss_lowres": (i32, [C.POINTER(PixelArgs), i32, i32, vp, sz, vp]),
+    "bacs_pseudo_label": (i32, [vp, i32, i32, i32, i32, i32, vp, vp]),
+    "bacs_pseudo_label_lowres": (i32, [vp, i32, i32, i32, i32, i32, i32, i32, vp, vp]),
     "bacs_distill_workspace_bytes": (sz, [i32, i32, i32, i32, i32, i32]),
     "bacs_teacher_distill": (i32, [vp, vp, i32, i32, i32, i32, i32, vp, i32, i32, f32, vp, vp, vp, vp, sz, vp]),
     "bacs_teacher_distill_add": (i32, [vp, vp, i32, i32, i32, i32, i32, vp, i32, i32, f32, vp, vp, vp, vp, vp, sz, vp]),

@@ -15,7 +15,7 @@ CSRC = os.path.join(PKG, "csrc")
 INCLUDE = os.path.join(ROOT, "include")
 LIB = os.path.join(PKG, "libbacs_b200.so")
 SOURCES = ["labels.cu", "prototypes.cu", "seen.cu", "pixel_loss.cu", "pixel_fast_bf16.cu", "pixel_fast_f32.cu",
-           "pixel_fast_f16.cu", "distill.cu", "distill_tc.cu", "misc.cu", "peer.cu", "class_distance.cu"]
+           "pixel_fast_f16.cu", "distill.cu", "distill_tc.cu", "misc.cu", "peer.cu", "class_distance.cu", "pseudo.cu"]
 
 
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17",

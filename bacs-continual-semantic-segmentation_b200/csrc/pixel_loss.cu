@@ -857,12 +857,6 @@ static bool make_regs_plan(const bacs_pixel_args& a, StreamPlan* plan) {
   return true;
 }
 
-struct LowresPlan {
-  int SX, R, groups, nsrc_max, grid;
-  bool exact;  // W == SX * lw: the instantiation with compile-time pixel offsets
-  size_t smem, part_bytes, g32_bytes;
-};
-
 // host copy of lerp_half_pixel's source coordinate (fp32, op by op)
 static float host_src(int dst, float scale) {
   volatile float t = (float)dst + 0.5f;
@@ -893,7 +887,7 @@ static int host_span_start(int j, int lw, int W, float scale) {
 // Accepted geometry: W == SX * lw with SX 8 or 16 and H a multiple of lh, or the network's output stride s = 16 or 8
 // applied to any input, lh == ceil(H / s) and lw == ceil(W / s) (DeepLab's padded stride-2 convolutions; s = 16 where
 // both match).  The seen heads (a.z) need the first form.
-static bool make_lowres_plan(const bacs_pixel_args& a, int lh, int lw, LowresPlan* plan) {
+bool make_lowres_plan(const bacs_pixel_args& a, int lh, int lw, LowresPlan* plan) {
   if (lh <= 0 || lw <= 0 || lw > kLowresThreads || a.K > 255) return false;
   int SX = 0;
   bool exact = false;

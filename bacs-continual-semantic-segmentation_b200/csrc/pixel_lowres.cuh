@@ -22,6 +22,10 @@
 // y-weights and sends one global fp32 RED per low-res cell (shared-memory fp32 atomics are CAS loops on sm_100).
 // The per-pixel stage (pixel_terms, seen heads) runs as a rolled loop over dynamically indexed copies of the
 // per-pixel statistics, so its code exists once instead of SX times.
+//
+// PSEUDO = true is the arg-max-only instantiation behind bacs_pseudo_label_lowres (csrc/pseudo.cu): `labels` and `preds`
+// are the same tensor; a thread reads its labels, runs pass 1a when one of them is 0, writes the arg-max at exactly
+// those pixels and returns -- the pseudo label is bit for bit the `preds` of the loss kernel at the same sem_logits.
 #pragma once
 #include "pixel_common.cuh"
 
@@ -46,6 +50,15 @@ constexpr int kLowresChunk = 8;   // channels per gradient-reduction round
 constexpr int kLowresMaxSrc = 8;  // source rows a row group may touch (the host halves R until it holds)
 constexpr size_t kLowresMaxSmem = (size_t)200 * 1024;  // dynamic shared memory of one CTA (two CTAs per SM)
 
+struct LowresPlan {
+  int SX, R, groups, nsrc_max, grid;
+  bool exact;  // W == SX * lw: the instantiation with compile-time pixel offsets
+  size_t smem, part_bytes, g32_bytes;
+};
+// The plan of a launch of pixel_lowres_kernel for `a` at low-res size lh x lw; false when the geometry is not served
+// (pixel_loss.cu).  bacs_pseudo_label_lowres accepts exactly what bacs_pixel_loss_lowres accepts without `z`.
+bool make_lowres_plan(const bacs_pixel_args& a, int lh, int lw, LowresPlan* plan);
+
 // half-pixel source column of output pixel x (lerp_half_pixel's src, op by op) and the column it rounds to
 __device__ __forceinline__ float lowres_src(int x, float scale) {
   const float s = __fsub_rn(__fmul_rn(scale, __fadd_rn((float)x, 0.5f)), 0.5f);
@@ -62,7 +75,7 @@ __device__ __forceinline__ int lowres_span_start(int j, int lw, int W, float sca
   return x;
 }
 
-template <int SX, bool EXACT>
+template <int SX, bool EXACT, bool PSEUDO = false>
 __global__ void __launch_bounds__(kLowresThreads, 2) pixel_lowres_kernel(const __grid_constant__ LowresParams p) {
   extern __shared__ __align__(16) unsigned char lr_smem[];
   __shared__ float red_scratch[kLowresThreads / 32][BACS_NACC];
@@ -192,7 +205,22 @@ __global__ void __launch_bounds__(kLowresThreads, 2) pixel_lowres_kernel(const _
     const int64_t pix0 = (int64_t)b * HW + (int64_t)Y * a.W + (EXACT ? (int64_t)SX * j : (int64_t)xs);
 
     // ---- labels: SX int64 -> one byte each (255 = ignored / invalid) ----------------------------------------------
-    if constexpr (!EXACT) {  // scalar loads; pixels past the span read as ignored
+    uint32_t bg = 0;  // PSEUDO: bit i set where pixel i is labelled 0
+    if constexpr (PSEUDO) {
+      const int64_t* lp = a.labels + pix0;
+      if (EXACT && (reinterpret_cast<uintptr_t>(lp) & 15) == 0) {
+#pragma unroll
+        for (int i = 0; i < SX; i += 2) {
+          const longlong2 v = *reinterpret_cast<const longlong2*>(lp + i);
+          bg |= ((uint32_t)(v.x == 0) << i) | ((uint32_t)(v.y == 0) << (i + 1));
+        }
+      } else {
+#pragma unroll
+        for (int i = 0; i < SX; ++i)
+          if (EXACT || i < npx) bg |= (uint32_t)(lp[i] == 0) << i;
+      }
+      if (bg == 0) return;  // no pixel to rewrite (no barrier follows in this instantiation)
+    } else if constexpr (!EXACT) {  // scalar loads; pixels past the span read as ignored
       const int64_t* lp = a.labels + pix0;
 #pragma unroll
       for (int q = 0; q < SX / 4; ++q) ypk[q] = 0;
@@ -249,8 +277,8 @@ __global__ void __launch_bounds__(kLowresThreads, 2) pixel_lowres_kernel(const _
     // (x16 align_corners=True: the thread's SX pixels touch the low-res columns cb, cb+1, cb+2 only)
     float Lseen[SX], Lzf[SX], Lwx1[SX];
     uint32_t fdm = 0;  // bit i: pixel i's left tap is column cb+1 (else cb); its right tap is the next column, clamped
-    const int cb = (EXACT && a.z) ? lerp_align_corners(SX * j, a.w, p.sx).i0 : 0;
-    if (EXACT && a.z) {  // (the plan accepts the seen logits at the exact geometry only)
+    const int cb = (!PSEUDO && EXACT && a.z) ? lerp_align_corners(SX * j, a.w, p.sx).i0 : 0;
+    if (!PSEUDO && EXACT && a.z) {  // (the plan accepts the seen logits at the exact geometry only)
       float wx1[SX], zmx[SX], zf[SX];
 #pragma unroll
       for (int i = 0; i < SX; ++i) {
@@ -305,6 +333,12 @@ __global__ void __launch_bounds__(kLowresThreads, 2) pixel_lowres_kernel(const _
             am[i] = c;
           }
         }
+      }
+      if constexpr (PSEUDO) {  // the arg-max replaces the label where it is 0; nothing else is written
+#pragma unroll
+        for (int i = 0; i < SX; ++i)
+          if ((bg >> i) & 1u) a.preds[pix0 + i] = am[i];
+        return;
       }
       if (a.preds) {
         int64_t* out = a.preds + pix0;
@@ -451,6 +485,7 @@ __global__ void __launch_bounds__(kLowresThreads, 2) pixel_lowres_kernel(const _
       }
     }
   }
+  if constexpr (PSEUDO) return;
 
   // ---- pass 2: gradients, reduced over the thread's pixels in registers, over the CTA's rows in shared memory --------
   if (p.g32) {

@@ -153,11 +153,15 @@ class BACSLoss(ExperienceReplay):
 
     # ---- step ------------------------------------------------------------------------------------
     def post_process_mask(self, img, mask):
-        """bacs_loss.py:205-210: optional pseudo-labelling of background by the old model."""
+        """bacs_loss.py:205-210: optional pseudo-labelling of background by the old model, in place on ``mask`` by one
+        kernel (no host synchronisation).  With ``fused_logit_upsample`` the teacher's low-res sem_logits are read and
+        the pseudo labels follow that flag's arg-max contract (identical except at fp32 near-ties)."""
         if self.pseudo_label and self.prev_model is not None:
             with torch.no_grad():
-                pseudo_labels = self._argmax(self.prev_model(img))
-            mask[mask == 0] = pseudo_labels[mask == 0]
+                if self.fused_logit_upsample:
+                    ops.pseudo_label_inplace(mask, self.prev_model(img, return_sem_logits=True), lowres=True)
+                else:
+                    ops.pseudo_label_inplace(mask, self.prev_model(img))
         return mask
 
     def compute_loss(self, batch, model, train=True):

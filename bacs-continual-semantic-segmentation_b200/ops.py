@@ -361,6 +361,33 @@ def pixel_loss(logits: torch.Tensor, labels: torch.Tensor, mode: int, *, want_gr
     return out
 
 
+def pseudo_label_inplace(labels: torch.Tensor, teacher_logits: torch.Tensor, lowres: bool = False) -> torch.Tensor:
+    """labels[labels == 0] = teacher_logits.argmax(1)[labels == 0] in place (bacs_loss.py:205-210), in one launch and
+    without a host synchronisation; ties go to the lowest channel, every other label keeps its value.  Returns
+    ``labels`` (int64 [B,H,W]; a non-contiguous tensor is rewritten through a contiguous copy).
+
+    ``teacher_logits``: [B,K_t,H,W], or with ``lowres=True`` the teacher's low-res ``sem_logits`` [B,K_t,lh,lw] whose
+    bilinear up-sample (align_corners=False) is evaluated inside the arg-max -- then the pseudo labels equal the
+    ``preds`` of ``pixel_loss(..., lowres=True)`` at the same sem_logits.  K_t may differ from the student's K."""
+    work = _cuda(labels, "pseudo_label_inplace", torch.int64)
+    teacher = _cuda(teacher_logits, "pseudo_label_inplace")
+    if work.dim() != 3 or teacher.dim() != 4 or teacher.shape[0] != work.shape[0] \
+            or (not lowres and tuple(teacher.shape[2:]) != tuple(work.shape[1:])):
+        raise ValueError("pseudo_label_inplace: labels %s do not match teacher logits %s"
+                         % (tuple(labels.shape), tuple(teacher_logits.shape)))
+    B, H, W = work.shape
+    Kt = teacher.shape[1]
+    if lowres:
+        check(_lib().bacs_pseudo_label_lowres(teacher.data_ptr(), _dt(teacher), B, Kt, teacher.shape[2], teacher.shape[3],
+                                              H, W, work.data_ptr(), _stream()), "bacs_pseudo_label_lowres")
+    else:
+        check(_lib().bacs_pseudo_label(teacher.data_ptr(), _dt(teacher), B, Kt, H, W, work.data_ptr(), _stream()),
+              "bacs_pseudo_label")
+    if work is not labels:
+        labels.copy_(work)
+    return labels
+
+
 # --------------------------------------------------------------------------------------
 # teacher distillation / DER
 # --------------------------------------------------------------------------------------

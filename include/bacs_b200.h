@@ -269,6 +269,25 @@ int bacs_pixel_loss_lowres(const bacs_pixel_args* args_host, int32_t lh, int32_t
                            size_t workspace_bytes, bacs_stream_t stream);
 
 /* ---------------------------------------------------------------------------------
+ * Pseudo-labelled background (loss/bacs_loss.py:205-210):
+ *   pseudo = argmax_c teacher[:, c];  labels[labels == 0] = pseudo[labels == 0]
+ * in place on labels int64 [B,H,W]: where a label is 0 it becomes the teacher's arg-max (ties -> lowest channel);
+ * every other value (255, other classes, negative or out-of-range values) keeps its bits.  K_t, the teacher's channel
+ * count, may differ from the student's; dtype is the teacher's (fp32, bf16, fp16).  Asynchronous on `stream`, no
+ * workspace, no host synchronisation (graph-capturable).  Null pointers or B, K_t, H, W <= 0 give BACS_ERR_INVALID.
+ *
+ * bacs_pseudo_label: full-resolution teacher logits [B,K_t,H,W] (NCHW), any K_t >= 1.
+ * bacs_pseudo_label_lowres: the teacher's low-res sem_logits [B,K_t,lh,lw]; the bilinear align_corners=False
+ *   up-sample to H x W is evaluated inside the arg-max, and the result equals bit for bit the preds of
+ *   bacs_pixel_loss_lowres for the same sem_logits.  Geometry: what bacs_pixel_loss_lowres accepts without z (K = K_t);
+ *   anything else returns BACS_ERR_UNSUPPORTED and leaves the labels untouched.
+ * --------------------------------------------------------------------------------- */
+int bacs_pseudo_label(const void* teacher, int32_t dtype, int32_t B, int32_t K_t, int32_t H, int32_t W,
+                      int64_t* labels, bacs_stream_t stream);
+int bacs_pseudo_label_lowres(const void* sem_logits, int32_t dtype, int32_t B, int32_t K_t, int32_t lh, int32_t lw,
+                             int32_t H, int32_t W, int64_t* labels, bacs_stream_t stream);
+
+/* ---------------------------------------------------------------------------------
  * Teacher distillation on the last attention map (loss/bacs_loss.py:258-294):
  *   L = lkd * mean_{b,a,y} sqrt( sum_x ( m * (U(old)^2 - U(new)^2) )^2 ),
  *   U = bilinear up-sample to HxW, align_corners=False; gradient to `new` only.
