@@ -49,6 +49,7 @@ _SIGNATURES = {
     "bacs_proto_update": (i32, [vp, vp, i32, vp, vp, i32, i32, vp, vp]),
     "bacs_seen_logits": (i32, [vp, i32, i32, i32, i32, i32, vp, vp, vp, i32, vp, vp]),
     "bacs_seen_logits_heads": (i32, [vp, i32, i32, i32, i32, i32, vp, vp, vp, i32, vp, vp, vp]),
+    "bacs_seen_logits_many": (i32, [vp, i32, i32, i32, i32, i32, vp, vp, vp, vp, vp, i32, vp, vp, vp]),
     "bacs_seen_upsample": (i32, [vp, i32, i32, i32, i32, i32, i32, vp, vp]),
     "bacs_seen_head_backward": (i32, [vp, i32, i32, i32, i32, i32, vp, vp, vp, vp, vp, vp, vp, vp]),
     "bacs_focal_scale": (i32, [vp, vp, f32, vp, vp, vp]),

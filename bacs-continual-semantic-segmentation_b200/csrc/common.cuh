@@ -36,6 +36,8 @@ extern unsigned long long g_launch_count;
 
 int sm_count();
 
+constexpr int kMaxTasks = BACS_MAX_TASKS;
+
 // ---- programmatic dependent launch ---------------------------------------------------
 // The kernels of a training step run back to back on one stream.  Launched through launch_pdl() a kernel may become
 // resident while its predecessor drains: everything before pdl_wait() (shared-memory tables, barrier and tensor-memory

@@ -216,8 +216,9 @@ __global__ void __launch_bounds__(256) remap_apply_kernel(const int64_t* __restr
 // Nearest down-sample + task id + raster rank inside (image, task).
 // One block per image; pixels are processed in raster order in chunks of blockDim.
 // -------------------------------------------------------------------------------------
-constexpr int kMaxTasks = 32;
+// KMAX is the task capacity of the per-warp counters: 32 up to 32 tasks, kMaxTasks above.
 
+template <int KMAX>
 __global__ void __launch_bounds__(1024) downsample_task_kernel(const int64_t* __restrict__ labels, int H, int W, int h,
                                                                int w, float sy, float sx,
                                                                const int32_t* __restrict__ task_lut, int T,
@@ -225,12 +226,12 @@ __global__ void __launch_bounds__(1024) downsample_task_kernel(const int64_t* __
                                                                int8_t* __restrict__ task, int32_t* __restrict__ rank,
                                                                int32_t* __restrict__ n_bt) {
   __shared__ int lut[256];
-  __shared__ int warp_cnt[32][kMaxTasks + 1];
-  __shared__ int base[kMaxTasks];
+  __shared__ int warp_cnt[32][KMAX + 1];
+  __shared__ int base[KMAX];
   const int b = blockIdx.x;
   const int tid = threadIdx.x, lane = tid & 31, wid = tid >> 5;
   const int nwarp = blockDim.x >> 5;
-  if (tid < kMaxTasks) base[tid] = 0;
+  if (tid < KMAX) base[tid] = 0;
   pdl_wait();
   pdl_trigger();
   for (int i = tid; i < 256; i += blockDim.x) lut[i] = task_lut[i];
@@ -336,8 +337,8 @@ int bacs_label_downsample_task(const int64_t* labels, int B, int H, int W, int h
   BACS_REQUIRE(B > 0 && H > 0 && W > 0 && h > 0 && w > 0, "bacs_label_downsample_task: bad shape");
   BACS_REQUIRE(T > 0 && T <= kMaxTasks, "bacs_label_downsample_task: T=%d not in [1,%d]", T, kMaxTasks);
   const float sy = (float)H / (float)h, sx = (float)W / (float)w;
-  launch_pdl(downsample_task_kernel, dim3(B), dim3(1024), 0, (cudaStream_t)stream, labels, H, W, h, w, sy, sx, task_lut, T,
-             labels_down, task, rank, n_bt);
+  launch_pdl(T <= 32 ? downsample_task_kernel<32> : downsample_task_kernel<kMaxTasks>, dim3(B), dim3(1024), 0,
+             (cudaStream_t)stream, labels, H, W, h, w, sy, sx, task_lut, T, labels_down, task, rank, n_bt);
   BACS_CHECK_LAUNCH("bacs_label_downsample_task");
   return BACS_OK;
 }

@@ -47,6 +47,8 @@ __device__ __forceinline__ unsigned long long global_timer_ns() {
 
 static unsigned long long g_peer_timeout_ns = 30ull * 1000ull * 1000ull * 1000ull;
 
+// TCAP: task capacity of the fused update's shared arrays (64 up to 64 tasks, kMaxTasks above).
+template <int TCAP>
 __global__ void __launch_bounds__(1024) peer_allreduce_update_kernel(PeerPtrs pp, int rank, int world, int n, int n_max,
                                                                      unsigned long long timeout_ns,
                                                                      double* __restrict__ packed,
@@ -116,8 +118,8 @@ __global__ void __launch_bounds__(1024) peer_allreduce_update_kernel(PeerPtrs pp
   if (proto == nullptr) return;
   __syncthreads();  // packed[] (global, this block) is complete
   // ---- fused running-mean update (same arithmetic as proto_update_kernel) ----
-  __shared__ float s_old[64], s_den[64];
-  __shared__ int s_upd[64];
+  __shared__ float s_old[TCAP], s_den[TCAP];
+  __shared__ int s_upd[TCAP];
   __shared__ int s_nonzero;
   const double* sums = packed;
   const double* counts = packed + (size_t)Tn * D;
@@ -179,14 +181,18 @@ int bacs_peer_allreduce(double* packed, int n, int n_max, int rank, int world, c
   BACS_REQUIRE(packed && peer_buf_host && peer_flag_host && step_dev, "bacs_peer_allreduce: null pointer");
   BACS_REQUIRE(world >= 1 && world <= kPeerMaxWorld && rank >= 0 && rank < world, "bacs_peer_allreduce: bad rank/world");
   BACS_REQUIRE(n > 0 && n <= n_max, "bacs_peer_allreduce: n=%d exceeds the symmetric buffer (%d)", n, n_max);
-  if (proto) BACS_REQUIRE(count && T > 0 && T <= 64 && D > 0 && n >= T * D + T, "bacs_peer_allreduce: bad prototype shape");
+  if (proto) {
+    BACS_REQUIRE(count && D > 0 && n >= T * D + T, "bacs_peer_allreduce: bad prototype shape");
+    BACS_REQUIRE(T > 0 && T <= kMaxTasks, "bacs_peer_allreduce: T=%d not in [1,%d]", T, kMaxTasks);
+  }
   PeerPtrs pp;
   for (int r = 0; r < kPeerMaxWorld; ++r) {
     pp.buf[r] = r < world ? reinterpret_cast<double*>(peer_buf_host[r]) : nullptr;
     pp.flag[r] = r < world ? reinterpret_cast<unsigned int*>(peer_flag_host[r]) : nullptr;
   }
-  launch_pdl(peer_allreduce_update_kernel, dim3(1), dim3(1024), 0, (cudaStream_t)stream, pp, rank, world, n, n_max,
-             g_peer_timeout_ns, packed, step_dev, error_dev, proto, count, count_is_int64, T, D, ready);
+  launch_pdl(proto && T > 64 ? peer_allreduce_update_kernel<kMaxTasks> : peer_allreduce_update_kernel<64>, dim3(1),
+             dim3(1024), 0, (cudaStream_t)stream, pp, rank, world, n, n_max, g_peer_timeout_ns, packed, step_dev,
+             error_dev, proto, count, count_is_int64, T, D, ready);
   BACS_CHECK_LAUNCH("bacs_peer_allreduce");
   return BACS_OK;
 }

@@ -14,8 +14,11 @@ namespace bacs {
 // Each lane accumulates into its own column of a warp-private shared-memory table
 // acc[task][low/high][lane] (conflict-free, no atomics): a pixel touches exactly one entry, so
 // the cost per element does not grow with the number of tasks.
+// MANY (more than kTaskWindow tasks): blockIdx.z picks a window of kTaskWindow tasks; the block sums only the pixels of
+// those tasks and writes their columns, so its shared memory and split bookkeeping are those of a 32-task launch.
 constexpr int kAccWarps = 8;
-template <typename T>
+constexpr int kTaskWindow = 32;
+template <typename T, bool MANY = false>
 __global__ void __launch_bounds__(32 * kAccWarps) proto_accumulate_kernel(const T* __restrict__ feat, int B, int D,
                                                                           int hw, const int8_t* __restrict__ task,
                                                                           const int32_t* __restrict__ rank,
@@ -24,28 +27,30 @@ __global__ void __launch_bounds__(32 * kAccWarps) proto_accumulate_kernel(const 
                                                                           float* __restrict__ partial /* [B,D,Tn,2] */,
                                                                           const void* __restrict__ count_raw, int count_is_int64,
                                                                           unsigned long long* __restrict__ count_snap) {
-  extern __shared__ float s_acc[];  // [warp][Tn][2][32]
+  extern __shared__ float s_acc[];  // [warp][Tw][2][32]
   const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
   const int b = blockIdx.y;
   const int c = blockIdx.x * kAccWarps + wid;
+  const int t_lo = MANY ? (int)blockIdx.z * kTaskWindow : 0;      // first task of this block
+  const int Tw = MANY ? min(kTaskWindow, Tn - t_lo) : Tn;         // tasks of this block
   pdl_wait();
   pdl_trigger();
-  if (count_snap && blockIdx.x == 0 && blockIdx.y == 0 && threadIdx.x < Tn)
-    count_snap[threadIdx.x] = count_is_int64 ? reinterpret_cast<const unsigned long long*>(count_raw)[threadIdx.x]
-                                             : (unsigned long long)reinterpret_cast<const unsigned*>(count_raw)[threadIdx.x];
+  if (count_snap && blockIdx.x == 0 && blockIdx.y == 0 && threadIdx.x < Tw)
+    count_snap[t_lo + threadIdx.x] = count_is_int64 ? reinterpret_cast<const unsigned long long*>(count_raw)[t_lo + threadIdx.x]
+                                                    : (unsigned long long)reinterpret_cast<const unsigned*>(count_raw)[t_lo + threadIdx.x];
   if (c >= D) return;
-  float* acc = s_acc + (size_t)wid * Tn * 64;
-  for (int i = lane; i < Tn * 64; i += 32) acc[i] = 0.f;
-  // lane g holds the split point of task g
+  float* acc = s_acc + (size_t)wid * Tw * 64;
+  for (int i = lane; i < Tw * 64; i += 32) acc[i] = 0.f;
+  // lane g holds the split point of task t_lo + g
   int split = 0x7fffffff;
-  if (mode == 0 && lane < Tn) {
+  if (mode == 0 && lane < Tw) {
     long long pre = 0, tot = 0;
     for (int bb = 0; bb < B; ++bb) {
-      const int n = n_bt[bb * Tn + lane];
+      const int n = n_bt[bb * Tn + t_lo + lane];
       if (bb < b) pre += n;
       tot += n;
     }
-    const long long nb = n_bt[b * Tn + lane];
+    const long long nb = n_bt[b * Tn + t_lo + lane];
     if (tot > 0) {
       const long long base = (long long)D * pre + (long long)c * nb;
       const long long r0 = base / tot;
@@ -65,6 +70,7 @@ __global__ void __launch_bounds__(32 * kAccWarps) proto_accumulate_kernel(const 
     for (int u = 0; u < U; ++u) {
       const int q = q0 + u * 32 + lane;
       t[u] = q < hw ? (int)tk[q] : -1;
+      if constexpr (MANY) t[u] = (t[u] >= t_lo && t[u] < t_lo + Tw) ? t[u] - t_lo : -1;
       v[u] = (t[u] >= 0) ? DT<T>::to_f(row[q]) : 0.f;
       k[u] = (t[u] >= 0) ? rk[q] : 0;
     }
@@ -75,8 +81,8 @@ __global__ void __launch_bounds__(32 * kAccWarps) proto_accumulate_kernel(const 
     }
   }
   __syncwarp();
-  float* out = partial + (((int64_t)b * D + c) * Tn) * 2;
-  for (int e = 0; e < Tn * 2; ++e) {
+  float* out = partial + (((int64_t)b * D + c) * Tn + t_lo) * 2;
+  for (int e = 0; e < Tw * 2; ++e) {
     const float r = warp_sum(acc[e * 32 + lane]);
     if (lane == 0) out[e] = r;
   }
@@ -85,7 +91,7 @@ __global__ void __launch_bounds__(32 * kAccWarps) proto_accumulate_kernel(const 
 // Vectorised variant (hw a multiple of 8, 16-byte aligned rows): a lane handles 8 consecutive pixels per step; task
 // bytes and features of a row's first step are requested before the split points are worked out.  The per-warp table
 // has one 32-float row per (task, low / high) entry: a lane only ever touches its own bank.
-template <typename T>
+template <typename T, bool MANY = false>
 __global__ void __launch_bounds__(32 * kAccWarps, 4) proto_accumulate_vec_kernel(const T* __restrict__ feat, int B, int D,
                                                                                  int hw, const int8_t* __restrict__ task,
                                                                                  const int32_t* __restrict__ rank,
@@ -94,12 +100,14 @@ __global__ void __launch_bounds__(32 * kAccWarps, 4) proto_accumulate_vec_kernel
                                                                                  const void* __restrict__ count_raw,
                                                                                  int count_is_int64,
                                                                                  unsigned long long* __restrict__ count_snap) {
-  extern __shared__ float s_acc[];  // [warp][Tn*2 + 2][32] | [warp][33] split points
+  extern __shared__ float s_acc[];  // [warp][Tw*2 + 2][32] | [warp][33] split points
   __shared__ long long s_pre[32], s_tot[32];  // per task: masked pixels in the images before b / in all images
   __shared__ int s_nb[32];
   const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
   const int b = blockIdx.y;
   const int c = blockIdx.x * kAccWarps + wid;
+  const int t_lo = MANY ? (int)blockIdx.z * kTaskWindow : 0;
+  const int Tw = MANY ? min(kTaskWindow, Tn - t_lo) : Tn;
   const bool live = c < D;
   pdl_wait();
   pdl_trigger();
@@ -138,14 +146,14 @@ __global__ void __launch_bounds__(32 * kAccWarps, 4) proto_accumulate_vec_kernel
   load_step(0);
   // fused update: the finalize launch reads the counts of BEFORE the step from this snapshot while one of its blocks
   // already writes the new ones (8 bytes per task whatever the count type; a float count sits in the low word)
-  if (count_snap && blockIdx.x == 0 && blockIdx.y == 0 && threadIdx.x < Tn)
-    count_snap[threadIdx.x] = count_is_int64 ? reinterpret_cast<const unsigned long long*>(count_raw)[threadIdx.x]
-                                             : (unsigned long long)reinterpret_cast<const unsigned*>(count_raw)[threadIdx.x];
+  if (count_snap && blockIdx.x == 0 && blockIdx.y == 0 && threadIdx.x < Tw)
+    count_snap[t_lo + threadIdx.x] = count_is_int64 ? reinterpret_cast<const unsigned long long*>(count_raw)[t_lo + threadIdx.x]
+                                                    : (unsigned long long)reinterpret_cast<const unsigned*>(count_raw)[t_lo + threadIdx.x];
   if (mode == 0) {  // the same for all channels of the block: warp w takes tasks w, w + 8, ..., its lanes the images
-    for (int t = wid; t < Tn; t += kAccWarps) {
+    for (int t = wid; t < Tw; t += kAccWarps) {
       long long pre = 0, tot = 0;
       for (int bb = lane; bb < B; bb += 32) {
-        const int n = n_bt[bb * Tn + t];
+        const int n = n_bt[bb * Tn + t_lo + t];
         if (bb < b) pre += n;
         tot += n;
       }
@@ -154,18 +162,18 @@ __global__ void __launch_bounds__(32 * kAccWarps, 4) proto_accumulate_vec_kernel
       if (lane == 0) {
         s_pre[t] = pre;
         s_tot[t] = tot;
-        s_nb[t] = n_bt[b * Tn + t];
+        s_nb[t] = n_bt[b * Tn + t_lo + t];
       }
     }
   }
   __syncthreads();
   if (!live) return;
-  const int ne = Tn * 2;
+  const int ne = Tw * 2;
   float* acc = s_acc + (size_t)wid * (ne + 2) * 32;          // + the dump entry of pixels without a task
   int* s_split = reinterpret_cast<int*>(s_acc + (size_t)kAccWarps * (ne + 2) * 32) + wid * 33;
   for (int i = lane; i < (ne + 2) * 32; i += 32) acc[i] = 0.f;
   int split = 0x7fffffff;
-  if (mode == 0 && lane < Tn) {
+  if (mode == 0 && lane < Tw) {
     const long long tot = s_tot[lane], nb = s_nb[lane];
     if (tot > 0) {
       const long long base = (long long)D * s_pre[lane] + (long long)c * nb;
@@ -176,7 +184,7 @@ __global__ void __launch_bounds__(32 * kAccWarps, 4) proto_accumulate_vec_kernel
       split = sp > 0x7fffffffLL ? 0x7fffffff : (int)sp;
     }
   }
-  s_split[lane] = split;                    // lanes >= Tn hold INT_MAX: the dump entry (index Tn) never splits
+  s_split[lane] = split;                    // lanes >= Tw hold INT_MAX: the dump entry (index Tw) never splits
   if (lane == 0) s_split[32] = 0x7fffffff;
   __syncwarp();
   // Branch-free inner loop: a pixel without a task (-1: background / ignore / later task) adds into a dump entry
@@ -191,8 +199,12 @@ __global__ void __launch_bounds__(32 * kAccWarps, 4) proto_accumulate_vec_kernel
       const T* e8 = reinterpret_cast<const T*>(&raw[u][0]);
       // labels are blocky: 8 pixels of ONE task whose ranks (increasing along the row) lie on one side of the split
       // point are added in registers and cost a single table update
-      const unsigned t0 = t8[u].x & 0xffu;
+      unsigned t0 = t8[u].x & 0xffu;
       if (t8[u].x == t0 * 0x01010101u && t8[u].y == t8[u].x) {
+        if constexpr (MANY) {   // 8 pixels of one task outside the window add nothing here
+          t0 -= (unsigned)t_lo;
+          if (t0 >= (unsigned)Tw) continue;
+        }
         const int sp = s_split[t0];
         if (rr[7] < sp || rr[0] >= sp) {
           float v = 0.f;
@@ -205,7 +217,8 @@ __global__ void __launch_bounds__(32 * kAccWarps, 4) proto_accumulate_vec_kernel
 #pragma unroll
       for (int e = 0; e < 8; ++e) {
         const unsigned tb = ((e < 4 ? t8[u].x >> (8 * e) : t8[u].y >> (8 * (e - 4))) & 0xffu);
-        const int tt = (int)min(tb, (unsigned)Tn);                 // 0xff (-1) -> the dump entry
+        // 0xff (-1) -> the dump entry; so does a task outside the window (the subtraction wraps below it)
+        const int tt = MANY ? (int)min(tb - (unsigned)t_lo, (unsigned)Tw) : (int)min(tb, (unsigned)Tn);
         const int hi = rr[e] < s_split[tt] ? 0 : 32;
         acc[tt * 64 + hi + lane] += DT<T>::to_f(e8[e]);         // bank = lane: conflict-free whatever the tasks
       }
@@ -215,7 +228,7 @@ __global__ void __launch_bounds__(32 * kAccWarps, 4) proto_accumulate_vec_kernel
   // The ne column sums of the warp as a reduce-scatter over groups of 16 entries: after the exchange with lane ^ 16 a
   // lane keeps 8 entries, then 4, 2, 1 -- 16 shuffles per group instead of 5 per entry, and the same association
   // ((l, l^16), then ^8, ^4, ^2, ^1) as warp_sum(), so the sums are bit-identical to the entry-by-entry form.
-  float* out = partial + (((int64_t)b * D + c) * Tn) * 2;
+  float* out = partial + (((int64_t)b * D + c) * Tn + t_lo) * 2;
   for (int e0 = 0; e0 < ne; e0 += 16) {
     float v[16];
 #pragma unroll
@@ -261,7 +274,7 @@ __device__ __forceinline__ void mma_16816(float (&d)[4], uint32_t a0, uint32_t a
                  : "r"(a0), "r"(a1), "r"(a2), "r"(a3), "r"(b0), "r"(b1));
 }
 
-template <typename T, int NT>  // NT = ceil(Tn / 8) task tiles
+template <typename T, int NT, bool MANY = false>  // NT = ceil(Tn / 8) task tiles (4 with MANY: one 32-task window)
 __global__ void __launch_bounds__(32 * kMmaWarps) proto_accumulate_mma_kernel(const T* __restrict__ feat, int B, int D, int hw,
                                                                               const int8_t* __restrict__ task,
                                                                               const int32_t* __restrict__ rank,
@@ -277,11 +290,13 @@ __global__ void __launch_bounds__(32 * kMmaWarps) proto_accumulate_mma_kernel(co
   const int b = blockIdx.y;
   const int cb = (blockIdx.x * kMmaWarps + wid) * 16;  // first channel of this warp
   const int g = lane >> 2, tig = lane & 3;
+  const int t_lo = MANY ? (int)blockIdx.z * kTaskWindow : 0;
+  const int Tw = MANY ? min(kTaskWindow, Tn - t_lo) : Tn;
   pdl_wait();
   pdl_trigger();
-  if (count_snap && blockIdx.x == 0 && blockIdx.y == 0 && threadIdx.x < Tn)
-    count_snap[threadIdx.x] = count_is_int64 ? reinterpret_cast<const unsigned long long*>(count_raw)[threadIdx.x]
-                                             : (unsigned long long)reinterpret_cast<const unsigned*>(count_raw)[threadIdx.x];
+  if (count_snap && blockIdx.x == 0 && blockIdx.y == 0 && threadIdx.x < Tw)
+    count_snap[t_lo + threadIdx.x] = count_is_int64 ? reinterpret_cast<const unsigned long long*>(count_raw)[t_lo + threadIdx.x]
+                                                    : (unsigned long long)reinterpret_cast<const unsigned*>(count_raw)[t_lo + threadIdx.x];
   // the first loads go out before the split bookkeeping
   const bool live = cb < D;
   const T* rowA = feat + ((int64_t)b * D + (live ? cb : 0) + g) * hw + tig * 8;
@@ -306,10 +321,10 @@ __global__ void __launch_bounds__(32 * kMmaWarps) proto_accumulate_mma_kernel(co
   };
   load_step(0);
   if (mode == 0) {  // per task: masked pixels in the images before b / in all images / in this image
-    for (int t = wid; t < Tn; t += kMmaWarps) {
+    for (int t = wid; t < Tw; t += kMmaWarps) {
       long long pre = 0, tot = 0;
       for (int bb = lane; bb < B; bb += 32) {
-        const int n = n_bt[bb * Tn + t];
+        const int n = n_bt[bb * Tn + t_lo + t];
         if (bb < b) pre += n;
         tot += n;
       }
@@ -318,7 +333,7 @@ __global__ void __launch_bounds__(32 * kMmaWarps) proto_accumulate_mma_kernel(co
       if (lane == 0) {
         s_pre[t] = pre;
         s_tot[t] = tot;
-        s_nb[t] = n_bt[b * Tn + t];
+        s_nb[t] = n_bt[b * Tn + t_lo + t];
       }
     }
   }
@@ -339,7 +354,7 @@ __global__ void __launch_bounds__(32 * kMmaWarps) proto_accumulate_mma_kernel(co
         const uint32_t tb = j ? tw[u].y : tw[u].x;
 #pragma unroll
         for (int nt = 0; nt < NT; ++nt) {
-          const uint32_t m = __vcmpeq4(tb, (uint32_t)(8 * nt + g) * 0x01010101u);  // 0xff where the pixel's task is this lane's n
+          const uint32_t m = __vcmpeq4(tb, (uint32_t)(t_lo + 8 * nt + g) * 0x01010101u);  // 0xff where the pixel's task is this lane's n
           mma_16816<T>(d[nt], a0, a1, a2, a3, __byte_perm(m, 0u, 0x1100) & MmaOne<T>::pair,
                        __byte_perm(m, 0u, 0x3322) & MmaOne<T>::pair);
         }
@@ -359,7 +374,7 @@ __global__ void __launch_bounds__(32 * kMmaWarps) proto_accumulate_mma_kernel(co
       const int t = 8 * nt + 2 * tig + (e & 1), c = cb + g + (e >> 1) * 8;
       int row = c, sp = 0x7fffffff;
       bool is_split = false;
-      if (t < Tn && mode == 0) {
+      if (t < Tw && mode == 0) {
         const long long tot = s_tot[t], nb = s_nb[t];
         if (tot > 0 && nb > 0) {
           const long long base = (long long)D * s_pre[t] + (long long)c * nb;
@@ -372,12 +387,12 @@ __global__ void __launch_bounds__(32 * kMmaWarps) proto_accumulate_mma_kernel(co
           sp = is_split ? (int)spl : 0x7fffffff;
         }
       }
-      if (t < Tn && !is_split && d[nt][e] != 0.f) atomicAdd(sums + (int64_t)t * D + row, (double)d[nt][e]);
+      if (t < Tw && !is_split && d[nt][e] != 0.f) atomicAdd(sums + (int64_t)(t_lo + t) * D + row, (double)d[nt][e]);
       unsigned todo = __ballot_sync(0xffffffffu, is_split);
       while (todo) {
         const int src = __ffs(todo) - 1;
         todo &= todo - 1;
-        const int sc = __shfl_sync(0xffffffffu, c, src), st = __shfl_sync(0xffffffffu, t, src);
+        const int sc = __shfl_sync(0xffffffffu, c, src), st = t_lo + __shfl_sync(0xffffffffu, t, src);
         const int ssp = __shfl_sync(0xffffffffu, sp, src), srow = __shfl_sync(0xffffffffu, row, src);
         const T* rowp = feat + ((int64_t)b * D + sc) * hw;
         const int8_t* tkr = task + (int64_t)b * hw;
@@ -557,13 +572,14 @@ __global__ void __launch_bounds__(kFinRows* kFinLanes) proto_finalize_kernel(con
 }
 
 // proto[g] = (S[g] + cnt[g]*proto[g]) / (cnt[g] + N[g]), cnt[g] += N[g]; separate fp32
-// roundings per operation (torch evaluates them as separate kernels).
+// roundings per operation (torch evaluates them as separate kernels).  TCAP: task capacity of the shared arrays.
+template <int TCAP>
 __global__ void __launch_bounds__(512) proto_update_kernel(float* __restrict__ proto, void* __restrict__ count,
                                                            int count_is_int64, const double* __restrict__ sums,
                                                            const double* __restrict__ counts, int Tn, int D,
                                                            int32_t* __restrict__ ready) {
-  __shared__ float s_old[64], s_den[64];
-  __shared__ int s_upd[64];
+  __shared__ float s_old[TCAP], s_den[TCAP];
+  __shared__ int s_upd[TCAP];
   __shared__ int s_nonzero;
   if (threadIdx.x == 0) s_nonzero = 0;
   pdl_wait();
@@ -614,7 +630,8 @@ using namespace bacs;
 extern "C" {
 
 size_t bacs_proto_workspace_bytes(int B, int D, int T) {
-  return align_up((size_t)B * D * T * 2 * sizeof(float), 256) + 256;   // partial sums | snapshot of the counts
+  // partial sums | snapshot of the counts (8 bytes per task)
+  return align_up((size_t)B * D * T * 2 * sizeof(float), 256) + align_up((size_t)T * 8, 256);
 }
 
 static int proto_accumulate_impl(const void* features, int dtype, int B, int D, int h, int w, const int8_t* task,
@@ -623,7 +640,7 @@ static int proto_accumulate_impl(const void* features, int dtype, int B, int D, 
                                  int32_t* ready, bacs_stream_t stream) {
   BACS_REQUIRE(features && task && rank && n_bt && sums && counts && workspace, "bacs_proto_accumulate: null pointer");
   BACS_REQUIRE(B > 0 && D > 0 && h > 0 && w > 0 && B <= kFinMaxB, "bacs_proto_accumulate: bad shape (B <= 1024)");
-  BACS_REQUIRE(T > 0 && T <= 32, "bacs_proto_accumulate: T=%d not in [1,32]", T);
+  BACS_REQUIRE(T > 0 && T <= kMaxTasks, "bacs_proto_accumulate: T=%d not in [1,%d]", T, kMaxTasks);
   BACS_REQUIRE(mode == 0 || mode == 1, "bacs_proto_accumulate: mode must be 0 (exact) or 1 (channel)");
   if (workspace_bytes < bacs_proto_workspace_bytes(B, D, T)) {
     set_error("bacs_proto_accumulate: workspace %zu < %zu", workspace_bytes, bacs_proto_workspace_bytes(B, D, T));
@@ -636,9 +653,14 @@ static int proto_accumulate_impl(const void* features, int dtype, int B, int D, 
                                    : nullptr;
   const void* count_raw = count;
   const int hw = h * w;
-  dim3 grid((D + kAccWarps - 1) / kAccWarps, B);
-  const size_t acc_smem = (size_t)kAccWarps * T * 64 * sizeof(float);
-  const size_t vec_smem = (size_t)kAccWarps * ((T * 2 + 2) * 32 + 33) * sizeof(float);
+  // more than kTaskWindow tasks: one launch with a grid dimension over 32-task windows (the MANY instantiations), each
+  // block with the shared memory of a 32-task launch; the features are read once per window, the later reads from L2
+  const bool many = T > kTaskWindow;
+  const int n_win = (T + kTaskWindow - 1) / kTaskWindow;
+  const int Tw = many ? kTaskWindow : T;
+  dim3 grid((D + kAccWarps - 1) / kAccWarps, B, n_win);
+  const size_t acc_smem = (size_t)kAccWarps * Tw * 64 * sizeof(float);
+  const size_t vec_smem = (size_t)kAccWarps * ((Tw * 2 + 2) * 32 + 33) * sizeof(float);
   const bool vec = hw % 8 == 0 && (reinterpret_cast<uintptr_t>(features) & 15) == 0 &&
                    (reinterpret_cast<uintptr_t>(task) & 7) == 0 && (reinterpret_cast<uintptr_t>(rank) & 15) == 0;
   // 16-bit features on 32-pixel chunks, 16-channel blocks: one-hot GEMM on the tensor cores (BACS_NO_PROTO_MMA=1: off)
@@ -646,17 +668,18 @@ static int proto_accumulate_impl(const void* features, int dtype, int B, int D, 
   if (mma) {
     launch_pdl(proto_zero_sums_kernel, dim3((T * D + 255) / 256), dim3(256), 0, s, sums, T * D);
     BACS_CHECK_LAUNCH("bacs_proto_accumulate(zero)");
-    dim3 mgrid((D / 16 + kMmaWarps - 1) / kMmaWarps, B);
+    dim3 mgrid((D / 16 + kMmaWarps - 1) / kMmaWarps, B, n_win);
     const int nt = (T + 7) / 8;
-#define BACS_MMA_LAUNCH(TT, NTV)                                                                                        \
-  launch_pdl(proto_accumulate_mma_kernel<TT, NTV>, mgrid, dim3(32 * kMmaWarps), 0, s, reinterpret_cast<const TT*>(features), \
+#define BACS_MMA_LAUNCH(TT, NTV, M)                                                                                     \
+  launch_pdl(proto_accumulate_mma_kernel<TT, NTV, M>, mgrid, dim3(32 * kMmaWarps), 0, s, reinterpret_cast<const TT*>(features), \
              B, D, hw, task, rank, n_bt, T, mode, sums, count_raw, count_is_int64, snap)
 #define BACS_MMA_NT(TT)                                 \
   do {                                                  \
-    if (nt == 1) BACS_MMA_LAUNCH(TT, 1);                \
-    else if (nt == 2) BACS_MMA_LAUNCH(TT, 2);           \
-    else if (nt == 3) BACS_MMA_LAUNCH(TT, 3);           \
-    else BACS_MMA_LAUNCH(TT, 4);                        \
+    if (many) BACS_MMA_LAUNCH(TT, 4, true);             \
+    else if (nt == 1) BACS_MMA_LAUNCH(TT, 1, false);    \
+    else if (nt == 2) BACS_MMA_LAUNCH(TT, 2, false);    \
+    else if (nt == 3) BACS_MMA_LAUNCH(TT, 3, false);    \
+    else BACS_MMA_LAUNCH(TT, 4, false);                 \
   } while (0)
     if (dtype == BACS_BF16) BACS_MMA_NT(__nv_bfloat16);
     else BACS_MMA_NT(__half);
@@ -664,21 +687,19 @@ static int proto_accumulate_impl(const void* features, int dtype, int B, int D, 
 #undef BACS_MMA_LAUNCH
   } else {
   BACS_DISPATCH_DTYPE(dtype, TT, {
-    if (vec) {
-      auto kern = proto_accumulate_vec_kernel<TT>;
-      if (vec_smem > 48 * 1024) {
-        cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)vec_smem);
-        if (e != cudaSuccess) {
-          set_error("bacs_proto_accumulate: shared memory opt-in failed: %s", cudaGetErrorString(e));
-          return BACS_ERR_CUDA;
-        }
+    // the table of a 32-task window (vec: 68.6 KB, scalar: 64 KB) needs the opt-in above the 48 KB default
+    auto kern = vec ? (many ? proto_accumulate_vec_kernel<TT, true> : proto_accumulate_vec_kernel<TT>)
+                    : (many ? proto_accumulate_kernel<TT, true> : proto_accumulate_kernel<TT>);
+    const size_t smem = vec ? vec_smem : acc_smem;
+    if (smem > 48 * 1024) {
+      cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+      if (e != cudaSuccess) {
+        set_error("bacs_proto_accumulate: shared memory opt-in failed: %s", cudaGetErrorString(e));
+        return BACS_ERR_CUDA;
       }
-      launch_pdl(kern, grid, dim3(32 * kAccWarps), vec_smem, s, reinterpret_cast<const TT*>(features), B, D, hw, task, rank,
-                 n_bt, T, mode, partial, count_raw, count_is_int64, snap);
-    } else {
-      launch_pdl(proto_accumulate_kernel<TT>, grid, dim3(32 * kAccWarps), acc_smem, s,
-                 reinterpret_cast<const TT*>(features), B, D, hw, task, rank, n_bt, T, mode, partial, count_raw, count_is_int64, snap);
     }
+    launch_pdl(kern, grid, dim3(32 * kAccWarps), smem, s, reinterpret_cast<const TT*>(features), B, D, hw, task, rank,
+               n_bt, T, mode, partial, count_raw, count_is_int64, snap);
   });
   }
   BACS_CHECK_LAUNCH("bacs_proto_accumulate");
@@ -700,7 +721,7 @@ int bacs_proto_accumulate_update(const void* features, int dtype, int B, int D, 
                                  void* workspace, size_t workspace_bytes, float* proto, void* count, int count_is_int64,
                                  int32_t* ready, bacs_stream_t stream) {
   BACS_REQUIRE(proto && count, "bacs_proto_accumulate_update: null pointer");
-  BACS_REQUIRE(T <= 32, "bacs_proto_accumulate_update: T=%d not in [1,32]", T);
+  BACS_REQUIRE(T > 0 && T <= kMaxTasks, "bacs_proto_accumulate_update: T=%d not in [1,%d]", T, kMaxTasks);
   return proto_accumulate_impl(features, dtype, B, D, h, w, task, rank, n_bt, T, mode, sums, counts, workspace,
                                workspace_bytes, proto, count, count_is_int64, ready, stream);
 }
@@ -708,8 +729,9 @@ int bacs_proto_accumulate_update(const void* features, int dtype, int B, int D, 
 int bacs_proto_update(float* proto, void* count, int count_is_int64, const double* sums, const double* counts, int T,
                       int D, int32_t* ready, bacs_stream_t stream) {
   BACS_REQUIRE(proto && count && sums && counts, "bacs_proto_update: null pointer");
-  BACS_REQUIRE(T > 0 && T <= 64 && D > 0, "bacs_proto_update: bad shape");
-  launch_pdl(proto_update_kernel, dim3(1), dim3(512), 0, (cudaStream_t)stream, proto, count, count_is_int64, sums, counts, T, D,
+  BACS_REQUIRE(D > 0, "bacs_proto_update: bad shape");
+  BACS_REQUIRE(T > 0 && T <= kMaxTasks, "bacs_proto_update: T=%d not in [1,%d]", T, kMaxTasks);
+  launch_pdl(T <= 64 ? proto_update_kernel<64> : proto_update_kernel<kMaxTasks>, dim3(1), dim3(512), 0, (cudaStream_t)stream, proto, count, count_is_int64, sums, counts, T, D,
              ready);
   BACS_CHECK_LAUNCH("bacs_proto_update");
   return BACS_OK;

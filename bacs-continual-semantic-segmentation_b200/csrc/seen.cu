@@ -4,6 +4,7 @@
 // z[b,t,q] = bias_t + sum_c w[t,c] * |sigmoid(f[b,c,q]) - sigmoid(proto[t,c])|
 // A weighted L1 distance per task head: HBM/ALU work, no GEMM form (SURVEY 7).
 #include <algorithm>
+#include <type_traits>
 
 #include "common.cuh"
 
@@ -54,19 +55,27 @@ struct HeadRows {
   const float* w[32];
   const float* b[32];
 };
+// The same for bacs_seen_logits_many: up to kMaxTasks heads (2 KB of kernel parameters).
+struct HeadRowsMany {
+  const float* w[kMaxTasks];
+  const float* b[kMaxTasks];
+};
 
 // A CTA covers 32*PX consecutive pixels of one image (lane -> PX adjacent pixels, one vector load per channel
 // row) and a slice of the channels; its 8 warps stride over the slice.  The CS CTAs of a thread-block cluster
 // split the channels and the leader adds their partial sums through distributed shared memory, so the grid
 // has enough CTAs to fill the machine while the summation order stays fixed.
 // Per channel the T (weight, sigmoid(proto)) pairs sit in one shared-memory row read with broadcast 128-bit loads.
-template <typename T, int TMAX, int PX>
+// MANY (bacs_seen_logits_many): blockIdx.z picks the chunk of TMAX heads h0 .. h0 + TMAX - 1 that the CTA evaluates;
+// the chunks of a pixel tile read the same features, the later ones mostly from L2.
+template <typename T, int TMAX, int PX, bool MANY = false>
 __global__ void __launch_bounds__(32 * kSeenWarps, (TMAX * PX <= 32 ? 3 : (TMAX * PX <= 48 ? 2 : 1))) seen_logits_kernel(const T* __restrict__ feat, int D, int hw,
                                                                        const float* __restrict__ proto,
                                                                        const float* __restrict__ weight,
                                                                        const float* __restrict__ bias, int Tn,
                                                                        int chunk, int cs, float* __restrict__ z,
-                                                                       const HeadRows rows, float* __restrict__ zero_out) {
+                                                                       const std::conditional_t<MANY, HeadRowsMany, HeadRows> rows,
+                                                                       float* __restrict__ zero_out) {
   extern __shared__ __align__(16) float smem[];
   constexpr int PS = 32 * PX;            // pixels per CTA
   constexpr int stride = 2 * TMAX;       // floats per channel row: w[0..TMAX) | sigmoid(proto)[0..TMAX)
@@ -74,6 +83,8 @@ __global__ void __launch_bounds__(32 * kSeenWarps, (TMAX * PX <= 32 ? 3 : (TMAX 
   const int tid = threadIdx.x;
   const int rank = (int)blockIdx.x % cs, pb = (int)blockIdx.x / cs;
   const int b = blockIdx.y;
+  const int h0 = MANY ? (int)blockIdx.z * TMAX : 0;   // first head of this CTA
+  const int Th = MANY ? min(TMAX, Tn - h0) : Tn;      // heads of this CTA
   const int q0 = pb * PS + lane * PX;
   const int per = (D + cs - 1) / cs;
   const int c_begin = rank * per, c_end = min(D, c_begin + per);
@@ -91,8 +102,8 @@ __global__ void __launch_bounds__(32 * kSeenWarps, (TMAX * PX <= 32 ? 3 : (TMAX 
     __syncthreads();
     for (int i = tid; i < TMAX * cn; i += 32 * kSeenWarps) {
       const int t = i / cn, c = i - t * cn;
-      smem[c * stride + t] = t < Tn ? (weight ? weight[t * D + c0 + c] : rows.w[t][c0 + c]) : 0.f;
-      smem[c * stride + TMAX + t] = t < Tn ? sigmoid_fast(proto[t * D + c0 + c]) : 0.f;
+      smem[c * stride + t] = t < Th ? (weight ? weight[(h0 + t) * D + c0 + c] : rows.w[h0 + t][c0 + c]) : 0.f;
+      smem[c * stride + TMAX + t] = t < Th ? sigmoid_fast(proto[(h0 + t) * D + c0 + c]) : 0.f;
     }
     __syncthreads();
     // warp wid handles channels wid, wid + 8, ... of the chunk; U channel rows in flight per lane
@@ -121,7 +132,7 @@ __global__ void __launch_bounds__(32 * kSeenWarps, (TMAX * PX <= 32 ? 3 : (TMAX 
             const float4 v = row[k];
             tab[4 * k] = v.x; tab[4 * k + 1] = v.y; tab[4 * k + 2] = v.z; tab[4 * k + 3] = v.w;
           }
-          // heads t >= Tn have weight 0 in the table: no predicate in the inner loop
+          // heads t >= Th have weight 0 in the table: no predicate in the inner loop
 #pragma unroll
           for (int t = 0; t < TMAX; ++t) {
             if constexpr (PX % 2 == 0) {
@@ -148,13 +159,13 @@ __global__ void __launch_bounds__(32 * kSeenWarps, (TMAX * PX <= 32 ? 3 : (TMAX 
   float* red = smem;
 #pragma unroll
   for (int t = 0; t < TMAX; ++t)
-    if (t < Tn) {
+    if (t < Th) {
 #pragma unroll
-      for (int i = 0; i < PX; ++i) red[(wid * Tn + t) * PS + lane * PX + i] = acc[i][t];
+      for (int i = 0; i < PX; ++i) red[(wid * Th + t) * PS + lane * PX + i] = acc[i][t];
     }
   __syncthreads();
-  float* xfer = smem + kSeenWarps * Tn * PS;  // [cs][Tn][PS] in the leader's shared memory
-  const int n_out = Tn * PS;
+  float* xfer = smem + kSeenWarps * Th * PS;  // [cs][Th][PS] in the leader's shared memory
+  const int n_out = Th * PS;
   if (cs > 1) {
     // non-leaders push their CTA sums into the leader's xfer[rank]
     uint32_t remote;
@@ -174,14 +185,14 @@ __global__ void __launch_bounds__(32 * kSeenWarps, (TMAX * PX <= 32 ? 3 : (TMAX 
   }
   for (int e = tid; e < n_out; e += 32 * kSeenWarps) {
     const int t = e / PS, px = e - t * PS;
-    float s = weight ? bias[t] : rows.b[t][0];
+    float s = weight ? bias[h0 + t] : rows.b[h0 + t][0];
 #pragma unroll
     for (int g = 0; g < kSeenWarps; ++g) s += red[g * n_out + e];
     for (int r = 1; r < cs; ++r) s += xfer[(size_t)r * n_out + e];
     const int q = pb * PS + px;
     if (q < hw) {
-      z[((int64_t)b * Tn + t) * hw + q] = s;
-      if (zero_out && t == 0) zero_out[(int64_t)b * hw + q] = 0.f;   // accumulator of the following pixel kernel
+      z[((int64_t)b * Tn + h0 + t) * hw + q] = s;
+      if (zero_out && h0 + t == 0) zero_out[(int64_t)b * hw + q] = 0.f;   // accumulator of the following pixel kernel
     }
   }
 }
@@ -376,15 +387,20 @@ __global__ void focal_scale_loss_kernel(const double* __restrict__ acc, const in
 
 using namespace bacs;
 
-extern "C" {
-
+// MANY: bacs_seen_logits_many, chunks of 32 heads over the grid's z dimension (the T = 32 plan per chunk).
+template <bool MANY>
 static int seen_logits_impl(const void* features, int dtype, int B, int D, int h, int w, const float* proto,
-                            const float* weight, const float* bias, const HeadRows& rows, int T, float* z,
+                            const float* weight, const float* bias,
+                            const std::conditional_t<MANY, HeadRowsMany, HeadRows>& rows, int T, float* z,
                             float* zero_out, bacs_stream_t stream) {
-  BACS_REQUIRE(B > 0 && B < 65536 && D > 0 && h > 0 && w > 0, "bacs_seen_logits: bad shape");
-  BACS_REQUIRE(T > 0 && T <= 32, "bacs_seen_logits: T=%d not in [1,32]", T);
+  const char* name = MANY ? "bacs_seen_logits_many" : "bacs_seen_logits";
+  BACS_REQUIRE(B > 0 && B < 65536 && D > 0 && h > 0 && w > 0, "%s: bad shape", name);
+  if (MANY) BACS_REQUIRE(T > 0 && T <= kMaxTasks, "%s: T=%d not in [1,%d]", name, T, kMaxTasks);
+  else BACS_REQUIRE(T > 0 && T <= 32, "%s: T=%d not in [1,32]", name, T);
   const int hw = h * w;
-  const int tmax = T <= 2 ? 2 : (T <= 4 ? 4 : (T <= 6 ? 6 : (T <= 8 ? 8 : (T <= 12 ? 12 : (T <= 16 ? 16 : 32)))));
+  const int n_ch = (T + 31) / 32;          // chunks of 32 heads (MANY), else 1
+  const int th = MANY ? std::min(T, 32) : T;  // heads per CTA
+  const int tmax = MANY ? 32 : (T <= 2 ? 2 : (T <= 4 ? 4 : (T <= 6 ? 6 : (T <= 8 ? 8 : (T <= 12 ? 12 : (T <= 16 ? 16 : 32))))));
   int px = tmax <= 8 ? 4 : (tmax <= 16 ? 2 : 1);   // measured: 4 pixels x 12 heads (112 registers) is slower than 2 x 12
   const size_t es = dtype_size(dtype);
   if (hw % px != 0 || (reinterpret_cast<uintptr_t>(features) % (px * es)) != 0) px = 1;
@@ -393,18 +409,19 @@ static int seen_logits_impl(const void* features, int dtype, int B, int D, int h
   // cluster size: split the channels while the whole grid still fits the machine in one wave
   const int per_sm = tmax * px <= 32 ? 3 : (tmax * px <= 48 ? 2 : 1);  // resident CTAs (register budget, see the kernel)
   int cs = 1;
-  while (cs < 8 && (int64_t)n_pb * B * cs * 2 <= (int64_t)per_sm * sm_count() && D / (2 * cs) >= 2 * kSeenWarps) cs *= 2;
+  while (cs < 8 && (int64_t)n_pb * B * n_ch * cs * 2 <= (int64_t)per_sm * sm_count() && D / (2 * cs) >= 2 * kSeenWarps)
+    cs *= 2;
   const int stride = 2 * tmax;
   const int per = (D + cs - 1) / cs;
   int chunk = (32 * 1024 / 4) / stride;  // table of <= 32 KB
   chunk = std::max(kSeenWarps, chunk / kSeenWarps * kSeenWarps);
   if (chunk > per) chunk = (per + kSeenWarps - 1) / kSeenWarps * kSeenWarps;
   const size_t table = (size_t)chunk * stride * sizeof(float);
-  const size_t red = (size_t)(kSeenWarps + cs) * T * ps * sizeof(float);
+  const size_t red = (size_t)(kSeenWarps + cs) * th * ps * sizeof(float);
   const size_t smem = std::max(table, red);
   cudaStream_t s = (cudaStream_t)stream;
   cudaLaunchConfig_t cfg = {};
-  cfg.gridDim = dim3((unsigned)(n_pb * cs), (unsigned)B);
+  cfg.gridDim = dim3((unsigned)(n_pb * cs), (unsigned)B, (unsigned)n_ch);
   cfg.blockDim = dim3(32 * kSeenWarps);
   cfg.dynamicSmemBytes = smem;
   cfg.stream = s;
@@ -419,18 +436,18 @@ static int seen_logits_impl(const void* features, int dtype, int B, int D, int h
   cfg.numAttrs = 2;
 #define LAUNCH_Z(TT, TM, PXV)                                                                                     \
   do {                                                                                                            \
-    auto kern = seen_logits_kernel<TT, TM, PXV>;                                                                  \
+    auto kern = seen_logits_kernel<TT, TM, PXV, MANY>;                                                            \
     if (smem > 48 * 1024) {                                                                                       \
       cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);         \
       if (e != cudaSuccess) {                                                                                     \
-        set_error("bacs_seen_logits: shared memory opt-in failed: %s", cudaGetErrorString(e));                   \
+        set_error("%s: shared memory opt-in failed: %s", name, cudaGetErrorString(e));                           \
         return BACS_ERR_CUDA;                                                                                     \
       }                                                                                                           \
     }                                                                                                             \
     cudaError_t le = cudaLaunchKernelEx(&cfg, kern, reinterpret_cast<const TT*>(features), D, hw, proto, weight,  \
                                         bias, T, chunk, cs, z, rows, zero_out);                                   \
     if (le != cudaSuccess) {                                                                                      \
-      set_error("bacs_seen_logits: launch failed: %s", cudaGetErrorString(le));                                  \
+      set_error("%s: launch failed: %s", name, cudaGetErrorString(le));                                          \
       return BACS_ERR_CUDA;                                                                                       \
     }                                                                                                             \
   } while (0)
@@ -440,7 +457,8 @@ static int seen_logits_impl(const void* features, int dtype, int B, int D, int h
     else LAUNCH_Z(TT, TM, PXV);      \
   } while (0)
   BACS_DISPATCH_DTYPE(dtype, TT, {
-    if (tmax == 2) LAUNCH_Z_PX(TT, 2, 4);
+    if constexpr (MANY) LAUNCH_Z(TT, 32, 1);
+    else if (tmax == 2) LAUNCH_Z_PX(TT, 2, 4);
     else if (tmax == 4) LAUNCH_Z_PX(TT, 4, 4);
     else if (tmax == 6) LAUNCH_Z_PX(TT, 6, 4);
     else if (tmax == 8) LAUNCH_Z_PX(TT, 8, 4);
@@ -450,15 +468,17 @@ static int seen_logits_impl(const void* features, int dtype, int B, int D, int h
   });
 #undef LAUNCH_Z_PX
 #undef LAUNCH_Z
-  BACS_CHECK_LAUNCH("bacs_seen_logits");
+  BACS_CHECK_LAUNCH(name);
   return BACS_OK;
 }
+
+extern "C" {
 
 int bacs_seen_logits(const void* features, int dtype, int B, int D, int h, int w, const float* proto,
                      const float* weight, const float* bias, int T, float* z, bacs_stream_t stream) {
   BACS_REQUIRE(features && proto && weight && bias && z, "bacs_seen_logits: null pointer");
   HeadRows rows = {};
-  return seen_logits_impl(features, dtype, B, D, h, w, proto, weight, bias, rows, T, z, nullptr, stream);
+  return seen_logits_impl<false>(features, dtype, B, D, h, w, proto, weight, bias, rows, T, z, nullptr, stream);
 }
 
 int bacs_seen_logits_heads(const void* features, int dtype, int B, int D, int h, int w, const float* proto,
@@ -472,7 +492,27 @@ int bacs_seen_logits_heads(const void* features, int dtype, int B, int D, int h,
     rows.w[t] = weight_rows_host[t];
     rows.b[t] = bias_host[t];
   }
-  return seen_logits_impl(features, dtype, B, D, h, w, proto, nullptr, nullptr, rows, T, z, zero_out, stream);
+  return seen_logits_impl<false>(features, dtype, B, D, h, w, proto, nullptr, nullptr, rows, T, z, zero_out, stream);
+}
+
+int bacs_seen_logits_many(const void* features, int dtype, int B, int D, int h, int w, const float* proto,
+                          const float* weight, const float* bias, const float* const* weight_rows_host,
+                          const float* const* bias_host, int T, float* z, float* zero_out, bacs_stream_t stream) {
+  BACS_REQUIRE(features && proto && z, "bacs_seen_logits_many: null pointer");
+  BACS_REQUIRE(T > 0 && T <= kMaxTasks, "bacs_seen_logits_many: T=%d not in [1,%d]", T, kMaxTasks);
+  HeadRowsMany rows = {};
+  if (weight_rows_host) {   // the heads' own parameters
+    BACS_REQUIRE(bias_host, "bacs_seen_logits_many: null pointer");
+    for (int t = 0; t < T; ++t) {
+      BACS_REQUIRE(weight_rows_host[t] && bias_host[t], "bacs_seen_logits_many: null head %d", t);
+      rows.w[t] = weight_rows_host[t];
+      rows.b[t] = bias_host[t];
+    }
+    weight = bias = nullptr;
+  } else {                  // stacked weight [T,D] and bias [T]
+    BACS_REQUIRE(weight && bias, "bacs_seen_logits_many: null pointer");
+  }
+  return seen_logits_impl<true>(features, dtype, B, D, h, w, proto, weight, bias, rows, T, z, zero_out, stream);
 }
 
 int bacs_seen_upsample(const float* z, int B, int T, int h, int w, int scale, int apply_sigmoid, float* out,

@@ -123,10 +123,10 @@ _peer_reducers = {}
 
 
 def peer_reducer(n: int, device: torch.device) -> "Optional[PeerReducer]":
-    """Cached per device; sized for the largest state of the reference's settings (64 tasks)."""
+    """Cached per device; sized for the largest prototype state the kernels take (128 tasks x 2048 channels)."""
     key = (device.index, world_size())
     if key not in _peer_reducers:
-        _peer_reducers[key] = PeerReducer.create(max(int(n), 64 * 2048 + 64), device)
+        _peer_reducers[key] = PeerReducer.create(max(int(n), 128 * 2048 + 128), device)
     red = _peer_reducers[key]
     return red if (red is not None and n <= red.n_max) else None
 

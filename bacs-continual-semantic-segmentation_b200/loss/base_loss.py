@@ -182,6 +182,8 @@ class BaseLoss:
         ``return_attentions and train``, ``(loss, logits, old_atts, attentions, seen_map)``
         where ``seen_map`` is a :class:`SeenMap` (call ``.materialize()`` for the tensor)."""
         old_atts, attentions, seen_map = None, None, None
+        if self._prototypes is not None and self._prototypes._prototypes_tensors is not None:
+            ops.check_task_count(self._prototypes._prototypes_tensors.shape[0], "compute_base_loss")
         is_experience_replay = task_num != -1
         if self.weighted_ce.old_cl != self.old_classes:      # (nn.Module.__setattr__ is slow: only on change)
             self.weighted_ce.old_cl = self.old_classes
@@ -220,13 +222,15 @@ class BaseLoss:
                 if train_seen_detector:
                     cfg["gz"] = torch.empty((penultimate_output.shape[0],) + tuple(penultimate_output.shape[2:]),
                                             dtype=torch.float32, device=penultimate_output.device)
-                z = ops.seen_logits_heads(penultimate_output.detach(), protos[:n_eval],
-                                          [p.detach() for p in params[:n_eval]], [p.detach() for p in params[n_eval:]],
-                                          zero_out=cfg.get("gz"))
+                # more than 32 heads (continual runs longer than 32 tasks): the chunked kernel
+                seen = ops.seen_logits_many if n_eval > 32 else ops.seen_logits_heads
+                z = seen(penultimate_output.detach(), protos[:n_eval], [p.detach() for p in params[:n_eval]],
+                         [p.detach() for p in params[n_eval:]], zero_out=cfg.get("gz"))
             else:
                 weight, bias = self._stack_heads(seen_net, protos.shape[0])
                 n_eval = weight.shape[0]
-                z = ops.seen_logits(penultimate_output.detach(), protos[:n_eval], weight, bias)
+                seen = ops.seen_logits_many if n_eval > 32 else ops.seen_logits
+                z = seen(penultimate_output.detach(), protos[:n_eval], weight, bias)
             cfg["z"] = z
             cfg["proto"] = protos
         if wce_on:

@@ -151,7 +151,7 @@ class Prototypes(BaseLoss):
         """Inspection helper with the reference's return shape (prototypes.py:177-205);
         synchronises (torch.unique) and is not used by update_feats_prototypes."""
         B, D, h, w = features.shape
-        T = 32
+        T = ops.MAX_TASKS
         lut = self._device_task_lut(features.device, T)
         labels = target if labels_down is None else labels_down.reshape(B, h, w)
         _, _, _, down = ops.label_downsample_task(labels.long(), h, w, lut, T, want_labels_down=True)

@@ -113,7 +113,8 @@ class BgDetector(nn.Module):
     def forward_seen_before_lowres(self, x, prototypes):
         """All heads at feature resolution in one kernel (no gradient): [B,T,h,w]."""
         w, b = self._stacked(prototypes.shape[0])
-        return ops.seen_logits(x.detach(), prototypes[:w.shape[0]].detach(), w, b)
+        seen = ops.seen_logits_many if w.shape[0] > 32 else ops.seen_logits
+        return seen(x.detach(), prototypes[:w.shape[0]].detach(), w, b)
 
     def forward_seen_before(self, x, prototypes):
         """bg_detector.py:119-139 (no gradient -- the loss only uses it under no_grad)."""

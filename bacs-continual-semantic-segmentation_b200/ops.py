@@ -56,6 +56,16 @@ def _ws(nbytes: int, device) -> torch.Tensor:
     return torch.empty(max(int(nbytes), 16), dtype=torch.uint8, device=device)
 
 
+MAX_TASKS = 128   # BACS_MAX_TASKS: the int8 task map holds task ids 0..127
+
+
+def check_task_count(T: int, name: str) -> None:
+    """Raises BacsError unless 1 <= T <= MAX_TASKS (before any launch)."""
+    if not 1 <= T <= MAX_TASKS:
+        raise _cabi.BacsError("bacs_b200.%s: %d tasks; the task count must lie in [1, %d] (int8 task map)"
+                              % (name, T, MAX_TASKS))
+
+
 # --------------------------------------------------------------------------------------
 # labels
 # --------------------------------------------------------------------------------------
@@ -89,6 +99,7 @@ def label_remap(labels: torch.Tensor, map1: torch.Tensor, masking1: int, map2: O
 
 def label_downsample_task(labels: torch.Tensor, h: int, w: int, task_lut: torch.Tensor, T: int,
                           want_labels_down: bool = False):
+    check_task_count(T, "label_downsample_task")
     labels = _cuda(labels, "label_downsample_task", torch.int64)
     task_lut = _cuda(task_lut, "label_downsample_task", torch.int32)
     B, H, W = labels.shape
@@ -110,6 +121,7 @@ def proto_accumulate(features: torch.Tensor, task: torch.Tensor, rank: torch.Ten
                      mode: int = 0, out: Optional[torch.Tensor] = None) -> Tuple[torch.Tensor, torch.Tensor]:
     """Returns (sums fp64 [T,D], counts fp64 [T]) as two views of ONE packed fp64 buffer
     [T*D + T] so that a single all-reduce moves both."""
+    check_task_count(T, "proto_accumulate")
     features = _cuda(features, "proto_accumulate")
     B, D, h, w = features.shape
     dev = features.device
@@ -128,6 +140,7 @@ def proto_accumulate_update(features: torch.Tensor, task: torch.Tensor, rank: to
                             ready: Optional[torch.Tensor] = None) -> Tuple[torch.Tensor, torch.Tensor, torch.Tensor]:
     """proto_accumulate + proto_update without a launch of its own for the update (single-process step).
     Returns (sums, counts, ready)."""
+    check_task_count(proto.shape[0], "proto_accumulate_update")
     features = _cuda(features, "proto_accumulate_update")
     proto = _cuda(proto, "proto_accumulate_update", torch.float32)
     if not proto.is_contiguous() or not count.is_contiguous():
@@ -152,6 +165,7 @@ def proto_accumulate_update(features: torch.Tensor, task: torch.Tensor, rank: to
 
 def proto_update(proto: torch.Tensor, count: torch.Tensor, sums: torch.Tensor, counts: torch.Tensor,
                  ready: Optional[torch.Tensor] = None) -> torch.Tensor:
+    check_task_count(proto.shape[0], "proto_update")
     proto = _cuda(proto, "proto_update", torch.float32)
     if not proto.is_contiguous() or not count.is_contiguous():
         raise ValueError("proto_update works in place: proto and count must be contiguous")
@@ -205,6 +219,48 @@ def seen_logits_heads(features: torch.Tensor, proto: torch.Tensor, weights: Sequ
     z = torch.empty((B, T, h, w), dtype=torch.float32, device=features.device)
     check(_lib().bacs_seen_logits_heads(features.data_ptr(), _dt(features), B, D, h, w, proto.data_ptr(), wp, bp, T,
                                         z.data_ptr(), _ptr(zero_out), _stream()), "bacs_seen_logits_heads")
+    return z
+
+
+def seen_logits_many(features: torch.Tensor, proto: torch.Tensor, weight, bias,
+                     zero_out: Optional[torch.Tensor] = None) -> torch.Tensor:
+    """seen_logits for any head count up to MAX_TASKS (seen_logits / seen_logits_heads take at most 32).  ``weight`` /
+    ``bias`` are either the stacked fp32 [T,D] / [T] tensors of seen_logits or the per-head sequences of
+    seen_logits_heads; ``zero_out`` as in seen_logits_heads."""
+    stacked = isinstance(weight, torch.Tensor)
+    T = weight.shape[0] if stacked else len(weight)
+    check_task_count(T, "seen_logits_many")
+    features = _cuda(features, "seen_logits_many")
+    proto = _cuda(proto.float(), "seen_logits_many")
+    B, D, h, w = features.shape
+    if stacked:
+        weight = _cuda(weight.float(), "seen_logits_many")
+        bias = _cuda(bias.float(), "seen_logits_many")
+        if tuple(weight.shape) != (T, D) or bias.numel() != T:
+            raise ValueError("seen_logits_many: weight must be [T,D=%d] and bias [T]" % D)
+    else:
+        if T != len(bias):
+            raise ValueError("seen_logits_many: %d weights, %d biases" % (T, len(bias)))
+        for t in list(weight) + list(bias):
+            if t.dtype != torch.float32 or not t.is_cuda or not t.is_contiguous():
+                raise TypeError("seen_logits_many: head parameters must be contiguous fp32 CUDA tensors")
+        if any(wt.numel() != D for wt in weight):
+            raise ValueError("seen_logits_many: a head weight does not have D=%d entries" % D)
+    if T > proto.shape[0]:
+        raise ValueError("seen_logits_many: %d heads, %d prototypes" % (T, proto.shape[0]))
+    if zero_out is not None and (zero_out.dtype != torch.float32 or tuple(zero_out.shape) != (B, h, w)
+                                 or not zero_out.is_contiguous()):
+        raise ValueError("seen_logits_many: zero_out must be a contiguous fp32 [B,h,w] tensor")
+    if stacked:
+        wp = bp = None
+        wd, bd = weight.data_ptr(), bias.data_ptr()
+    else:
+        wp = (C.c_void_p * T)(*[wt.data_ptr() for wt in weight])
+        bp = (C.c_void_p * T)(*[bt.data_ptr() for bt in bias])
+        wd = bd = None
+    z = torch.empty((B, T, h, w), dtype=torch.float32, device=features.device)
+    check(_lib().bacs_seen_logits_many(features.data_ptr(), _dt(features), B, D, h, w, proto.data_ptr(), wd, bd, wp, bp,
+                                       T, z.data_ptr(), _ptr(zero_out), _stream()), "bacs_seen_logits_many")
     return z
 
 

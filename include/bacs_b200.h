@@ -38,6 +38,11 @@ enum bacs_status {
 
 enum bacs_dtype { BACS_F32 = 0, BACS_BF16 = 1, BACS_F16 = 2 };
 
+/* Largest task count T of the task down-sample, the prototype sums and update, the peer all-reduce's prototype update
+ * and bacs_seen_logits_many: the range of the int8 task map (ids 0..127, -1 = no task).  bacs_seen_logits and
+ * bacs_seen_logits_heads take at most 32 heads. */
+#define BACS_MAX_TASKS 128
+
 int bacs_version(void);
 const char* bacs_last_error_string(void);
 /* number of SMs of the current device (grid sizing by the host side) */
@@ -139,6 +144,17 @@ int bacs_seen_logits_heads(const void* features, int dtype, int B, int D, int h,
                            const float* proto, const float* const* weight_rows_host,
                            const float* const* bias_host, int T, float* z, float* zero_out,
                            bacs_stream_t stream);
+
+/* Any number of heads 1 <= T <= BACS_MAX_TASKS (continual runs longer than 32 tasks).  The heads come as host arrays
+ * of device pointers as in bacs_seen_logits_heads, or, when weight_rows_host is NULL, stacked as weight fp32[T,D] and
+ * bias fp32[T] as in bacs_seen_logits.  zero_out as in bacs_seen_logits_heads (may be NULL).  One launch: a grid
+ * dimension over chunks of 32 heads, each evaluated with the T = 32 plan of bacs_seen_logits; the chunks after the
+ * first read the features mostly from L2.  At T <= 32 the result equals bacs_seen_logits' bit for bit when both
+ * launches split the channels over the same cluster size. */
+int bacs_seen_logits_many(const void* features, int dtype, int B, int D, int h, int w,
+                          const float* proto, const float* weight, const float* bias,
+                          const float* const* weight_rows_host, const float* const* bias_host, int T,
+                          float* z, float* zero_out, bacs_stream_t stream);
 
 /* Materialised seen logits of the reference for callers that need the full-res map
  * (get_seen_map_task / get_seen_probs, bg_detector.py:100-165): out[b,t,Y,X] =
