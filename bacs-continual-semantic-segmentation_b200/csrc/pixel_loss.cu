@@ -476,7 +476,7 @@ __global__ void __launch_bounds__(kConsumers + 32, PPT == 1 ? 2 : 1) pixel_loss_
       }
       if (a.distill_mask) {
         uint8_t* out = a.distill_mask + (int64_t)b * HW + p0 + px0;
-        if (PPT == 2 && px0 + 1 < npx) {
+        if (PPT == 2 && px0 + 1 < npx && ((reinterpret_cast<uintptr_t>(out) & 1) == 0)) {
           *reinterpret_cast<uchar2*>(out) = make_uchar2(dmask[0], dmask[PPT - 1]);
         } else {
 #pragma unroll
@@ -989,8 +989,11 @@ static int check_pixel_args(const bacs_pixel_args* a, const char* fn) {
   if (a->mode == BACS_PIX_WEIGHTED_CE)
     BACS_REQUIRE(a->old_cl >= 1 && (a->z || a->seen_max),
                  "%s: WEIGHTED_CE needs old_cl >= 1 and the seen logits / probabilities", fn);
-  if (a->mode != BACS_PIX_WEIGHTED_CE && a->dlogits)
+  if (a->mode != BACS_PIX_WEIGHTED_CE && a->dlogits) {
     BACS_REQUIRE(a->hist, "%s: CE-type gradients need the label histogram", fn);
+    // the normaliser sums hist[c] over the classes: the 257-bin histogram counts labels >= 256 together
+    BACS_REQUIRE(a->K <= 256, "%s: CE-type gradients need K <= 256 (the 257-bin label histogram), K=%d", fn, a->K);
+  }
   if (a->mode == BACS_PIX_SCORE)
     BACS_REQUIRE(a->score && !a->dlogits, "%s: SCORE mode needs score and no gradient", fn);
   return BACS_OK;

@@ -231,7 +231,9 @@ typedef struct bacs_pixel_args {
                              accumulated (caller zeroes), or NULL = no focal term */
   const float* class_w;   /* [K] class weights (CE / SCORE modes) or NULL = ones */
   const int64_t* hist;    /* [257] label histogram: needed when class_w != NULL or mode is
-                             CE/UNBIASED_CE and dlogits != NULL (gradient normaliser) */
+                             CE/UNBIASED_CE and dlogits != NULL (gradient normaliser); such a
+                             gradient request needs K <= 256, since the histogram's last bin
+                             counts every label >= 256 together */
   double* acc;            /* [BACS_NACC] OVERWRITTEN with the reduced accumulators */
   double* score;          /* [B] per-image score (SCORE mode), or NULL */
   int32_t B, K, H, W, T, h, w;

@@ -102,6 +102,7 @@ INVALID = [
     pytest.param(dict(gz=GZ), id="focal-without-z"),
     pytest.param(dict(mode=_cabi.PIX_WEIGHTED_CE, old_cl=16), id="wce-without-seen"),
     pytest.param(dict(hist=None), id="ce-grad-without-hist"),
+    pytest.param(dict(K=300, ignore_index=-1), id="ce-grad-K300"),
     pytest.param(_score(score=None), id="score-without-score"),
     pytest.param(_score(dlogits=DLOGITS), id="score-with-grad"),
 ]
