@@ -46,6 +46,9 @@ _SIGNATURES = {
     "bacs_proto_accumulate": (i32, [vp, i32, i32, i32, i32, i32, vp, vp, vp, i32, i32, vp, vp, vp, sz, vp]),
     "bacs_proto_accumulate_update": (i32, [vp, i32, i32, i32, i32, i32, vp, vp, vp, i32, i32, vp, vp, vp, sz, vp, vp, i32,
                                            vp, vp]),
+    "bacs_proto_accumulate_view": (i32, [vp, i32, i32, i32, i32, i32, vp, vp, vp, i32, i32, vp, vp, vp, vp, vp, sz, vp]),
+    "bacs_proto_task_totals": (i32, [vp, i32, i32, vp, vp]),
+    "bacs_proto_count_view": (i32, [vp, i32, i32, i32, vp, vp, vp]),
     "bacs_proto_update": (i32, [vp, vp, i32, vp, vp, i32, i32, vp, vp]),
     "bacs_seen_logits": (i32, [vp, i32, i32, i32, i32, i32, vp, vp, vp, i32, vp, vp]),
     "bacs_seen_logits_heads": (i32, [vp, i32, i32, i32, i32, i32, vp, vp, vp, i32, vp, vp, vp]),
@@ -82,6 +85,8 @@ _SIGNATURES = {
     "bacs_scale_inplace_multi": (i32, [i32, C.POINTER(vp), C.POINTER(i32), C.POINTER(i64), vp, vp]),
     "bacs_peer_allreduce": (i32, [vp, i32, i32, i32, i32, C.POINTER(C.c_uint64), C.POINTER(C.c_uint64), vp, vp, vp, vp, i32,
                                   i32, i32, vp, vp]),
+    "bacs_peer_count_exchange": (i32, [vp, i32, i32, i32, i32, C.POINTER(C.c_uint64), C.POINTER(C.c_uint64), vp, vp, vp,
+                                       vp, vp]),
     "bacs_peer_set_timeout_ms": (i32, [i64]),
     "bacs_pack_state": (i32, [vp, vp, i32, i32, vp, i32, vp, vp]),
     "bacs_unpack_state": (i32, [vp, i32, i32, vp, vp, vp, i32, vp]),

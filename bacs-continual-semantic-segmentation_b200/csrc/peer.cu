@@ -15,6 +15,14 @@
 // (distributed.PeerReducer.check).  A rank never applies a sum that may contain a stale or half-written peer slot.
 // A peer can only be one step ahead (it needs my flag of step e+1 to finish step e+1), and it then writes the
 // OTHER parity slot, so reads of step e never race with writes of step e+1.
+//
+// Count phase (global view of the exact-mode prototype sums, before the accumulate launch): every rank pushes its
+// task totals sum_b n_bt[b][t] into row `rank` of every peer's count table (double-buffered by the parity of a step
+// counter of its own), publishes with a release-store into the peers' count-flag rows (apart from the flags of the sums
+// phase), waits for every peer as above, then sums its local table in rank order into view_pre (ranks below) and view_n
+// (all ranks).  On a time-out the view is marked invalid (view_n = -1): the accumulate launch then adds nothing and
+// writes -inf counts, so the running-mean update that follows leaves every prototype and count untouched on this rank
+// (and on every rank that combines its state); the sticky error word receives the count step as above.
 #include "common.cuh"
 
 namespace bacs {
@@ -163,11 +171,90 @@ __global__ void __launch_bounds__(1024) peer_allreduce_update_kernel(PeerPtrs pp
   if (threadIdx.x == 0 && ready) *ready = (s_nonzero == Tn) ? 1 : 0;
 }
 
+__global__ void __launch_bounds__(kMaxTasks) peer_count_exchange_kernel(PeerPtrs pp, int rank, int world,
+                                                                       unsigned long long timeout_ns,
+                                                                       const int32_t* __restrict__ n_bt, int B, int Tn,
+                                                                       unsigned int* __restrict__ step_dev,
+                                                                       int* __restrict__ error_dev,
+                                                                       long long* __restrict__ view_pre,
+                                                                       long long* __restrict__ view_n) {
+  __shared__ long long s_tot[kMaxTasks];
+  __shared__ int s_timeout;
+  pdl_wait();     // n_bt comes from the task down-sample
+  pdl_trigger();  // the accumulate launch waits for this grid's completion itself
+  const unsigned int step = *step_dev + 1u;
+  const size_t slot = (size_t)(step & 1u) * world * kMaxTasks;   // table: [2][world][kMaxTasks] int64 per rank
+  if (threadIdx.x == 0) s_timeout = 0;
+  if (threadIdx.x < Tn) {
+    long long n = 0;
+    for (int bb = 0; bb < B; ++bb) n += n_bt[bb * Tn + threadIdx.x];
+    s_tot[threadIdx.x] = n;
+  }
+  __syncthreads();
+  for (int i = threadIdx.x; i < world * Tn; i += blockDim.x) {
+    const int r = i / Tn, t = i - r * Tn;
+    reinterpret_cast<long long*>(pp.buf[r])[slot + (size_t)rank * kMaxTasks + t] = s_tot[t];
+  }
+  __threadfence_system();
+  __syncthreads();
+  if (threadIdx.x < world) {
+    st_release_sys(pp.flag[threadIdx.x] + rank, step);
+    const unsigned int* f = pp.flag[rank] + threadIdx.x;
+    const unsigned long long t0 = global_timer_ns();
+    unsigned int polls = 0;
+    while ((int)(ld_acquire_sys(f) - step) < 0) {
+      if ((++polls & 1023u) == 0 && global_timer_ns() - t0 > timeout_ns) {
+        s_timeout = 1;
+        break;
+      }
+    }
+  }
+  __syncthreads();
+  if (threadIdx.x == 0) *step_dev = step;
+  if (threadIdx.x >= Tn) return;
+  const int t = threadIdx.x;
+  if (s_timeout) {
+    if (t == 0 && error_dev) *error_dev = (int)step;
+    view_pre[t] = 0;
+    view_n[t] = -1;
+    return;
+  }
+  const double* mine = pp.buf[rank] + slot + t;
+  long long pre = 0, n = 0;
+  for (int r = 0; r < world; ++r) {   // rank order: the images of rank r come after those of ranks 0 .. r-1
+    const long long v = __double_as_longlong(ld_relaxed_sys_f64(mine + (size_t)r * kMaxTasks));
+    if (r < rank) pre += v;
+    n += v;
+  }
+  view_pre[t] = pre;
+  view_n[t] = n;
+}
+
 }  // namespace bacs
 
 using namespace bacs;
 
 extern "C" {
+
+int bacs_peer_count_exchange(const int32_t* n_bt, int B, int T, int rank, int world, const uint64_t* peer_table_host,
+                             const uint64_t* peer_flag_host, uint32_t* step_dev, int32_t* error_dev, int64_t* view_pre,
+                             int64_t* view_n, bacs_stream_t stream) {
+  BACS_REQUIRE(n_bt && peer_table_host && peer_flag_host && step_dev && view_pre && view_n,
+               "bacs_peer_count_exchange: null pointer");
+  BACS_REQUIRE(world >= 1 && world <= kPeerMaxWorld && rank >= 0 && rank < world, "bacs_peer_count_exchange: bad rank/world");
+  BACS_REQUIRE(B > 0, "bacs_peer_count_exchange: bad shape");
+  BACS_REQUIRE(T > 0 && T <= kMaxTasks, "bacs_peer_count_exchange: T=%d not in [1,%d]", T, kMaxTasks);
+  PeerPtrs pp;
+  for (int r = 0; r < kPeerMaxWorld; ++r) {
+    pp.buf[r] = r < world ? reinterpret_cast<double*>(peer_table_host[r]) : nullptr;
+    pp.flag[r] = r < world ? reinterpret_cast<unsigned int*>(peer_flag_host[r]) : nullptr;
+  }
+  launch_pdl(peer_count_exchange_kernel, dim3(1), dim3(kMaxTasks), 0, (cudaStream_t)stream, pp, rank, world,
+             g_peer_timeout_ns, n_bt, B, T, step_dev, error_dev, reinterpret_cast<long long*>(view_pre),
+             reinterpret_cast<long long*>(view_n));
+  BACS_CHECK_LAUNCH("bacs_peer_count_exchange");
+  return BACS_OK;
+}
 
 int bacs_peer_set_timeout_ms(int64_t ms) {
   BACS_REQUIRE(ms > 0, "bacs_peer_set_timeout_ms: the time-out must be positive");

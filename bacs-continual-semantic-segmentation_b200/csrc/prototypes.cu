@@ -14,11 +14,16 @@ namespace bacs {
 // Each lane accumulates into its own column of a warp-private shared-memory table
 // acc[task][low/high][lane] (conflict-free, no atomics): a pixel touches exactly one entry, so
 // the cost per element does not grow with the number of tasks.
+// VIEW (global view of a data-parallel batch, exact mode): pre and N_g also count the masked pixels of the images of
+// other ranks -- view_pre[g] (images of lower ranks, added to pre) and view_n[g] (all ranks, in place of N_g) -- so the
+// rows are those of one process fed every rank's images in rank order.  view_n[g] < 0 marks a view that could not be
+// formed (peer time-out): such a task adds nothing and its count comes out as -inf, which makes every later running-mean
+// update skip it.
 // MANY (more than kTaskWindow tasks): blockIdx.z picks a window of kTaskWindow tasks; the block sums only the pixels of
 // those tasks and writes their columns, so its shared memory and split bookkeeping are those of a 32-task launch.
 constexpr int kAccWarps = 8;
 constexpr int kTaskWindow = 32;
-template <typename T, bool MANY = false>
+template <typename T, bool MANY = false, bool VIEW = false>
 __global__ void __launch_bounds__(32 * kAccWarps) proto_accumulate_kernel(const T* __restrict__ feat, int B, int D,
                                                                           int hw, const int8_t* __restrict__ task,
                                                                           const int32_t* __restrict__ rank,
@@ -26,7 +31,9 @@ __global__ void __launch_bounds__(32 * kAccWarps) proto_accumulate_kernel(const 
                                                                           int mode,
                                                                           float* __restrict__ partial /* [B,D,Tn,2] */,
                                                                           const void* __restrict__ count_raw, int count_is_int64,
-                                                                          unsigned long long* __restrict__ count_snap) {
+                                                                          unsigned long long* __restrict__ count_snap,
+                                                                          const long long* __restrict__ view_pre,
+                                                                          const long long* __restrict__ view_n) {
   extern __shared__ float s_acc[];  // [warp][Tw][2][32]
   const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
   const int b = blockIdx.y;
@@ -49,6 +56,10 @@ __global__ void __launch_bounds__(32 * kAccWarps) proto_accumulate_kernel(const 
       const int n = n_bt[bb * Tn + t_lo + lane];
       if (bb < b) pre += n;
       tot += n;
+    }
+    if constexpr (VIEW) {
+      pre += view_pre[t_lo + lane];
+      tot = view_n[t_lo + lane];
     }
     const long long nb = n_bt[b * Tn + t_lo + lane];
     if (tot > 0) {
@@ -91,7 +102,7 @@ __global__ void __launch_bounds__(32 * kAccWarps) proto_accumulate_kernel(const 
 // Vectorised variant (hw a multiple of 8, 16-byte aligned rows): a lane handles 8 consecutive pixels per step; task
 // bytes and features of a row's first step are requested before the split points are worked out.  The per-warp table
 // has one 32-float row per (task, low / high) entry: a lane only ever touches its own bank.
-template <typename T, bool MANY = false>
+template <typename T, bool MANY = false, bool VIEW = false>
 __global__ void __launch_bounds__(32 * kAccWarps, 4) proto_accumulate_vec_kernel(const T* __restrict__ feat, int B, int D,
                                                                                  int hw, const int8_t* __restrict__ task,
                                                                                  const int32_t* __restrict__ rank,
@@ -99,7 +110,9 @@ __global__ void __launch_bounds__(32 * kAccWarps, 4) proto_accumulate_vec_kernel
                                                                                  int mode, float* __restrict__ partial,
                                                                                  const void* __restrict__ count_raw,
                                                                                  int count_is_int64,
-                                                                                 unsigned long long* __restrict__ count_snap) {
+                                                                                 unsigned long long* __restrict__ count_snap,
+                                                                                 const long long* __restrict__ view_pre,
+                                                                                 const long long* __restrict__ view_n) {
   extern __shared__ float s_acc[];  // [warp][Tw*2 + 2][32] | [warp][33] split points
   __shared__ long long s_pre[32], s_tot[32];  // per task: masked pixels in the images before b / in all images
   __shared__ int s_nb[32];
@@ -159,6 +172,10 @@ __global__ void __launch_bounds__(32 * kAccWarps, 4) proto_accumulate_vec_kernel
       }
       pre = warp_sum(pre);
       tot = warp_sum(tot);
+      if constexpr (VIEW) {
+        pre += view_pre[t_lo + t];
+        tot = view_n[t_lo + t];
+      }
       if (lane == 0) {
         s_pre[t] = pre;
         s_tot[t] = tot;
@@ -274,7 +291,7 @@ __device__ __forceinline__ void mma_16816(float (&d)[4], uint32_t a0, uint32_t a
                  : "r"(a0), "r"(a1), "r"(a2), "r"(a3), "r"(b0), "r"(b1));
 }
 
-template <typename T, int NT, bool MANY = false>  // NT = ceil(Tn / 8) task tiles (4 with MANY: one 32-task window)
+template <typename T, int NT, bool MANY = false, bool VIEW = false>  // NT = ceil(Tn / 8) task tiles (4 with MANY: one 32-task window)
 __global__ void __launch_bounds__(32 * kMmaWarps) proto_accumulate_mma_kernel(const T* __restrict__ feat, int B, int D, int hw,
                                                                               const int8_t* __restrict__ task,
                                                                               const int32_t* __restrict__ rank,
@@ -282,7 +299,9 @@ __global__ void __launch_bounds__(32 * kMmaWarps) proto_accumulate_mma_kernel(co
                                                                               double* __restrict__ sums /* [Tn][D], zeroed */,
                                                                               const void* __restrict__ count_raw,
                                                                               int count_is_int64,
-                                                                              unsigned long long* __restrict__ count_snap) {
+                                                                              unsigned long long* __restrict__ count_snap,
+                                                                              const long long* __restrict__ view_pre,
+                                                                              const long long* __restrict__ view_n) {
   static_assert(sizeof(T) == 2, "16-bit tensor-core operands");
   __shared__ long long s_pre[32], s_tot[32];
   __shared__ int s_nb[32];
@@ -330,6 +349,10 @@ __global__ void __launch_bounds__(32 * kMmaWarps) proto_accumulate_mma_kernel(co
       }
       pre = warp_sum(pre);
       tot = warp_sum(tot);
+      if constexpr (VIEW) {
+        pre += view_pre[t_lo + t];
+        tot = view_n[t_lo + t];
+      }
       if (lane == 0) {
         s_pre[t] = pre;
         s_tot[t] = tot;
@@ -387,7 +410,7 @@ __global__ void __launch_bounds__(32 * kMmaWarps) proto_accumulate_mma_kernel(co
           sp = is_split ? (int)spl : 0x7fffffff;
         }
       }
-      if (t < Tw && !is_split && d[nt][e] != 0.f) atomicAdd(sums + (int64_t)(t_lo + t) * D + row, (double)d[nt][e]);
+      if (t < Tw && !is_split && d[nt][e] != 0.f && (!VIEW || s_tot[t] > 0)) atomicAdd(sums + (int64_t)(t_lo + t) * D + row, (double)d[nt][e]);
       unsigned todo = __ballot_sync(0xffffffffu, is_split);
       while (todo) {
         const int src = __ffs(todo) - 1;
@@ -438,6 +461,7 @@ __global__ void __launch_bounds__(256) proto_zero_sums_kernel(double* __restrict
 constexpr int kFinMaxB = 1024;
 constexpr int kFinRows = 32;   // output rows per block
 constexpr int kFinLanes = 8;   // images are strided over this many threads per row
+template <bool VIEW = false>   // VIEW: rows of the global view (gather only, no fused update)
 __global__ void __launch_bounds__(kFinRows* kFinLanes) proto_finalize_kernel(const float* __restrict__ partial, int B,
                                                                             int D, const int32_t* __restrict__ n_bt,
                                                                             int Tn, int mode,
@@ -446,7 +470,9 @@ __global__ void __launch_bounds__(kFinRows* kFinLanes) proto_finalize_kernel(con
                                                                             float* __restrict__ proto, void* __restrict__ count,
                                                                             int count_is_int64,
                                                                             const unsigned long long* __restrict__ count_snap,
-                                                                            int32_t* __restrict__ ready, int gather) {
+                                                                            int32_t* __restrict__ ready, int gather,
+                                                                            const long long* __restrict__ view_pre,
+                                                                            const long long* __restrict__ view_n) {
   __shared__ long long s_pre[kFinMaxB];
   __shared__ int s_nb[kFinMaxB], s_lo[kFinMaxB], s_hi[kFinMaxB];
   __shared__ long long s_tot;
@@ -459,18 +485,24 @@ __global__ void __launch_bounds__(kFinRows* kFinLanes) proto_finalize_kernel(con
   __syncthreads();
   if (tid == 0) {
     long long run = 0;
+    if constexpr (VIEW) run = view_pre[g];
     for (int bb = 0; bb < B; ++bb) {
       s_pre[bb] = run;
       run += s_nb[bb];
     }
-    s_tot = run;
-    if (blockIdx.y == 0) counts[g] = (double)run;
+    if constexpr (VIEW) {   // the counts stay local: the exchange of the sums adds them up
+      s_tot = view_n[g];
+      if (blockIdx.y == 0) counts[g] = view_n[g] < 0 ? -INFINITY : (double)(run - view_pre[g]);
+    } else {
+      s_tot = run;
+      if (blockIdx.y == 0) counts[g] = (double)run;
+    }
   }
   __syncthreads();
   const long long tot = s_tot;
   // fused running-mean update (prototypes.py:158-163; the arithmetic of proto_update_kernel): old count from the snapshot
   float upd_old = 0.f, upd_den = 1.f;
-  if (proto) {
+  if (!VIEW && proto) {
     if (count_is_int64) {
       const long long o = (long long)count_snap[g];
       upd_old = (float)o;
@@ -564,11 +596,41 @@ __global__ void __launch_bounds__(kFinRows* kFinLanes) proto_finalize_kernel(con
     } else {
       t = sums[(int64_t)g * D + r];  // the accumulate launch has already added every image into the row
     }
-    if (proto && tot > 0) {
+    if (!VIEW && proto && tot > 0) {
       const int64_t i = (int64_t)g * D + r;
       proto[i] = __fdiv_rn(__fadd_rn((float)t, __fmul_rn(upd_old, proto[i])), upd_den);
     }
   }
+}
+
+// Count exchange without peer memory: this rank's task totals (the payload of the all-gather), then the view of rank
+// `rank` from the gathered [world][Tn] table, summed in rank order.
+__global__ void __launch_bounds__(kMaxTasks) proto_task_totals_kernel(const int32_t* __restrict__ n_bt, int B, int Tn,
+                                                                     long long* __restrict__ totals) {
+  pdl_wait();
+  pdl_trigger();
+  const int t = threadIdx.x;
+  if (t >= Tn) return;
+  long long n = 0;
+  for (int bb = 0; bb < B; ++bb) n += n_bt[bb * Tn + t];
+  totals[t] = n;
+}
+
+__global__ void __launch_bounds__(kMaxTasks) proto_count_view_kernel(const long long* __restrict__ table, int world,
+                                                                    int rank, int Tn, long long* __restrict__ view_pre,
+                                                                    long long* __restrict__ view_n) {
+  pdl_wait();
+  pdl_trigger();
+  const int t = threadIdx.x;
+  if (t >= Tn) return;
+  long long pre = 0, n = 0;
+  for (int r = 0; r < world; ++r) {
+    const long long v = table[(int64_t)r * Tn + t];
+    if (r < rank) pre += v;
+    n += v;
+  }
+  view_pre[t] = pre;
+  view_n[t] = n;
 }
 
 // proto[g] = (S[g] + cnt[g]*proto[g]) / (cnt[g] + N[g]), cnt[g] += N[g]; separate fp32
@@ -637,7 +699,8 @@ size_t bacs_proto_workspace_bytes(int B, int D, int T) {
 static int proto_accumulate_impl(const void* features, int dtype, int B, int D, int h, int w, const int8_t* task,
                                  const int32_t* rank, const int32_t* n_bt, int T, int mode, double* sums, double* counts,
                                  void* workspace, size_t workspace_bytes, float* proto, void* count, int count_is_int64,
-                                 int32_t* ready, bacs_stream_t stream) {
+                                 int32_t* ready, const long long* view_pre, const long long* view_n,
+                                 bacs_stream_t stream) {
   BACS_REQUIRE(features && task && rank && n_bt && sums && counts && workspace, "bacs_proto_accumulate: null pointer");
   BACS_REQUIRE(B > 0 && D > 0 && h > 0 && w > 0 && B <= kFinMaxB, "bacs_proto_accumulate: bad shape (B <= 1024)");
   BACS_REQUIRE(T > 0 && T <= kMaxTasks, "bacs_proto_accumulate: T=%d not in [1,%d]", T, kMaxTasks);
@@ -665,14 +728,16 @@ static int proto_accumulate_impl(const void* features, int dtype, int B, int D, 
                    (reinterpret_cast<uintptr_t>(task) & 7) == 0 && (reinterpret_cast<uintptr_t>(rank) & 15) == 0;
   // 16-bit features on 32-pixel chunks, 16-channel blocks: one-hot GEMM on the tensor cores (BACS_NO_PROTO_MMA=1: off)
   const bool mma = vec && dtype != BACS_F32 && hw % 32 == 0 && D % 16 == 0 && getenv("BACS_NO_PROTO_MMA") == nullptr;
+  const bool view = view_pre != nullptr;   // global view: its own instantiations, the local ones stay as they are
   if (mma) {
     launch_pdl(proto_zero_sums_kernel, dim3((T * D + 255) / 256), dim3(256), 0, s, sums, T * D);
     BACS_CHECK_LAUNCH("bacs_proto_accumulate(zero)");
     dim3 mgrid((D / 16 + kMmaWarps - 1) / kMmaWarps, B, n_win);
     const int nt = (T + 7) / 8;
 #define BACS_MMA_LAUNCH(TT, NTV, M)                                                                                     \
-  launch_pdl(proto_accumulate_mma_kernel<TT, NTV, M>, mgrid, dim3(32 * kMmaWarps), 0, s, reinterpret_cast<const TT*>(features), \
-             B, D, hw, task, rank, n_bt, T, mode, sums, count_raw, count_is_int64, snap)
+  launch_pdl(view ? proto_accumulate_mma_kernel<TT, NTV, M, true> : proto_accumulate_mma_kernel<TT, NTV, M>, mgrid,      \
+             dim3(32 * kMmaWarps), 0, s, reinterpret_cast<const TT*>(features), B, D, hw, task, rank, n_bt, T, mode, sums, \
+             count_raw, count_is_int64, snap, view_pre, view_n)
 #define BACS_MMA_NT(TT)                                 \
   do {                                                  \
     if (many) BACS_MMA_LAUNCH(TT, 4, true);             \
@@ -688,8 +753,10 @@ static int proto_accumulate_impl(const void* features, int dtype, int B, int D, 
   } else {
   BACS_DISPATCH_DTYPE(dtype, TT, {
     // the table of a 32-task window (vec: 68.6 KB, scalar: 64 KB) needs the opt-in above the 48 KB default
-    auto kern = vec ? (many ? proto_accumulate_vec_kernel<TT, true> : proto_accumulate_vec_kernel<TT>)
-                    : (many ? proto_accumulate_kernel<TT, true> : proto_accumulate_kernel<TT>);
+    auto kern = view ? (vec ? (many ? proto_accumulate_vec_kernel<TT, true, true> : proto_accumulate_vec_kernel<TT, false, true>)
+                            : (many ? proto_accumulate_kernel<TT, true, true> : proto_accumulate_kernel<TT, false, true>))
+                     : (vec ? (many ? proto_accumulate_vec_kernel<TT, true> : proto_accumulate_vec_kernel<TT>)
+                            : (many ? proto_accumulate_kernel<TT, true> : proto_accumulate_kernel<TT>));
     const size_t smem = vec ? vec_smem : acc_smem;
     if (smem > 48 * 1024) {
       cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
@@ -699,12 +766,13 @@ static int proto_accumulate_impl(const void* features, int dtype, int B, int D, 
       }
     }
     launch_pdl(kern, grid, dim3(32 * kAccWarps), smem, s, reinterpret_cast<const TT*>(features), B, D, hw, task, rank,
-               n_bt, T, mode, partial, count_raw, count_is_int64, snap);
+               n_bt, T, mode, partial, count_raw, count_is_int64, snap, view_pre, view_n);
   });
   }
   BACS_CHECK_LAUNCH("bacs_proto_accumulate");
-  launch_pdl(proto_finalize_kernel, dim3(T, (D + kFinRows - 1) / kFinRows), dim3(kFinRows * kFinLanes), 0, s, partial, B, D,
-             n_bt, T, mode, sums, counts, proto, count, count_is_int64, (const unsigned long long*)snap, ready, mma ? 0 : 1);
+  launch_pdl(view ? proto_finalize_kernel<true> : proto_finalize_kernel<>, dim3(T, (D + kFinRows - 1) / kFinRows),
+             dim3(kFinRows * kFinLanes), 0, s, partial, B, D, n_bt, T, mode, sums, counts, proto, count, count_is_int64,
+             (const unsigned long long*)snap, ready, mma ? 0 : 1, view_pre, view_n);
   BACS_CHECK_LAUNCH("bacs_proto_accumulate(finalize)");
   return BACS_OK;
 }
@@ -713,7 +781,41 @@ int bacs_proto_accumulate(const void* features, int dtype, int B, int D, int h, 
                           const int32_t* rank, const int32_t* n_bt, int T, int mode, double* sums, double* counts,
                           void* workspace, size_t workspace_bytes, bacs_stream_t stream) {
   return proto_accumulate_impl(features, dtype, B, D, h, w, task, rank, n_bt, T, mode, sums, counts, workspace,
-                               workspace_bytes, nullptr, nullptr, 0, nullptr, stream);
+                               workspace_bytes, nullptr, nullptr, 0, nullptr, nullptr, nullptr, stream);
+}
+
+int bacs_proto_accumulate_view(const void* features, int dtype, int B, int D, int h, int w, const int8_t* task,
+                               const int32_t* rank, const int32_t* n_bt, int T, int mode, const int64_t* view_pre,
+                               const int64_t* view_n, double* sums, double* counts, void* workspace,
+                               size_t workspace_bytes, bacs_stream_t stream) {
+  BACS_REQUIRE((view_pre == nullptr) == (view_n == nullptr), "bacs_proto_accumulate_view: view_pre and view_n go together");
+  BACS_REQUIRE(T > 0 && T <= kMaxTasks, "bacs_proto_accumulate_view: T=%d not in [1,%d]", T, kMaxTasks);
+  BACS_REQUIRE(view_pre == nullptr || mode == 0, "bacs_proto_accumulate_view: a view needs mode 0 (exact)");
+  return proto_accumulate_impl(features, dtype, B, D, h, w, task, rank, n_bt, T, mode, sums, counts, workspace,
+                               workspace_bytes, nullptr, nullptr, 0, nullptr, reinterpret_cast<const long long*>(view_pre),
+                               reinterpret_cast<const long long*>(view_n), stream);
+}
+
+int bacs_proto_task_totals(const int32_t* n_bt, int B, int T, int64_t* totals, bacs_stream_t stream) {
+  BACS_REQUIRE(n_bt && totals, "bacs_proto_task_totals: null pointer");
+  BACS_REQUIRE(B > 0, "bacs_proto_task_totals: bad shape");
+  BACS_REQUIRE(T > 0 && T <= kMaxTasks, "bacs_proto_task_totals: T=%d not in [1,%d]", T, kMaxTasks);
+  launch_pdl(proto_task_totals_kernel, dim3(1), dim3(kMaxTasks), 0, (cudaStream_t)stream, n_bt, B, T,
+             reinterpret_cast<long long*>(totals));
+  BACS_CHECK_LAUNCH("bacs_proto_task_totals");
+  return BACS_OK;
+}
+
+int bacs_proto_count_view(const int64_t* table, int world, int rank, int T, int64_t* view_pre, int64_t* view_n,
+                          bacs_stream_t stream) {
+  BACS_REQUIRE(table && view_pre && view_n, "bacs_proto_count_view: null pointer");
+  BACS_REQUIRE(world >= 1 && rank >= 0 && rank < world, "bacs_proto_count_view: bad rank/world");
+  BACS_REQUIRE(T > 0 && T <= kMaxTasks, "bacs_proto_count_view: T=%d not in [1,%d]", T, kMaxTasks);
+  launch_pdl(proto_count_view_kernel, dim3(1), dim3(kMaxTasks), 0, (cudaStream_t)stream,
+             reinterpret_cast<const long long*>(table), world, rank, T, reinterpret_cast<long long*>(view_pre),
+             reinterpret_cast<long long*>(view_n));
+  BACS_CHECK_LAUNCH("bacs_proto_count_view");
+  return BACS_OK;
 }
 
 int bacs_proto_accumulate_update(const void* features, int dtype, int B, int D, int h, int w, const int8_t* task,
@@ -723,7 +825,7 @@ int bacs_proto_accumulate_update(const void* features, int dtype, int B, int D, 
   BACS_REQUIRE(proto && count, "bacs_proto_accumulate_update: null pointer");
   BACS_REQUIRE(T > 0 && T <= kMaxTasks, "bacs_proto_accumulate_update: T=%d not in [1,%d]", T, kMaxTasks);
   return proto_accumulate_impl(features, dtype, B, D, h, w, task, rank, n_bt, T, mode, sums, counts, workspace,
-                               workspace_bytes, proto, count, count_is_int64, ready, stream);
+                               workspace_bytes, proto, count, count_is_int64, ready, nullptr, nullptr, stream);
 }
 
 int bacs_proto_update(float* proto, void* count, int count_is_int64, const double* sums, const double* counts, int T,

@@ -42,12 +42,14 @@ def allreduce_packed(sums: torch.Tensor, counts: torch.Tensor, group=None) -> No
 class PeerReducer:
     """One-shot all-reduce over NVLink peer memory, fused with the prototype update (csrc/peer.cu).
 
-    The symmetric buffer (two step-parity slots of ``n_max`` doubles + one flag row) is allocated with
+    The symmetric buffer (two step-parity slots of ``n_max`` doubles, one flag row, and the count table of the
+    global prototype view: two step-parity slots of ``world`` x 128 int64) is allocated with
     ``torch.distributed._symmetric_memory`` and exchanged once; afterwards a step is ONE kernel launch with no
     host synchronisation, capturable in a CUDA graph.  ``create`` returns None when symmetric memory is not
     available for the group (the caller then uses the packed NCCL all-reduce)."""
 
-    FLAG_DOUBLES = 32                      # 64 uint32 flags (16 used)
+    FLAG_DOUBLES = 32                      # 64 uint32 flags: 0..15 the sums phase, 32..47 the count phase
+    COUNT_FLAG_OFFSET = 32                 # first uint32 of the count phase's flags
 
     def __init__(self, n_max: int, device: torch.device, group=None):
         import ctypes as C
@@ -55,7 +57,8 @@ class PeerReducer:
         group = group or dist.group.WORLD
         self.n_max, self.device = int(n_max), device
         self.rank, self.world = dist.get_rank(group), dist.get_world_size(group)
-        self.buf = symm.empty(2 * self.n_max + self.FLAG_DOUBLES, dtype=torch.float64, device=device)
+        count_table = 2 * self.world * 128
+        self.buf = symm.empty(2 * self.n_max + self.FLAG_DOUBLES + count_table, dtype=torch.float64, device=device)
         self.buf.zero_()
         torch.cuda.synchronize(device)
         self.handle = symm.rendezvous(self.buf, group)
@@ -64,7 +67,11 @@ class PeerReducer:
             raise RuntimeError("unexpected symmetric-memory layout")
         self.peer_buf = (C.c_uint64 * self.world)(*ptrs)
         self.peer_flag = (C.c_uint64 * self.world)(*[p + 2 * self.n_max * 8 for p in ptrs])
+        self.peer_count_flag = (C.c_uint64 * self.world)(*[p + 2 * self.n_max * 8 + self.COUNT_FLAG_OFFSET * 4
+                                                            for p in ptrs])
+        self.peer_count_table = (C.c_uint64 * self.world)(*[p + (2 * self.n_max + self.FLAG_DOUBLES) * 8 for p in ptrs])
         self.step = torch.zeros(1, dtype=torch.int32, device=device)
+        self.count_step = torch.zeros(1, dtype=torch.int32, device=device)
         self.error = torch.zeros(1, dtype=torch.int32, device=device)
         dist.barrier(group)                # every rank has zeroed its flags before anybody publishes
         torch.cuda.synchronize(device)
@@ -119,6 +126,23 @@ class PeerReducer:
         return ready
 
 
+    def count_view(self, n_bt: torch.Tensor):
+        """Count phase of the global prototype view (one launch): returns (view_pre, view_n) int64 [T] for
+        ops.proto_accumulate_view.  On a time-out the view is marked invalid, the step then changes no prototype or
+        count, and ``check`` raises."""
+        from . import _cabi, ops
+        n_bt = ops._cuda(n_bt, "PeerReducer.count_view", torch.int32)
+        B, T = n_bt.shape
+        view_pre = torch.empty(T, dtype=torch.int64, device=n_bt.device)
+        view_n = torch.empty(T, dtype=torch.int64, device=n_bt.device)
+        _cabi.check(_cabi.load().bacs_peer_count_exchange(n_bt.data_ptr(), B, T, self.rank, self.world,
+                                                          self.peer_count_table, self.peer_count_flag,
+                                                          self.count_step.data_ptr(), self.error.data_ptr(),
+                                                          view_pre.data_ptr(), view_n.data_ptr(), ops._stream()),
+                    "bacs_peer_count_exchange")
+        return view_pre, view_n
+
+
 _peer_reducers = {}
 
 
@@ -136,6 +160,28 @@ def check_peer_errors() -> None:
     for red in _peer_reducers.values():
         if red is not None:
             red.check()
+
+
+def gather_task_counts(totals: torch.Tensor, group=None) -> torch.Tensor:
+    """[world, T] table of every rank's task totals, rank r in row r (one all-gather; the table is ``totals`` itself
+    at world size 1)."""
+    world = world_size()
+    if world == 1:
+        return totals.reshape(1, -1)
+    table = torch.empty(world * totals.numel(), dtype=totals.dtype, device=totals.device)
+    dist.all_gather_into_tensor(table, totals, group=group)
+    return table.view(world, totals.numel())
+
+
+def exchange_task_counts(n_bt: torch.Tensor, reducer: "Optional[PeerReducer]" = None):
+    """Global view of the exact-mode prototype sums: (view_pre, view_n) int64 [T], task t's masked pixels in the images
+    of the lower ranks / of all ranks.  Through peer memory when ``reducer`` is given, else one all-gather of the
+    [T] task totals; no host synchronisation either way."""
+    if reducer is not None:
+        return reducer.count_view(n_bt)
+    from . import ops
+    table = gather_task_counts(ops.proto_task_totals(n_bt))
+    return ops.proto_count_view(table, dist.get_rank() if world_size() > 1 else 0)
 
 
 def allreduce_state(sums: Optional[torch.Tensor], counts: Optional[torch.Tensor],

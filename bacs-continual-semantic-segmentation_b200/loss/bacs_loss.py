@@ -38,13 +38,16 @@ class BACSLoss(ExperienceReplay):
                  same_task: bool = False, ignore_rep_bg: bool = True, bg_weighted_ce: bool = False,
                  seen_gamma: float = 2, seen_threshold: float = 0.5, seen_ukd: bool = True,
                  seen_focal_alpha: float = None, lkd: float = 0.25, lkd_alpha: float = 0.2,
-                 lkd_threshold: float = 0.5, pseudo_label: bool = False, fused_logit_upsample: bool = False):
+                 lkd_threshold: float = 0.5, pseudo_label: bool = False, fused_logit_upsample: bool = False,
+                 exact_prototypes_across_ranks: bool = False):
         super().__init__(name, ignore_index=ignore_index, same_task=same_task,
                          replay_minibatch_size=replay_minibatch_size, buffer_size=buffer_size,
                          bg_weighted_ce=bg_weighted_ce)
         self.alpha = alpha
         self.beta = beta
         self.fused_logit_upsample = bool(fused_logit_upsample)   # extra keyword (not in the reference), default off
+        # extra keyword (not in the reference), default off: exact-mode prototype sums of the global batch at N > 1
+        self.exact_prototypes_across_ranks = bool(exact_prototypes_across_ranks)
         self.dark_plus_plus = dark_plus_plus
         self.use_cosine_dist = use_cosine_dist
         if use_cosine_dist:

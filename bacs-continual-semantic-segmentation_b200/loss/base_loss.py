@@ -69,6 +69,9 @@ class BaseLoss:
         # opt-in, not in the reference: evaluate the network's final logit up-sample inside the loss kernel (see
         # compute_base_loss); False keeps the reference's data flow ([B,K,H,W] logits from the network)
         self.fused_logit_upsample = False
+        # opt-in, not in the reference: at world size > 1 keep the exact-mode prototype sums, over the rows of the
+        # global batch (Prototypes(exact_across_ranks=True)); False sums per channel there
+        self.exact_prototypes_across_ranks = False
         # fused-kernel by-products of the last compute_base_loss call
         self._fused_preds = None
         self._fused_logits_ref = None
@@ -117,7 +120,8 @@ class BaseLoss:
 
     def init_prototype_compute(self):
         from .prototypes import Prototypes
-        self._prototypes = Prototypes(name="Prototype_{}".format(self.name), ignore_index=self.ignore_index)
+        self._prototypes = Prototypes(name="Prototype_{}".format(self.name), ignore_index=self.ignore_index,
+                                      exact_across_ranks=self.exact_prototypes_across_ranks)
 
     @property
     def prototypes(self):

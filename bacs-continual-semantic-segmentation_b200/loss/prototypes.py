@@ -6,9 +6,16 @@ this batch" early-out are device-side, so ``update_feats_prototypes`` never sync
 
 ``exact=True`` (default) reproduces the reference bit-for-bit in structure, including the
 channel-scrambled row sums of ``features[mask.expand(..)].view(D, -1)`` for B > 1 (Q1).
-``exact=False`` is the per-channel sum the reference computes for B == 1; it is the mode
-used when prototypes are all-reduced across data-parallel ranks (the sums then equal those
-of a single process fed every rank's images one by one)."""
+``exact=False`` is the per-channel sum the reference computes for B == 1.
+
+Across data-parallel ranks (``sync_across_ranks`` with world size > 1) the sums of the ranks
+are added up.  By default the exact mode is dropped there for the per-channel sum (the sums
+then equal those of a single process fed every rank's images one by one).
+``exact_across_ranks=True`` keeps it: one extra exchange of every rank's per-task pixel
+counts gives each rank its images' rows in the view of the global batch, so prototypes and
+counts equal those of one process fed the concatenation of the ranks' batches in rank order.
+It costs one more cross-rank wait per step, before the sums.  At world size 1 it has no
+effect."""
 from __future__ import annotations
 
 from typing import Optional
@@ -21,12 +28,14 @@ from .base_loss import BaseLoss
 
 
 class Prototypes(BaseLoss):
-    def __init__(self, name="Prototypes", ignore_index=255, exact: bool = True, sync_across_ranks: bool = True):
+    def __init__(self, name="Prototypes", ignore_index=255, exact: bool = True, sync_across_ranks: bool = True,
+                 exact_across_ranks: bool = False):
         super().__init__(name, ignore_index)
         self._prototypes_tensors = None
         self._count_features = None
         self.exact = exact
         self.sync_across_ranks = sync_across_ranks
+        self.exact_across_ranks = exact_across_ranks
         self.ready_flag: Optional[torch.Tensor] = None     # int32 [1] on the device
         self._task_lut = None
         self._task_lut_key = None
@@ -121,14 +130,20 @@ class Prototypes(BaseLoss):
         world = 1
         if self.sync_across_ranks and torch.distributed.is_available() and torch.distributed.is_initialized():
             world = torch.distributed.get_world_size()
-        mode = 0 if (self.exact and world == 1) else 1
+        global_view = self.exact and self.exact_across_ranks and world > 1
+        mode = 0 if (self.exact and world == 1) or global_view else 1
         if not self._prototypes_tensors.is_contiguous():
             self._prototypes_tensors = self._prototypes_tensors.contiguous()
         if world > 1:
-            from ..distributed import allreduce_packed, peer_reducer
+            from ..distributed import allreduce_packed, exchange_task_counts, peer_reducer
             packed = torch.empty(T * D + T, dtype=torch.float64, device=features.device)
-            sums, counts = ops.proto_accumulate(features, task, rank, n_bt, T, mode, out=packed)
-            reducer = peer_reducer(packed.numel(), features.device)
+            if global_view:
+                reducer = peer_reducer(packed.numel(), features.device)
+                view_pre, view_n = exchange_task_counts(n_bt, reducer)
+                sums, counts = ops.proto_accumulate_view(features, task, rank, n_bt, T, view_pre, view_n, out=packed)
+            else:
+                sums, counts = ops.proto_accumulate(features, task, rank, n_bt, T, mode, out=packed)
+                reducer = peer_reducer(packed.numel(), features.device)
             if reducer is not None and self._count_features.is_contiguous():
                 # one launch: sum over the ranks through NVLink peer memory + running-mean update
                 self.ready_flag = reducer.allreduce(packed, self._prototypes_tensors, self._count_features, T, D)

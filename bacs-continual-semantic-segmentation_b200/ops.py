@@ -163,6 +163,53 @@ def proto_accumulate_update(features: torch.Tensor, task: torch.Tensor, rank: to
     return sums, counts, ready
 
 
+def proto_accumulate_view(features: torch.Tensor, task: torch.Tensor, rank: torch.Tensor, n_bt: torch.Tensor, T: int,
+                          view_pre: torch.Tensor, view_n: torch.Tensor,
+                          out: Optional[torch.Tensor] = None) -> Tuple[torch.Tensor, torch.Tensor]:
+    """proto_accumulate in the exact mode over the global view of a data-parallel batch: ``view_pre`` / ``view_n``
+    (int64 [T], from distributed.exchange_task_counts) count each task's masked pixels in the images of the lower ranks
+    / of all ranks.  The sums over the ranks equal the exact sums of the concatenated batch; the counts stay local."""
+    check_task_count(T, "proto_accumulate_view")
+    features = _cuda(features, "proto_accumulate_view")
+    view_pre = _cuda(view_pre, "proto_accumulate_view", torch.int64)
+    view_n = _cuda(view_n, "proto_accumulate_view", torch.int64)
+    if view_pre.numel() != T or view_n.numel() != T:
+        raise ValueError("proto_accumulate_view: the view needs %d entries per array" % T)
+    B, D, h, w = features.shape
+    dev = features.device
+    packed = out if out is not None else torch.empty(T * D + T, dtype=torch.float64, device=dev)
+    sums, counts = packed[:T * D].view(T, D), packed[T * D:T * D + T]
+    lib = _lib()
+    ws = _ws(lib.bacs_proto_workspace_bytes(B, D, T), dev)
+    check(lib.bacs_proto_accumulate_view(features.data_ptr(), _dt(features), B, D, h, w, task.data_ptr(), rank.data_ptr(),
+                                         n_bt.data_ptr(), T, 0, view_pre.data_ptr(), view_n.data_ptr(), sums.data_ptr(),
+                                         counts.data_ptr(), ws.data_ptr(), ws.numel(), _stream()),
+          "bacs_proto_accumulate_view")
+    return sums, counts
+
+
+def proto_task_totals(n_bt: torch.Tensor) -> torch.Tensor:
+    """int64 [T]: every task's masked pixels over the images of ``n_bt`` [B, T]."""
+    n_bt = _cuda(n_bt, "proto_task_totals", torch.int32)
+    B, T = n_bt.shape
+    check_task_count(T, "proto_task_totals")
+    totals = torch.empty(T, dtype=torch.int64, device=n_bt.device)
+    check(_lib().bacs_proto_task_totals(n_bt.data_ptr(), B, T, totals.data_ptr(), _stream()), "bacs_proto_task_totals")
+    return totals
+
+
+def proto_count_view(table: torch.Tensor, rank: int) -> Tuple[torch.Tensor, torch.Tensor]:
+    """(view_pre, view_n) int64 [T] of rank ``rank`` from the gathered task totals ``table`` [world, T]."""
+    table = _cuda(table, "proto_count_view", torch.int64)
+    world, T = table.shape
+    check_task_count(T, "proto_count_view")
+    view_pre = torch.empty(T, dtype=torch.int64, device=table.device)
+    view_n = torch.empty(T, dtype=torch.int64, device=table.device)
+    check(_lib().bacs_proto_count_view(table.data_ptr(), world, int(rank), T, view_pre.data_ptr(), view_n.data_ptr(),
+                                       _stream()), "bacs_proto_count_view")
+    return view_pre, view_n
+
+
 def proto_update(proto: torch.Tensor, count: torch.Tensor, sums: torch.Tensor, counts: torch.Tensor,
                  ready: Optional[torch.Tensor] = None) -> torch.Tensor:
     check_task_count(proto.shape[0], "proto_update")

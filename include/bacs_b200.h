@@ -118,6 +118,27 @@ int bacs_proto_accumulate_update(const void* features, int dtype, int B, int D, 
                                  size_t workspace_bytes, float* proto, void* count, int count_is_int64,
                                  int32_t* ready, bacs_stream_t stream);
 
+/* bacs_proto_accumulate in the exact mode over the GLOBAL view of a data-parallel batch: this rank's images are
+ * rows of the D x N_t view of one process fed every rank's images in rank order (rank 0's first).  view_pre[t]
+ * (int64, device) counts task t's masked pixels in the images of the ranks below this one, view_n[t] over all ranks;
+ * image b's entry of channel c lands in row (D*(view_pre[t] + pre_bt) + c*n_bt) / view_n[t].  Summing the ranks'
+ * sums gives the exact sums of the concatenated batch.  counts stay LOCAL (the exchange of the sums adds them up).
+ * The view's values are read on the device and must satisfy view_pre[t] + sum_b n_bt[b][t] <= view_n[t], or
+ * view_n[t] < 0: an invalid view (a peer time-out of bacs_peer_count_exchange), for which task t adds nothing and
+ * counts[t] = -inf, so the running-mean update of bacs_proto_update / bacs_peer_allreduce skips it.
+ * NULL view_pre and view_n: the local view, i.e. exactly bacs_proto_accumulate.  BACS_ERR_INVALID before any launch
+ * when only one of the two is given, T is not in [1, BACS_MAX_TASKS] or a view comes with mode != 0. */
+int bacs_proto_accumulate_view(const void* features, int dtype, int B, int D, int h, int w,
+                               const int8_t* task, const int32_t* rank, const int32_t* n_bt, int T,
+                               int mode, const int64_t* view_pre, const int64_t* view_n, double* sums,
+                               double* counts, void* workspace, size_t workspace_bytes, bacs_stream_t stream);
+
+/* Count exchange without peer memory: totals[t] = sum_b n_bt[b][t] (int64[T]), the payload of an all-gather into a
+ * [world][T] table; bacs_proto_count_view turns that table into rank `rank`'s view (sums in rank order). */
+int bacs_proto_task_totals(const int32_t* n_bt, int B, int T, int64_t* totals, bacs_stream_t stream);
+int bacs_proto_count_view(const int64_t* table, int world, int rank, int T, int64_t* view_pre, int64_t* view_n,
+                          bacs_stream_t stream);
+
 /* Running-mean update proto[g] = (S[g] + cnt[g]*proto[g]) / (cnt[g] + N[g]); cnt[g] += N[g]
  * for rows with N[g] > 0 (prototypes.py:158-163), fp32 arithmetic like torch's.
  * count_is_int64: the reference keeps int64 counts at task 0 and float32 afterwards (Q3).
@@ -448,6 +469,23 @@ int bacs_peer_allreduce(double* packed, int n, int n_max, int rank, int world,
                         const uint64_t* peer_buf_host, const uint64_t* peer_flag_host, uint32_t* step_dev,
                         int32_t* error_dev, float* proto, void* count, int count_is_int64, int T, int D,
                         int32_t* ready, bacs_stream_t stream);
+
+/* Count phase of the global prototype view over NVLink PEER MEMORY (one launch, no host synchronisation,
+ * graph-capturable): this rank's task totals sum_b n_bt[b][t] are pushed into every peer's count table, and after
+ * every peer has published, view_pre / view_n (int64[T], the inputs of bacs_proto_accumulate_view) are summed from
+ * the local table in rank order.
+ *   peer_table_host[r] : device address of rank r's count table of 2 * world * BACS_MAX_TASKS int64
+ *   peer_flag_host[r]  : device address of rank r's count-flag row of >= 16 zero-initialised uint32, apart from
+ *                        the flag row of bacs_peer_allreduce
+ *   step_dev           : device uint32 step counter of the count phase (its own, not that of the sums)
+ *   error_dev          : sticky device int32 (or NULL), as in bacs_peer_allreduce.
+ * On a time-out the view is marked invalid (view_pre = 0, view_n = -1) and error_dev receives the count step: the
+ * accumulate launch adds nothing and reports -inf counts, so the update after the exchange of the sums leaves this
+ * rank's prototypes and counts untouched for the step; the caller must check error_dev and fail.  Every rank must
+ * make the same sequence of calls. */
+int bacs_peer_count_exchange(const int32_t* n_bt, int B, int T, int rank, int world, const uint64_t* peer_table_host,
+                             const uint64_t* peer_flag_host, uint32_t* step_dev, int32_t* error_dev,
+                             int64_t* view_pre, int64_t* view_n, bacs_stream_t stream);
 
 /* Wall-clock bound (milliseconds, > 0) of the peer wait of bacs_peer_allreduce; process-wide. */
 int bacs_peer_set_timeout_ms(int64_t ms);
