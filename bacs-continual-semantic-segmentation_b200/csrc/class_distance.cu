@@ -248,9 +248,12 @@ __global__ void __launch_bounds__(kThreads, 1) class_distance_kernel(const __gri
       }
       s_xx[hf * kTileM + ml] = xx;
       asm volatile("bar.sync 1, %0;" ::"n"(kBuilders) : "memory");
+      // warpgroup (it * nchunks + r) % 4 holds the chunks c = r, r + 4, ... of this tile: adding the partials in
+      // residue order r = 0..3 gives every pixel the same association wherever its tile falls in the CTA's run, so
+      // the distances do not depend on the batch split or the SM count
       xx = 0.f;
 #pragma unroll
-      for (int pt = 0; pt < kParts; ++pt) xx += s_xx[pt * kTileM + ml];   // the same order in every warpgroup
+      for (int r = 0; r < kParts; ++r) xx += s_xx[((it * (uint32_t)nchunks + r) & (kParts - 1)) * kTileM + ml];
       // ---- epilogue: distances of classes [hf*Nh, hf*Nh + Nh) for this pixel ----
       mbar_wait(bar_dfull, it & 1);
       CD_FENCE_AFTER();

@@ -71,6 +71,8 @@ def check_task_count(T: int, name: str) -> None:
 # --------------------------------------------------------------------------------------
 def label_hist(labels: torch.Tensor, out: Optional[torch.Tensor] = None) -> torch.Tensor:
     labels = _cuda(labels, "label_hist", torch.int64)
+    if labels.data_ptr() % 16:       # a view such as big[1:]: the kernel reads labels in 16-byte pairs
+        labels = labels.clone()
     if out is None:
         out = torch.zeros(257, dtype=torch.int64, device=labels.device)
     check(_lib().bacs_label_hist(labels.data_ptr(), labels.numel(), out.data_ptr(), _stream()), "bacs_label_hist")

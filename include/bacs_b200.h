@@ -413,7 +413,8 @@ int bacs_confmat_metrics(const int64_t* confmat, int K, float* out, bacs_stream_
  * resident in one SM's shared memory next to 32 KB of staging (<= 224 KB; 150 x 512 fits); BACS_ERR_UNSUPPORTED
  * otherwise.  One hand-written kernel (csrc/class_distance.cu): TMA -> tensor memory (A) / shared memory (B) ->
  * tcgen05.mma -> norms, clamp and arg-min in the epilogue.  The workspace is not used (size query kept for callers).
- * nearest may be NULL.
+ * nearest may be NULL.  The results do not depend on how the batch is split over calls, on the device's SM count or
+ * on nearest being NULL: every pixel's distances are summed in the same order wherever its tile is computed.
  * --------------------------------------------------------------------------------- */
 size_t bacs_class_distance_workspace_bytes(int32_t B, int32_t Kc, int32_t D, int32_t h, int32_t w);
 int bacs_class_distance(const void* features, int dtype, int32_t B, int32_t D, int32_t h, int32_t w, const void* protos,
@@ -423,8 +424,9 @@ int bacs_class_distance(const void* features, int dtype, int32_t B, int32_t D, i
 /* Per-class feature sums of the same family (SDR's per-class prototypes, loss/sdr.py:120-159; the segmented reduction
  * of bacs_proto_accumulate with one group per CLASS instead of per task): sums[k][c] = sum over the low-res pixels of
  * class k of features[b][c][pixel], fp64 [K, D], OVERWRITTEN.  labels_down int64 [B,h,w] holds class ids (what
- * bacs_label_downsample_task returns as labels_down); ids outside [0, K) -- ignore-255 -- are skipped.  The per-class
- * pixel counts are bacs_label_hist of the same labels.  workspace >= bacs_class_sums_workspace_bytes. */
+ * bacs_label_downsample_task returns as labels_down); ids outside [0, K) -- ignore-255 when K <= 255 -- are skipped,
+ * and 255 is summed as a class when K = 256.  Limits: 0 < B < 65536 and 0 < K <= 1024.  The per-class pixel counts
+ * are bacs_label_hist of the same labels (257 bins: classes 0..255).  workspace >= bacs_class_sums_workspace_bytes. */
 size_t bacs_class_sums_workspace_bytes(int32_t B, int32_t D, int32_t K);
 int bacs_class_sums(const void* features, int dtype, int32_t B, int32_t D, int32_t h, int32_t w,
                     const int64_t* labels_down, int32_t K, double* sums, void* workspace,
