@@ -113,6 +113,7 @@ __global__ void __launch_bounds__(256) remap_presence_kernel(const int64_t* __re
       for (int u = 0; u < 4; ++u) x[u] = (i + u * step < nv) ? __ldg(v + i + u * step) : make_longlong2(lo, lo);
 #pragma unroll
       for (int u = 0; u < 4; ++u) {
+        if (i + u * step >= nv) break;  // a padded lane: lo is not in the image just because the sweep ran past it
         mark(x[u].x);
         mark(x[u].y);
       }

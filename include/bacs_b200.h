@@ -69,7 +69,8 @@ int bacs_label_hist(const int64_t* labels, int64_t n, int64_t* hist, bacs_stream
  * that pass's masking value by the host; all map and masking values must lie inside the
  * domain.  map2 may be NULL (single pass).  Labels outside the domain behave like
  * unmapped ones.  The remap is per image (`n_images` x `pixels_per_image`) because the
- * reference transforms one target at a time.  in/out int64, may alias.
+ * reference transforms one target at a time.  in/out int64, may alias.  The result does not
+ * depend on the image shape, the batch size or the alignment of in/out.
  * workspace: bacs_label_remap_workspace_bytes(n_images). */
 size_t bacs_label_remap_workspace_bytes(int64_t n_images);
 int bacs_label_remap(const int64_t* in, int64_t* out, int64_t n_images, int64_t pixels_per_image,
@@ -391,7 +392,10 @@ int bacs_unbiased_kd(const void* logits, const void* old_logits, int dtype, int 
 /* confmat[t*K + p] += 1 for pixels with 0 <= t < K (rows = target).  preds are int64
  * (preds_is_float = 0) or fp32 truncated like .int() (metrics.py:45-46).  Predictions
  * outside [0,K) on a kept pixel are counted in oob[0] (torch.bincount would have
- * enlarged / raised); confmat int64[K*K] is accumulated in place. */
+ * enlarged / raised); confmat int64[K*K] is accumulated in place.  Both int64 operands
+ * wrap to int32 first, so 2^32 + c counts as c.  An fp32 prediction is truncated toward
+ * zero (-0.5 -> class 0); on a kept pixel, one at or beyond +-2^31, or infinite, counts
+ * as oob.  NaN predictions are not specified. */
 int bacs_confmat_accumulate(const void* preds, int preds_is_float, const int64_t* target,
                             int64_t n, int K, int64_t* confmat, int64_t* oob,
                             bacs_stream_t stream);
